@@ -49,7 +49,7 @@ METRIC = "batched env-steps/sec (CliffordGym 8q all-to-all {H,S,CX})"
 UNIT = "env-steps/s"
 
 
-def parse_args():
+def parse_args(argv=None):
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=50)
@@ -71,13 +71,52 @@ def parse_args():
     ap.add_argument("--obs-buffers", type=int, default=0, help="slabs of the observation / mask ring a launch rotates over: 0 = automatic (> 2x L2 in total)")
     ap.add_argument("--tile-envs", type=int, default=0, help="qg_config.tile_envs of the env-step legs: 0 = automatic, 16 or 32 (A/B runs)")
     ap.add_argument("--synth-all-backends", action="store_true", help="also time the two-kernel and PyTorch-policy searches")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed episode returned as DIR/<name>.npy "
+                                                          "(float32; a fixed sample of environments, under 64 MB in all)")
+    args = ap.parse_args(argv)
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA engine's outputs (--impl ours)")
+    return args
 
 
 def workload(args):
     from qiskit_gym_b200 import workloads as W
     kind, n, gateset, kw = W.baseline_configs()[args.config]
     return kind, n, gateset, dict(kw)
+
+
+def episode_inputs(args, envs, rank=0):
+    """The synthetic episode one rank plays, a function of the command line and the rank only (seeded per rank so that shards differ
+    but are reproducible): set_state targets int64[envs, payload], actions int32[T, envs] and, with add_inverts, coins uint8[T, envs]."""
+    from qiskit_gym_b200 import workloads as W
+    kind, n, gateset, _ = workload(args)
+    T = args.episode_steps
+    targets = W.random_targets(kind, n, gateset, envs, 20261017 + 3 + 1000 * rank, scramble=256)
+    rng = np.random.Generator(np.random.PCG64(20261017 + rank))
+    actions = W.random_actions(rng, T, envs, len(gateset))
+    coins = rng.integers(0, 2, size=(T, envs)).astype(np.uint8) if (args.add_inverts and kind != W.PAULI) else None
+    return targets, actions, coins
+
+
+DUMP_BYTES = 60 << 20          # what --dump-outputs writes, .npy headers aside: under 64 MB
+
+
+def dump_outputs(out_dir, obs_ring, mask_ring, reward, done, success):
+    """Writes what the last replayed episode returned, as float32 .npy files: obs [steps, S, obs_size] and mask [steps, S, A] of the
+    env-steps still in the ring (all T with the default ring, otherwise the last ones, oldest first), reward / done / success [T, S].
+    The S environments are np.random.default_rng(0).choice(B, S, replace=False) in ascending order, the whole batch where it fits."""
+    import torch
+    nbuf, B, obs_size = obs_ring.shape
+    T, A = reward.shape[0], mask_ring.shape[2]
+    steps = min(nbuf, T)
+    S = min(B, DUMP_BYTES // (4 * (steps * (obs_size + A) + 3 * T)))
+    envs = torch.from_numpy(np.sort(np.random.default_rng(0).choice(B, S, replace=False))).to(obs_ring.device)
+    slots = torch.tensor([t % nbuf for t in range(T - steps, T)], device=obs_ring.device)
+    out = {"obs": obs_ring.index_select(1, envs).index_select(0, slots), "mask": mask_ring.index_select(1, envs).index_select(0, slots),
+           "reward": reward.index_select(1, envs), "done": done.index_select(1, envs), "success": success.index_select(1, envs)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def config_json(args, n_gpus):
@@ -159,11 +198,8 @@ def cpu_run(args, envs, steps=1, warmup=0, threads=None):
         pk["add_inverts"] = bool(args.add_inverts)
     cfg = orc.make_config(kind, n, gateset, add_perms=False, **pk)
     T = args.episode_steps
-    targets = W.random_targets(kind, n, gateset, envs, 20261017 + 3, scramble=256)
+    targets, actions, coins = episode_inputs(args, envs)
     lens = W.payload_lengths(kind, n, targets)
-    rng = np.random.Generator(np.random.PCG64(20261017))
-    actions = W.random_actions(rng, T, envs, len(gateset))
-    coins = rng.integers(0, 2, size=(T, envs)).astype(np.uint8) if (args.add_inverts and kind != W.PAULI) else None
     times = []
     for i in range(warmup + steps):
         sec, _ = orc.bench(cfg, targets, lens, actions, coins=coins, threads=threads)
@@ -230,16 +266,11 @@ def run_ours(args):
         pk["add_inverts"] = bool(args.add_inverts)
     env = BatchedEnv(kind, n, gateset, B, device=local, max_depth=T, add_perms=False, tile_envs=args.tile_envs, **pk)
     obs_size = int(np.prod(env.obs_shape()))
-    # synthetic inputs (seeded per global env id range so shards differ but are reproducible)
-    targets = W.random_targets(kind, n, gateset, B, 20261017 + 3 + 1000 * rank, scramble=256)
+    targets, actions_h, coins_h = episode_inputs(args, B, rank)
     env.set_state(targets)
     env.snapshot()
-    rng = np.random.Generator(np.random.PCG64(20261017 + rank))
-    actions_h = W.random_actions(rng, T, B, A)
     actions = torch.from_numpy(actions_h).to(dev)
-    coins = None
-    if args.add_inverts and kind != W.PAULI:
-        coins = torch.from_numpy(rng.integers(0, 2, size=(T, B)).astype(np.uint8)).to(dev)
+    coins = None if coins_h is None else torch.from_numpy(coins_h).to(dev)
     # observation / mask ring: one slab per env-step of an episode, so that a launch never rewrites a line that may still be in L2 (with a short
     # ring and few tiles in flight the L2 absorbs part of the rewrites and the launch "beats" the DRAM bandwidth: profiles/r2_v26_pair_ab.txt)
     obs_bytes = B * obs_size * 4
@@ -322,6 +353,8 @@ def run_ours(args):
             stream.synchronize()
     load_t0[0] = time.time() - 0.7               # clock samples of the last 0.7 s of the pre-spin count as "under load"
     ms, clocks = timed(g_replay, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, obs_ring, mask_ring, rew_tb, done_tb, succ_tb)
     ms_steps = timed(g_steps)[0] if g_steps is not None else None
     packed = None
     if not args.no_packed and not (kind == W.PERM and n > 64):

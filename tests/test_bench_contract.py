@@ -1,8 +1,12 @@
-"""bench.py's contract on the CPU: the reference arm prints exactly one JSON line on stdout with the keys the driver reads."""
+"""bench.py's contract: the reference arm prints exactly one JSON line on stdout with the result keys (CPU), and --dump-outputs writes
+what the timed episode computed (GPU)."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -28,3 +32,31 @@ def test_reference_arm_other_ranks_stay_silent():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_oracle_episode(tmp_path):
+    """--steps sets the timed launches, and --dump-outputs writes the last timed episode: at 256 environments the sample is the whole
+    batch, and every array equals the CPU oracle's on the same seeded targets, actions and add_inverts coins."""
+    import bench
+    from oracle import oracle as orc
+    from qiskit_gym_b200 import workloads as W
+    argv = ["--steps", "3", "--warmup", "0", "--envs", "256", "--episode-steps", "24", "--add-inverts", "1", "--no-cpu-baseline", "--no-e2e",
+            "--no-per-step", "--no-synth", "--no-packed", "--no-collector", "--dump-outputs", str(tmp_path)]
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout)
+    assert line["steps"] == 3 and line["gpu_launches"] == 3 and line["engine_error_flags"] == 0
+
+    args = bench.parse_args(argv)
+    kind, n, gateset, kw = bench.workload(args)
+    targets, actions, coins = bench.episode_inputs(args, args.envs)
+    assert coins is not None
+    cfg = orc.make_config(kind, n, gateset, max_depth=args.episode_steps, add_perms=False, **dict(kw, add_inverts=True))
+    ref = orc.run_batch(cfg, targets, W.payload_lengths(kind, n, targets), actions, coins=coins)
+    got = {name: np.load(tmp_path / f"{name}.npy") for name in ("obs", "mask", "reward", "done", "success")}
+    assert all(a.dtype == np.float32 for a in got.values())
+    assert np.array_equal(got["obs"], ref["obs"].astype(np.float32))
+    assert np.array_equal(got["reward"].view(np.uint32), ref["reward"].view(np.uint32))
+    assert np.array_equal(got["done"], ref["done"].astype(np.float32)) and np.array_equal(got["success"], ref["success"].astype(np.float32))
+    assert np.array_equal(got["mask"], np.repeat(1 - ref["success"][..., None], len(gateset), axis=2).astype(np.float32))
