@@ -293,6 +293,14 @@ QG_API int qg_reset_select_dev(qg_engine* e, const uint64_t* seed_dev, int64_t f
 QG_API int qg_collect_step_dev(qg_engine* e, const uint64_t* seed_dev, const float* weights_dev, int32_t deterministic,
                                float* obs_dev, uint8_t* mask_dev, int32_t* chosen_dev,
                                float* reward_dev, uint8_t* done_dev, uint8_t* success_dev, qg_stream stream);
+/* qg_collect_step_dev for a collector with twists: weights_dev float[B][A] are in the policy's (twisted) action order and env action g of
+ * env i takes the weight weights[i][act_perm[twist[i]][g]] (act_perm_dev int32[K][A], the act_perms of qg_twists_copy; twist_dev int32[B]).
+ * The pick is bit-identical to qg_twist_gather(weights, act_perm, twist) followed by qg_collect_step_dev, without the gathered copy.
+ * policy_chosen_dev (int32[B], may be NULL): the chosen action in the policy's order, act_perm[twist[i]][chosen], or -1 where chosen is -1.
+ * No observation / mask output. */
+QG_API int qg_collect_step_twisted_dev(qg_engine* e, const uint64_t* seed_dev, const float* weights_dev, const int32_t* act_perm_dev,
+                                       const int32_t* twist_dev, int32_t deterministic, int32_t* chosen_dev, int32_t* policy_chosen_dev,
+                                       float* reward_dev, uint8_t* done_dev, uint8_t* success_dev, qg_stream stream);
 /* Generalised advantage estimation over a rollout laid out [num_steps][batch] (value_dev has num_steps + 1 rows, the
  * last one bootstraps the truncated episodes):  nd = !done[t];  delta = (reward[t] + (gamma*value[t+1])*nd) - value[t];
  * adv[t] = delta + ((gamma*lambda)*nd)*adv[t+1];  ret[t] = adv[t] + value[t]  — f32, every operation rounded on its
@@ -306,6 +314,14 @@ QG_API int qg_gae(const float* reward_dev, const float* value_dev, const uint8_t
  * the env's action order. */
 QG_API int qg_twist_gather(const float* in_dev, float* out_dev, const int32_t* table_dev, const int32_t* index_dev,
                            int64_t batch, int32_t len, qg_stream stream);
+/* Twists on packed observations (Permutation / LinearFunction / Clifford: every obs perm is the lift of a qubit permutation p, entry (r, c) of
+ * the dim x dim observation -> (lift(r), lift(c)), lift(i) = p[i] for i < n, n + p[i - n] otherwise; dim = n or 2n).  qperm_inv_dev uint8
+ * [num_twists][num_qubits] holds p^-1 per twist; out_bits = the packed bits of qg_twist_gather(unpacked in_bits, inverse obs perm, k).  The
+ * twist index k of env b is index_dev[b] when given, else drawn on the device: mulhi(philox(*seed_dev; first_env_id + b, draw, stream 5),
+ * num_twists), and written to index_out_dev[b] when that is not NULL.  in_bits / out_bits uint32[batch][ceil(obs_size / 32)], not in place. */
+QG_API int qg_twist_bits(const uint32_t* in_bits_dev, uint32_t* out_bits_dev, int64_t batch, int32_t obs_size, int32_t num_qubits, int32_t dim,
+                         const uint8_t* qperm_inv_dev, int32_t num_twists, const int32_t* index_dev, const uint64_t* seed_dev,
+                         int64_t first_env_id, int32_t draw, int32_t* index_out_dev, qg_stream stream);
 
 /* ---- packed-bit observations + fused policy network (SURVEY.md §8f row 3) ------------------------------------------
  * Env::observe returns the indices of the non-zero entries (e.g. clifford.rs:361-368) because twisterl's policy sums
@@ -366,6 +382,13 @@ QG_API int32_t qg_policy_tc_num_actions(const qg_policy_tc* p);
 QG_API int32_t qg_policy_tc_set_mode(qg_policy_tc* p, int32_t per_layer);
 QG_API int qg_policy_tc_forward_bits(qg_policy_tc* p, const uint32_t* obs_bits_dev, int64_t batch, float* probs_dev, float* logits_dev,
                                      float* values_dev, qg_stream stream);
+/* Refreshes the handle's weights in place from f32 DEVICE tensors (a training loop's parameters): the same hi / lo split as
+ * qg_policy_tc_create, stream-ordered, no allocation, every device pointer kept — a CUDA graph captured with this handle stays valid.  The
+ * shapes (obs_size, num_layers, out_features, value head present or not) must equal those of creation.  weights_dev[l] float[out][in]
+ * row-major, biases_dev[l] float[out], value_weight_dev float[in of the last layer], value_bias_dev float[1] (both NULL without a value head). */
+QG_API int qg_policy_tc_load_weights_dev(qg_policy_tc* p, int32_t obs_size, int32_t num_layers, const int32_t* out_features,
+                                         const float* const* weights_dev, const float* const* biases_dev,
+                                         const float* value_weight_dev, const float* value_bias_dev, qg_stream stream);
 
 /* The whole rollout search in ONE launch: every CTA owns 8 rollouts and loops  policy (packed observation -> action weights) ->
  * sample / arg-max + fused step -> next packed observation  until its rollouts are final or max_decisions decisions were taken;

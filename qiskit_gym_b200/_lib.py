@@ -32,7 +32,7 @@ SYMBOLS = [
     "qg_solutions", "qg_solutions_host", "qg_replay_host_packed", "qg_replay_host_packed_async", "qg_replay_packed", "qg_host_alloc", "qg_host_free", "qg_bind_thread_to_device",
     "qg_dlpack_obs", "qg_search_finish", "qg_nccl_unique_id", "qg_nccl_comm_create", "qg_nccl_comm_destroy",
     "qg_policy_tc_create", "qg_policy_tc_destroy", "qg_policy_tc_num_actions", "qg_policy_tc_forward_bits", "qg_policy_tc_set_mode",
-    "qg_reset_select_dev", "qg_collect_step_dev",
+    "qg_reset_select_dev", "qg_collect_step_dev", "qg_collect_step_twisted_dev", "qg_twist_bits", "qg_policy_tc_load_weights_dev",
 ]
 
 
@@ -154,6 +154,9 @@ def lib():
     L.qg_policy_tc_set_mode.argtypes = [vp, i32]
     L.qg_reset_select_dev.argtypes = [vp, vp, i64, vp, vp]
     L.qg_collect_step_dev.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]
+    L.qg_collect_step_twisted_dev.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp, vp]
+    L.qg_twist_bits.argtypes = [vp, vp, i64, i32, i32, i32, vp, i32, vp, vp, i64, i32, vp, vp]
+    L.qg_policy_tc_load_weights_dev.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, vp]
     _lib = L
     return L
 

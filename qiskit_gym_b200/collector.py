@@ -52,10 +52,7 @@ class Rollout:
 
     def unpack_obs(self, t0: int = 0, t1: int | None = None) -> torch.Tensor:
         """Dense f32 observations of decisions t0 .. t1-1 from the packed bits (for the update step of a trainer)."""
-        bits = self.obs_bits[t0:t1]
-        shifts = torch.arange(32, dtype=torch.int32, device=bits.device)
-        dense = ((bits.unsqueeze(-1) >> shifts) & 1).reshape(bits.shape[0], bits.shape[1], -1)
-        return dense[..., : self.obs_size].float()
+        return unpack_bits(self.obs_bits[t0:t1], self.obs_size)
 
     obs_size: int = 0
 
@@ -65,6 +62,13 @@ class Rollout:
         n = int(fin.sum().item())
         ok = int((self.successes & fin).sum().item())
         return n, (ok / n if n else 0.0)
+
+
+def unpack_bits(bits: torch.Tensor, obs_size: int) -> torch.Tensor:
+    """Packed observations int32 [..., obs_words] -> dense f32 [..., obs_size] (bit i % 32 of word i // 32 = entry i)."""
+    shifts = torch.arange(32, dtype=torch.int32, device=bits.device)
+    dense = ((bits.unsqueeze(-1) >> shifts) & 1).reshape(bits.shape[:-1] + (-1,))
+    return dense[..., :obs_size].float()
 
 
 def gae(rewards: torch.Tensor, values: torch.Tensor, dones: torch.Tensor, gamma: float, lam: float, valid: torch.Tensor | None = None):
@@ -96,6 +100,42 @@ def twist_gather(src: torch.Tensor, table: torch.Tensor, index: torch.Tensor | N
     return out.reshape(src.shape)
 
 
+def qubit_twist_table(obs_perms, num_qubits: int) -> np.ndarray:
+    """uint8 [K, n]: the inverse qubit permutation of every twist, for qg_twist_bits.  Every obs perm of Permutation / LinearFunction /
+    Clifford lifts a qubit permutation p to the d x d observation (d = n or 2n): entry (r, c) -> (lift(r), lift(c)), lift(i) = p[i] (i < n),
+    n + p[i - n] (i >= n).  p is read off the first column and every row is checked to have that form."""
+    op = np.asarray(obs_perms, dtype=np.int64)
+    K, size = op.shape
+    d, n = int(round(size ** 0.5)), int(num_qubits)
+    if d * d != size or d not in (n, 2 * n):
+        raise NotImplementedError(f"twists on packed observations need a square observation of side n or 2n (got {size} entries, n = {n})")
+    p = op[:, : n * d : d] // d                                          # lift(i) for i < n, from entry (i, 0) -> (lift(i), lift(0))
+    lift = p if d == n else np.concatenate([p, p + n], axis=1)
+    if not np.array_equal(op, (lift[:, :, None] * d + lift[:, None, :]).reshape(K, size)) or not np.array_equal(np.sort(p, axis=1), np.broadcast_to(np.arange(n), p.shape)):
+        raise NotImplementedError("an obs perm of these twists is not the lift of a qubit permutation: twists on packed observations do not apply")
+    return np.argsort(p, axis=1).astype(np.uint8)
+
+
+def twist_bits(src: torch.Tensor, out: torch.Tensor, qperm_inv: torch.Tensor, num_qubits: int, index: torch.Tensor | None = None,
+               seed_dev: torch.Tensor | None = None, first_env_id: int = 0, draw: int = 0, index_out: torch.Tensor | None = None, obs_size: int | None = None):
+    """qg_twist_bits: packed observations int32 [B, obs_words] -> the same observations in twist frame k[b] (entry i -> obs_perms[k][i]).
+    k = index[b], or drawn on the device from the Philox seed in seed_dev (int64 [1]) — mulhi(philox(seed; first_env_id + b, draw, 5), K) —
+    and written to index_out (int32 [B]) when given.  qperm_inv: uint8 [K, n] of qubit_twist_table."""
+    B, ow = int(src.shape[0]), int(src.shape[-1])
+    assert src.is_cuda and src.element_size() == 4 and src.is_contiguous() and out.is_contiguous() and out.shape == src.shape
+    assert qperm_inv.dtype == torch.uint8 and qperm_inv.is_contiguous() and qperm_inv.shape[1] == num_qubits
+    assert index is None or (index.dtype == torch.int32 and index.numel() == B)
+    assert index is not None or (seed_dev is not None and seed_dev.element_size() == 8)
+    assert index_out is None or (index_out.dtype == torch.int32 and index_out.numel() == B and index_out.is_contiguous())
+    size = obs_size if obs_size is not None else ow * 32
+    d = int(round(size ** 0.5))
+    st = C.c_void_p(torch.cuda.current_stream(src.device).cuda_stream)
+    with torch.cuda.device(src.device):
+        check(lib().qg_twist_bits(_dptr(src), _dptr(out), B, int(size), int(num_qubits), d, _dptr(qperm_inv), int(qperm_inv.shape[0]), _dptr(index),
+                                  _dptr(seed_dev), int(first_env_id), int(draw), _dptr(index_out), st))
+    return out
+
+
 class RolloutCollector:
     def __init__(self, env: BatchedEnv, policy: torch.nn.Module, gamma: float = 0.995, lam: float = 0.995, use_twists: bool = True,
                  seed: int = 0, first_env_id: int = 0, matmul_precision: str = "f32"):
@@ -119,6 +159,7 @@ class RolloutCollector:
                 self.obs_table = torch.from_numpy(inv.astype(np.int32)).to(env.device)
                 self.act_table = torch.from_numpy(np.asarray(act_perms, dtype=np.int32)).to(env.device)
         self.num_twists = 0 if self.obs_table is None else int(self.obs_table.shape[0])
+        self.qperm_table = None           # collect_packed: uint8 [K, n] inverse qubit permutations (qubit_twist_table), built on first use
         self._gen = torch.Generator(device=env.device)
         self._gen.manual_seed(self.seed & (2**63 - 1))
         self.hook = None                  # tests: called as hook(t, weights [B, A] in env action order) before each collect step
@@ -140,22 +181,41 @@ class RolloutCollector:
                 logits, value = self.policy(obs)
             return torch.softmax(logits.float(), dim=-1), value.float().reshape(-1)
 
+    def tensor_core_policy(self):
+        """The collect_packed policy handle (policy.TensorCorePolicy) for the current weights.  A weight update (optimizer step, load_state_dict)
+        is copied into the existing handle in place (TensorCorePolicy.load_weights: captured rollout graphs stay valid); the handle is rebuilt —
+        and the graphs dropped — only for a new shape, parameters that are not f32 / contiguous on the device, or a larger batch.
+        Raises NotImplementedError where the tensor-core policy cannot run (more than 127 actions, a value head that is not one Linear,
+        a device that is not sm_100)."""
+        from .policy import TensorCorePolicy, weights_version
+        B = self.env.batch
+        tcp = getattr(self, "_tcp", None)
+        if tcp is None or tcp.max_batch < B or not tcp.can_load(self.policy):
+            tcp = self._tcp = TensorCorePolicy(self.policy, max_batch=B, device=self.env.device, with_value=True)
+            self._packed = {}
+        elif tcp.version != weights_version(self.policy):
+            tcp.load_weights(self.policy)
+        return tcp
+
     def collect_packed(self, num_steps: int, deterministic: bool = False, use_cuda_graph: bool = True) -> Rollout:
         """The large-batch collection path: packed-bit observations (32x less observation traffic than dense f32) and the policy on the
-        tensor cores (policy.TensorCorePolicy, tcgen05).  Per decision: reset_select -> observe_bits -> qg_policy_tc_forward_bits (softmax
-        weights + value) -> qg_collect_step; log-probabilities and GAE once at the end.  No twists on this path.
+        tensor cores (policy.TensorCorePolicy, tcgen05).  Per decision: reset_select -> observe_bits [-> qg_twist_bits: the observation in a
+        twist frame drawn per env on the device] -> qg_policy_tc_forward_bits (softmax weights + value) -> qg_collect_step (twisted collectors:
+        qg_collect_step_twisted_dev, which maps the policy's actions back to the env's order while it samples); log-probabilities and GAE once
+        at the end.  Same contract as collect(): obs_bits hold what the policy saw, `twist` the twist indices, policy_actions the action in the
+        policy's order.  Twist k of env b at decision t is mulhi(philox(decision seed t; first_env_id + b, 0, stream 5), K); the bootstrap
+        observation after the last decision uses draw 1 of the last decision's seed.
         use_cuda_graph: the whole rollout (num_steps decisions, ~6 launches each) is captured once and replayed; the decisions' Philox seeds
-        are read from a device array the host refills before every replay (qg_reset_select_dev / qg_collect_step_dev).  The returned tensors
-        are the collector's own buffers: they are overwritten by the next call with the same num_steps."""
-        from .policy import TensorCorePolicy, weights_version
+        are read from a device array the host refills before every replay (qg_reset_select_dev / qg_collect_step_dev).  A weight update is
+        loaded into the policy handle in place, so the graph survives training steps.  The returned tensors are the collector's own buffers:
+        they are overwritten by the next call with the same num_steps."""
         env, T, B = self.env, int(num_steps), self.env.batch
         dev, A = env.device, env.num_actions()
-        if self.num_twists:
-            raise NotImplementedError("collect_packed does not apply twists (construct the collector with use_twists=False)")
-        tcp = getattr(self, "_tcp", None)
-        if tcp is None or tcp.version != weights_version(self.policy) or tcp.max_batch < B:
-            tcp = self._tcp = TensorCorePolicy(self.policy, max_batch=B, device=dev, with_value=True)
-            self._packed = {}
+        assert T >= 1
+        twisted = self.num_twists > 0
+        if twisted and self.qperm_table is None:
+            self.qperm_table = torch.from_numpy(qubit_twist_table(env.twists()[0], int(env.cfg.num_qubits))).to(dev)
+        tcp = self.tensor_core_policy()
         st = self._packed.get((T, deterministic))
         if st is None:
             ow = env.obs_words()
@@ -164,21 +224,41 @@ class RolloutCollector:
                   "dones": torch.zeros((T, B), dtype=torch.bool, device=dev), "succ": torch.zeros((T, B), dtype=torch.bool, device=dev),
                   "values": torch.zeros((T + 1, B), dtype=torch.float32, device=dev), "seeds": torch.zeros(T, dtype=torch.int64, device=dev),
                   "seeds_host": torch.zeros(T, dtype=torch.int64).pin_memory(), "graph": None, "runs": 0}
+            if twisted:
+                st["raw"] = torch.empty((B, ow), dtype=torch.int32, device=dev)                  # observe_bits before the twist
+                st["twist"] = torch.zeros((T + 1, B), dtype=torch.int32, device=dev)            # row T: the bootstrap observation's twist
+                st["pol_actions"] = torch.full((T, B), -1, dtype=torch.int32, device=dev)
             self._packed[(T, deterministic)] = st
+        difficulty = env.difficulty
+        if st.get("difficulty") != difficulty:       # the env config (difficulty included) is a launch parameter a captured graph keeps
+            st["graph"], st["runs"], st["difficulty"] = None, 0, difficulty
         bits, probs, actions, rewards, dones, succ, values, seeds = (st[k] for k in ("bits", "probs", "actions", "rewards", "dones", "succ", "values", "seeds"))
         for t in range(T):          # the seeds of this rollout's decisions (two's-complement view of the uint64 seeds)
             s_ = decision_seed(self.seed, self.counter + t)
             st["seeds_host"][t] = s_ - (1 << 64) if s_ >= (1 << 63) else s_
         seeds.copy_(st["seeds_host"], non_blocking=True)
         self.counter += T
+        n = int(env.cfg.num_qubits)
+
+        def observe(t, draw, seed_row):
+            if not twisted:
+                env.observe_bits(bits[t])
+                return
+            env.observe_bits(st["raw"])
+            twist_bits(st["raw"], bits[t], self.qperm_table, n, seed_dev=seeds[seed_row:seed_row + 1], first_env_id=self.first_env_id, draw=draw,
+                       index_out=st["twist"][t], obs_size=env._obs_size)
 
         def body():
             for t in range(T):
                 env.reset_select_dev(seeds[t:t + 1], self.first_env_id)
-                env.observe_bits(bits[t])
+                observe(t, 0, t)
                 tcp.forward_bits(bits[t], probs=probs[t], values=values[t])
-                env.collect_step_dev(probs[t], seeds[t:t + 1], deterministic=deterministic, chosen=actions[t], reward=rewards[t], done=dones[t], success=succ[t])
-            env.observe_bits(bits[T])
+                if twisted:
+                    env.collect_step_twisted_dev(probs[t], self.act_table, st["twist"][t], seeds[t:t + 1], deterministic=deterministic, chosen=actions[t],
+                                                 policy_chosen=st["pol_actions"][t], reward=rewards[t], done=dones[t], success=succ[t])
+                else:
+                    env.collect_step_dev(probs[t], seeds[t:t + 1], deterministic=deterministic, chosen=actions[t], reward=rewards[t], done=dones[t], success=succ[t])
+            observe(T, 1, T - 1)
             tcp.forward_bits(bits[T], values=values[T])
 
         if not use_cuda_graph:
@@ -195,11 +275,11 @@ class RolloutCollector:
                 st["graph"] = g
             st["graph"].replay()
         valid = actions >= 0
-        a = actions.long().clamp_(min=0)
+        a = (st["pol_actions"] if twisted else actions).long().clamp_(min=0)
         logp = torch.log(probs.gather(2, a[..., None]).squeeze(2).clamp_min(1e-38))
         adv, ret = gae(rewards, values, dones, self.gamma, self.lam, valid)
         return Rollout(obs=None, actions=actions, policy_actions=a, logp=logp, values=values, rewards=rewards, dones=dones, successes=succ, valid=valid,
-                       advantages=adv, returns=ret, twist=None, obs_bits=bits[:T], obs_size=env._obs_size)
+                       advantages=adv, returns=ret, twist=st["twist"][:T] if twisted else None, obs_bits=bits[:T], obs_size=env._obs_size)
 
     def collect(self, num_steps: int, deterministic: bool = False) -> Rollout:
         env, T, B = self.env, int(num_steps), self.env.batch

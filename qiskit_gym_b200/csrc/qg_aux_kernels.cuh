@@ -95,4 +95,34 @@ __global__ void k_twist_gather(const float* __restrict__ in, float* __restrict__
     }
 }
 
+// Twists on packed observations (qg_twist_bits).  Every obs perm of a Permutation / LinearFunction / Clifford twist is the lift of a qubit
+// permutation p: entry (r, c) of the d x d observation (d = n or 2n) moves to (lift(r), lift(c)), lift(i) = p[i] for i < n, n + p[i - n]
+// otherwise (qg_host.cpp compute_twists).  qpinv[k] = p^-1 of twist k, so output entry (R, C) is input entry (lift^-1(R), lift^-1(C)) —
+// qg_twist_gather with the inverse obs perm, on bits, from a [K][n] byte table instead of a [K][d*d] index table.
+// Thread = (env, output word).  Twist index: kidx_in[b], or drawn  mulhi(philox(*seed_dev, first + b, draw, STREAM_TWIST), K)  (the seed
+// is read at run time, so the launch can live in a CUDA graph); written to kidx_out[b] when given.
+__global__ void k_twist_bits(const uint32_t* __restrict__ in, uint32_t* __restrict__ out, int ow, int obs_size, int n, int d,
+                             const uint8_t* __restrict__ qpinv, uint32_t K, const int32_t* __restrict__ kidx_in, const uint64_t* __restrict__ seed_dev,
+                             int64_t first, uint32_t draw, int32_t* __restrict__ kidx_out, int64_t B) {
+    const int64_t total = B * (int64_t)ow;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t b = i / ow;
+        const int w = (int)(i - b * ow);
+        const uint32_t k = kidx_in ? (uint32_t)kidx_in[b] : __umulhi(philox_draw(*seed_dev, (uint64_t)(first + b), draw, STREAM_TWIST), K);
+        if (kidx_out && w == 0) kidx_out[b] = (int32_t)k;
+        const uint8_t* const pk = qpinv + (size_t)k * n;
+        const uint32_t* const row = in + (size_t)b * ow;
+        int j = w * 32, R = j / d, Cc = j - R * d;
+        uint32_t acc = 0;
+        for (int bit = 0; bit < 32 && j < obs_size; ++bit, ++j) {
+            const int sr = R < n ? (int)__ldg(pk + R) : n + (int)__ldg(pk + R - n);
+            const int sc = Cc < n ? (int)__ldg(pk + Cc) : n + (int)__ldg(pk + Cc - n);
+            const int s = sr * d + sc;
+            acc |= ((__ldg(row + (s >> 5)) >> (s & 31)) & 1u) << bit;
+            if (++Cc == d) { Cc = 0; ++R; }
+        }
+        out[i] = acc;
+    }
+}
+
 }  // namespace qg

@@ -36,8 +36,8 @@ enum { FL_SUCCESS = 1u, FL_INVERTED = 2u, FL_ERR_SHIFT = 8, FL_LEN_SHIFT = 16 };
 enum { PX_PLO = 0, PX_PHI = 1, PX_ALIVE = 2, PX_ORD0 = 3, PX_ORD1 = 4, PX_MISC = 5, PX_ANTI = 6 };
 // PX_MISC: bits 0..15 current_perm_idx, bits 16..23 rotations loaded (R), bits 24..31 live DAG nodes (m)
 
-// Philox stream ids (shared with oracle/qg_oracle.hpp)
-enum : uint32_t { STREAM_RESET = 1, STREAM_COIN = 2, STREAM_PERM = 3, STREAM_SAMPLE = 4 };
+// Philox stream ids (1..4 shared with oracle/qg_oracle.hpp; STREAM_TWIST: the collector's per-env twist pick, qg_twist_bits)
+enum : uint32_t { STREAM_RESET = 1, STREAM_COIN = 2, STREAM_PERM = 3, STREAM_SAMPLE = 4, STREAM_TWIST = 5 };
 
 constexpr int kThreads = 256;          // threads per CTA of the step kernels
 constexpr int kMaxRot = 16;            // rotations per PauliNetwork env (nibble-coded DAG order)

@@ -752,6 +752,19 @@ int qg_collect_step_dev(qg_engine* e, const uint64_t* seed_dev, const float* wei
     return rc;
 }
 
+int qg_collect_step_twisted_dev(qg_engine* e, const uint64_t* seed_dev, const float* weights_dev, const int32_t* act_perm_dev, const int32_t* twist_dev,
+                                int32_t deterministic, int32_t* chosen_dev, int32_t* policy_chosen_dev, float* reward_dev, uint8_t* done_dev,
+                                uint8_t* success_dev, qg_stream stream) {
+    if (!e || !weights_dev || !seed_dev || !act_perm_dev || !twist_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    e->dc.seed_dev = seed_dev;
+    StepArgs a{}; a.weights = weights_dev; a.deterministic = deterministic; a.chosen = chosen_dev;
+    a.act_perm = act_perm_dev; a.twist = twist_dev; a.policy_chosen = policy_chosen_dev;
+    a.reward = reward_dev; a.done = done_dev; a.success = success_dev;
+    const int rc = launch_step(e, MODE_SEARCH, a, (cudaStream_t)stream);
+    e->dc.seed_dev = nullptr;
+    return rc;
+}
+
 int qg_gae(const float* reward_dev, const float* value_dev, const uint8_t* done_dev, const uint8_t* valid_dev, int32_t num_steps, int64_t batch,
            float gamma, float lambda, float* adv_dev, float* ret_dev, qg_stream stream) {
     if (!reward_dev || !value_dev || !done_dev || !adv_dev) { set_error("null argument"); return QG_ERR_INVALID; }
@@ -771,6 +784,25 @@ int qg_twist_gather(const float* in_dev, float* out_dev, const int32_t* table_de
     const int64_t total = batch * (int64_t)len;
     const unsigned grid = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16);
     k_twist_gather<<<grid, 256, 0, (cudaStream_t)stream>>>(in_dev, out_dev, table_dev, index_dev, batch, len, magic);
+    CUDA_OK(cudaGetLastError());
+    return QG_OK;
+}
+
+int qg_twist_bits(const uint32_t* in_bits_dev, uint32_t* out_bits_dev, int64_t batch, int32_t obs_size, int32_t num_qubits, int32_t dim,
+                  const uint8_t* qperm_inv_dev, int32_t num_twists, const int32_t* index_dev, const uint64_t* seed_dev, int64_t first_env_id,
+                  int32_t draw, int32_t* index_out_dev, qg_stream stream) {
+    if (!in_bits_dev || !out_bits_dev || !qperm_inv_dev || (!index_dev && !seed_dev)) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (in_bits_dev == out_bits_dev) { set_error("qg_twist_bits cannot run in place"); return QG_ERR_INVALID; }
+    if (batch < 0 || num_qubits < 1 || num_twists < 1 || draw < 0 || (dim != num_qubits && dim != 2 * num_qubits) || obs_size != dim * dim) {
+        set_error("qg_twist_bits: bad size (obs_size must be dim * dim with dim = num_qubits or 2 * num_qubits)");
+        return QG_ERR_INVALID;
+    }
+    if (batch == 0) return QG_OK;
+    const int ow = (obs_size + 31) / 32;
+    const int64_t total = batch * (int64_t)ow;
+    const unsigned grid = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16);
+    k_twist_bits<<<grid, 256, 0, (cudaStream_t)stream>>>(in_bits_dev, out_bits_dev, ow, obs_size, num_qubits, dim, qperm_inv_dev, (uint32_t)num_twists,
+                                                         index_dev, seed_dev, first_env_id, (uint32_t)draw, index_out_dev, batch);
     CUDA_OK(cudaGetLastError());
     return QG_OK;
 }

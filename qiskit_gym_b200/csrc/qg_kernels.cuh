@@ -34,6 +34,9 @@ struct StepArgs {
     uint8_t* mask;               // [B][A] or null
     float* reward; uint8_t* done; uint8_t* success;   // [B] or null
     int32_t* chosen;             // [B] or null    (MODE_SEARCH)
+    const int32_t* act_perm;     // [K][A] or null (MODE_SEARCH, twisted collector): `weights` are in the policy's (twisted) action order and env
+    const int32_t* twist;        // [B]              action g reads weights[act_perm[twist[env]][g]]  (qg_collect_step_twisted_dev)
+    int32_t* policy_chosen;      // [B] or null    (MODE_SEARCH) the chosen action in the weights' order, act_perm[twist[env]][chosen]; -1: not stepped
     int32_t* num_active;         // [1] or null    (MODE_SEARCH)
     int32_t nsteps;              // steps played by this launch (MODE_STEP; 1 otherwise)
     int32_t ring;                // obs / mask hold `ring` step slots of [B][obs_size] / [B][A]; step t writes slot (slot0 + t) % ring
@@ -751,7 +754,8 @@ __device__ __forceinline__ void wait_input_chunk(const StepArgs& a, int step, in
 // EPW: environments per warp tile (32, or 16: twice the warps for the same batch, lanes 16..31 idle in phase 1 and at work in phase 2 —
 // at 65 536 environments that is 28 instead of 14 warps per SM to overlap one warp's latency-bound step logic with the others' stores).
 // The tile's shared-memory words are laid out [word][EPW + 1].
-template <int KIND, int MODE, int INV, int EPW = 32, int ROLE = 0>
+// TWIST: the launch may carry a twisted collector's action tables (a.act_perm); the fused search never does and compiles without that path.
+template <int KIND, int MODE, int INV, int EPW = 32, int ROLE = 0, bool TWIST = true>
 __device__ __forceinline__ uint32_t step_tile(const DevCfg& c, const StepArgs& a, uint32_t* const wbase, const uint32_t* const lut, const int lane,
                                               const int64_t e0, const int cnt, const bool resident = false, const float* const weights_tile = nullptr,
                                               const bool fused = false, float* const ret_local = nullptr) {
@@ -869,27 +873,37 @@ __device__ __forceinline__ uint32_t step_tile(const DevCfg& c, const StepArgs& a
             if (MODE == MODE_SEARCH) {
                 // twisterl-style rollout decision: skip rollouts that are final (is_final, clifford.rs:353)
                 enabled = !(depth == 0 || success);
+                // twisted collector: env action g's weight is wt[ap[g]] (the policy saw the twisted observation).  The arg-max and the sequential
+                // inverse-CDF sum run over g in the same order as on the result of qg_twist_gather(weights, act_perm, twist): bit-identical picks
+                const int32_t* const ap = (TWIST && a.act_perm && enabled) ? a.act_perm + (size_t)a.twist[env] * c.A : nullptr;
                 if (enabled) {
                     const float* wt = weights_tile ? weights_tile + (size_t)lane * c.A
                                       : (staged_wts ? staged_wts + (size_t)lane * (c.A | 1) : a.weights + (size_t)env * c.A);
-                    if (a.deterministic) {
-                        float best = wt[0]; action = 0;
-                        for (int k = 1; k < c.A; ++k) { const float v = wt[k]; if (v > best) { best = v; action = k; } }
-                    } else {
-                        float total = 0.0f;
+                    auto pick = [&](auto w_at) {
+                        int act;
+                        if (a.deterministic) {
+                            float best = w_at(0); act = 0;
+                            for (int k = 1; k < c.A; ++k) { const float v = w_at(k); if (v > best) { best = v; act = k; } }
+                        } else {
+                            float total = 0.0f;
 #pragma unroll 4
-                        for (int k = 0; k < c.A; ++k) total = __fadd_rn(total, wt[k]);
-                        const uint32_t raw = philox_draw(seed_of(c), (uint64_t)(c.first_id + env), tick, STREAM_SAMPLE);
-                        if (!(total > 0.0f)) action = (int)__umulhi(raw, (uint32_t)c.A);
-                        else {
-                            const float target = __fmul_rn((float)(raw >> 8) * (1.0f / 16777216.0f), total);
-                            float cum = 0.0f; action = c.A - 1;
+                            for (int k = 0; k < c.A; ++k) total = __fadd_rn(total, w_at(k));
+                            const uint32_t raw = philox_draw(seed_of(c), (uint64_t)(c.first_id + env), tick, STREAM_SAMPLE);
+                            if (!(total > 0.0f)) act = (int)__umulhi(raw, (uint32_t)c.A);
+                            else {
+                                const float target = __fmul_rn((float)(raw >> 8) * (1.0f / 16777216.0f), total);
+                                float cum = 0.0f; act = c.A - 1;
 #pragma unroll 4
-                            for (int k = 0; k < c.A; ++k) { cum = __fadd_rn(cum, wt[k]); if (cum > target) { action = k; break; } }
+                                for (int k = 0; k < c.A; ++k) { cum = __fadd_rn(cum, w_at(k)); if (cum > target) { act = k; break; } }
+                            }
                         }
-                    }
+                        return act;
+                    };
+                    if constexpr (TWIST) { if (ap) action = pick([&](int k) { return wt[__ldg(ap + k)]; }); else action = pick([&](int k) { return wt[k]; }); }
+                    else action = pick([&](int k) { return wt[k]; });
                 }
                 if (a.chosen) a.chosen[env] = enabled ? action : -1;
+                if constexpr (TWIST) { if (a.policy_chosen) a.policy_chosen[env] = enabled ? (ap ? __ldg(ap + action) : action) : -1; }
             }
 
             int oh_q0 = -1, oh_q1 = -1;                 // Permutation, fused + resident: the SWAP this step played (one-hot stream patch)

@@ -798,6 +798,26 @@ __global__ void k_tc_expand_bits(const uint32_t* __restrict__ bits, int obs_word
     reinterpret_cast<uint4*>(X)[i] = o;       // image order [mt][kb][ch][row] x 16 bytes == i
 }
 
+// in-place weight refresh (qg_policy_tc_load_weights_dev): f32 weights [rows][K] (row `rows` = the value head's when vw is set) -> the
+// [term][n_tile][kb][k/8][n][k%8] hi / lo images qg_policy_tc_create lays out on the host, same split; bias[n] alongside (when bias is set).
+// Padding rows / columns are not touched: they stay the zeros of creation.  Thread = (row, k), so the f32 rows are read coalesced
+__global__ void k_tc_load_layer(const float* __restrict__ W, const float* __restrict__ b, const float* __restrict__ vw, const float* __restrict__ vb,
+                                int rows, int K, int NT, int n_tiles, int Kb, __half* __restrict__ img, float* __restrict__ bias) {
+    const int nrows = rows + (vw ? 1 : 0);
+    const long long total = (long long)nrows * K, term = (long long)n_tiles * Kb * NT * kKB;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int n = (int)(i / K), k = (int)(i - (long long)n * K);
+        const bool vrow = n == rows;
+        const float w = vrow ? vw[k] : W[i];
+        const __half hi = __float2half_rn(w), lo = __float2half_rn(w - __half2float(hi));
+        const int nt = n / NT, nl = n - nt * NT, kb = k / kKB, kl = k - kb * kKB;
+        const long long at = ((long long)nt * Kb + kb) * NT * kKB + ((long long)(kl >> 3) * NT + nl) * 8 + (kl & 7);
+        img[at] = hi;
+        img[term + at] = lo;
+        if (bias && k == 0) bias[n] = vrow ? *vb : b[n];
+    }
+}
+
 }  // namespace tc
 }  // namespace qg
 
@@ -942,6 +962,39 @@ int qg_policy_tc_create(int32_t device, int32_t obs_size, int32_t num_layers, co
         p->fused = true;
     }
     *out = p;
+    return QG_OK;
+}
+
+int qg_policy_tc_load_weights_dev(qg_policy_tc* p, int32_t obs_size, int32_t num_layers, const int32_t* out_features, const float* const* weights_dev,
+                                  const float* const* biases_dev, const float* value_weight_dev, const float* value_bias_dev, qg_stream stream) {
+    if (!p || !out_features || !weights_dev || !biases_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (obs_size != p->obs_size || num_layers != (int)p->layers.size()) { set_error("qg_policy_tc_load_weights_dev: shapes differ from creation"); return QG_ERR_INVALID; }
+    if ((value_weight_dev != nullptr) != (p->has_value != 0) || (value_weight_dev && !value_bias_dev)) {
+        set_error("qg_policy_tc_load_weights_dev: the value head must be given exactly when the handle was created with one");
+        return QG_ERR_INVALID;
+    }
+    for (int l = 0; l < num_layers; ++l) {
+        const TcLayer& L = p->layers[l];
+        const int rows = L.N - ((l == num_layers - 1) ? p->has_value : 0);
+        if (out_features[l] != rows || !weights_dev[l] || !biases_dev[l]) { set_error("qg_policy_tc_load_weights_dev: shapes differ from creation"); return QG_ERR_INVALID; }
+    }
+    TC_CUDA_OK(cudaSetDevice(p->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    auto grid_for = [&](long long total) { return (unsigned)std::min<long long>((total + 255) / 256, (long long)p->num_sms * 8); };
+    for (int l = 0; l < num_layers; ++l) {
+        const TcLayer& L = p->layers[l];
+        const bool last = l == num_layers - 1;
+        const float* vw = (last && p->has_value) ? value_weight_dev : nullptr;
+        tc::k_tc_load_layer<<<grid_for((long long)L.N * L.K), 256, 0, st>>>(weights_dev[l], biases_dev[l], vw, value_bias_dev, out_features[l], L.K, L.NT,
+                                                                         L.n_tiles, L.Kb, L.W, L.bias);
+        TC_CUDA_OK(cudaGetLastError());
+    }
+    if (p->W2_fused) {          // the fused kernel's copy of layer 2: all C_pad rows in one tile
+        const TcLayer& L1 = p->layers[1];
+        tc::k_tc_load_layer<<<grid_for((long long)out_features[1] * L1.K), 256, 0, st>>>(weights_dev[1], nullptr, nullptr, nullptr, out_features[1], L1.K,
+                                                                                       L1.Npad, 1, L1.Kb, p->W2_fused, nullptr);
+        TC_CUDA_OK(cudaGetLastError());
+    }
     return QG_OK;
 }
 

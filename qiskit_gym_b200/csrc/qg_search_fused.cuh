@@ -46,7 +46,7 @@ __global__ void __launch_bounds__(kPolThreads) k_search_fused(const __grid_const
         __syncthreads();
         { QG_SP_T0();
         if (warp == 0) {
-            const uint32_t en = step_tile<KIND, MODE_SEARCH, 0>(c, a, wbase, nullptr, lane, row0, cnt, it > 0, s_probs, true, s_ret);
+            const uint32_t en = step_tile<KIND, MODE_SEARCH, 0, 32, 0, false>(c, a, wbase, nullptr, lane, row0, cnt, it > 0, s_probs, true, s_ret);
             if (lane == 0) s_active = en;
         }
         __syncthreads();                           // next observations in the step's stream, s_active set

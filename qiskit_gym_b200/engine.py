@@ -139,6 +139,20 @@ class BatchedEnv:
                                         _dptr(self.reward if reward is None else reward), _dptr(self.done if done is None else done),
                                         _dptr(self.success if success is None else success), self._stream()))
 
+    def collect_step_twisted_dev(self, weights: torch.Tensor, act_table: torch.Tensor, twist: torch.Tensor, seed_dev: torch.Tensor,
+                                 deterministic: bool = False, chosen: torch.Tensor | None = None, policy_chosen: torch.Tensor | None = None,
+                                 reward: torch.Tensor | None = None, done: torch.Tensor | None = None, success: torch.Tensor | None = None):
+        """collect_step_dev for a twisted collector (qg_collect_step_twisted_dev): `weights` [B, A] are in the policy's twisted action order,
+        env action g of env i takes weights[i, act_table[twist[i], g]]; `policy_chosen` receives act_table[twist[i], chosen] (-1: not stepped)."""
+        assert weights.dtype == torch.float32 and weights.is_cuda and weights.is_contiguous() and seed_dev.is_cuda and seed_dev.element_size() == 8
+        assert act_table.dtype == torch.int32 and act_table.is_contiguous() and act_table.shape[1] == self._A
+        assert twist.dtype == torch.int32 and twist.is_contiguous() and twist.numel() == self.batch
+        assert policy_chosen is None or (policy_chosen.dtype == torch.int32 and policy_chosen.numel() == self.batch)
+        check(lib().qg_collect_step_twisted_dev(self._h, _dptr(seed_dev), _dptr(weights), _dptr(act_table), _dptr(twist), 1 if deterministic else 0,
+                                                _dptr(chosen), _dptr(policy_chosen), _dptr(self.reward if reward is None else reward),
+                                                _dptr(self.done if done is None else done), _dptr(self.success if success is None else success),
+                                                self._stream()))
+
     def reset_select(self, seed: int = 0, first_env_id: int = 0, select: torch.Tensor | None = None):
         """Env::reset for the envs flagged in `select` (bool/uint8 [B]) or, with select=None, for every env that is final."""
         assert select is None or (select.is_cuda and select.numel() == self.batch and select.element_size() == 1)

@@ -136,6 +136,46 @@ class TensorCorePolicy:
         h = C.c_void_p()
         check(lib().qg_policy_tc_create(self.device_index, self.obs_size, n, widths, wp, bp, vw, C.c_float(vb), self.max_batch, C.byref(h)))
         self._h = h
+        self.out_features = [int(w.shape[0]) for w in ws]
+
+    def _device_params(self, policy: torch.nn.Module):
+        """The module's action-path weights / biases (and value head) when they can be read in place: f32, contiguous, on this device, with the
+        shapes of creation; else None."""
+        layers = action_layers(policy)
+        if len(layers) != len(self.out_features) or int(layers[0].in_features) != self.obs_size:
+            return None
+        if [int(l.out_features) for l in layers] != self.out_features:
+            return None
+        ts = [l.weight for l in layers] + [l.bias for l in layers]
+        head = simple_value_head(policy) if self.has_value else None
+        if self.has_value:
+            if head is None:
+                return None
+            ts += [head.weight, head.bias]
+        if any(t is None or t.device != self.device or t.dtype != torch.float32 or not t.is_contiguous() for t in ts):
+            return None
+        return layers, head
+
+    def can_load(self, policy: torch.nn.Module) -> bool:
+        """Whether load_weights(policy) applies (same shapes, parameters f32 / contiguous on this device)."""
+        return self._device_params(policy) is not None
+
+    def load_weights(self, policy: torch.nn.Module) -> None:
+        """Refreshes the handle's weights in place from the module's device parameters (qg_policy_tc_load_weights_dev): stream-ordered on the
+        current stream, no allocation, no host round trip; CUDA graphs captured with this handle stay valid and replay the new weights."""
+        got = self._device_params(policy)
+        if got is None:
+            raise ValueError("load_weights needs a module with the shapes of creation whose parameters are f32, contiguous and on " + str(self.device))
+        layers, head = got
+        n = len(layers)
+        widths = (C.c_int32 * n)(*self.out_features)
+        wp = (C.c_void_p * n)(*[l.weight.data_ptr() for l in layers])
+        bp = (C.c_void_p * n)(*[l.bias.data_ptr() for l in layers])
+        vw = C.c_void_p(head.weight.data_ptr()) if head is not None else None
+        vb = C.c_void_p(head.bias.data_ptr()) if head is not None else None
+        st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        check(lib().qg_policy_tc_load_weights_dev(self._h, self.obs_size, n, widths, wp, bp, vw, vb, st))
+        self.version = weights_version(policy)
 
     def __del__(self):
         h = getattr(self, "_h", None)

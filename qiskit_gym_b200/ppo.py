@@ -26,7 +26,7 @@ import time
 
 import torch
 
-from .collector import RolloutCollector, decision_seed
+from .collector import RolloutCollector, decision_seed, unpack_bits
 from .engine import BatchedEnv
 
 _EVAL_DEFAULT = {"num_episodes": 100, "deterministic": True, "num_searches": 1, "num_mcts_searches": 0, "num_cores": 32, "C": 1.41}
@@ -296,13 +296,23 @@ class PPO(Trainer):
 
     def __init__(self, env_kind: int, num_qubits: int, gateset, policy: torch.nn.Module, config: dict | None = None, device=None,
                  seed: int = 0, use_twists: bool = True, minibatch_size: int | None = None, matmul_precision: str = "f32", **env_kwargs):
+        """matmul_precision: "f32" (default), "tf32" or "bf16" run the policy in PyTorch on dense observations (RolloutCollector.collect);
+        "tensor_core" collects with packed-bit observations and the tcgen05 policy (RolloutCollector.collect_packed, twists included) and
+        the update unpacks each minibatch's observations from the bits.  "tensor_core" raises NotImplementedError where that path cannot run
+        (more than 127 actions, a value head that is not one Linear, a device that is not sm_100)."""
+        if matmul_precision not in ("f32", "tf32", "bf16", "tensor_core"):
+            raise ValueError(f"matmul_precision must be one of f32, tf32, bf16, tensor_core (got {matmul_precision!r})")
         super().__init__(env_kind, num_qubits, gateset, policy, config, device=device, seed=seed, minibatch_size=minibatch_size, **env_kwargs)
+        self.tensor_core = matmul_precision == "tensor_core"
         self.collector = RolloutCollector(self.env, self.policy, gamma=self.cfg["collecting"]["gamma"], lam=self.cfg["collecting"]["lambda"],
                                           use_twists=use_twists, seed=seed + 104729 * self.rank, first_env_id=self.rank * self.env.batch,
-                                          matmul_precision=matmul_precision)
+                                          matmul_precision="f32" if self.tensor_core else matmul_precision)
+        if self.tensor_core:
+            self.collector.tensor_core_policy()          # fails here, not in the first iteration, where the tensor-core policy cannot run
 
     def iterate(self) -> dict:
-        ro = self.collector.collect(self._episode_steps())
+        steps = self._episode_steps()
+        ro = self.collector.collect_packed(steps) if self.tensor_core else self.collector.collect(steps)
         episodes, success = ro.episode_stats()
         rec = {"episodes": episodes, "collect_success": success,
                "mean_reward": float(ro.rewards[ro.valid].mean().item()) if bool(ro.valid.any()) else 0.0}
@@ -313,7 +323,13 @@ class PPO(Trainer):
         """`num_epochs` passes of the clipped-surrogate update over the valid decisions of a Rollout."""
         t = self.cfg["training"]
         idx = ro.valid.reshape(-1).nonzero(as_tuple=False).squeeze(1)
-        obs = ro.obs.reshape((-1,) + tuple(ro.obs.shape[2:]))[idx]
+        if ro.obs is None:          # packed rollout: keep the gathered bits (32x smaller) and unpack one minibatch at a time
+            bits = ro.obs_bits.reshape(-1, ro.obs_bits.shape[-1])[idx]
+            shape = tuple(self.env.obs_shape())
+            obs_of = lambda sel: unpack_bits(bits[sel], ro.obs_size).reshape((-1,) + shape)      # noqa: E731
+        else:
+            obs = ro.obs.reshape((-1,) + tuple(ro.obs.shape[2:]))[idx]
+            obs_of = lambda sel: obs[sel]                                                         # noqa: E731
         act = ro.policy_actions.reshape(-1)[idx]
         logp_old = ro.logp.reshape(-1)[idx]
         adv = ro.advantages.reshape(-1)[idx]
@@ -326,7 +342,7 @@ class PPO(Trainer):
         stats = {}
         for _ in range(int(t["num_epochs"])):
             for sel in self._minibatches(n):
-                logits, value = self.policy(obs[sel])
+                logits, value = self.policy(obs_of(sel))
                 logp_all = torch.log_softmax(logits.float(), dim=-1)
                 logp = logp_all.gather(1, act[sel][:, None]).squeeze(1)
                 ratio = torch.exp(logp - logp_old[sel])
