@@ -105,7 +105,10 @@ class FusedPolicy:
 
 class TensorCorePolicy:
     """The same network for large batches on tcgen05 tensor cores (`qg_policy_tc_*`, csrc/qg_policy_tc.cu): packed observation bits in,
-    softmax action weights / logits / values out; f16 hi+lo split operands with f32 accumulation (logits within 1e-4 of the f32 module)."""
+    softmax action weights / logits / values out; f16 hi+lo split operands with f32 accumulation.
+    Error contract (u = 2^-24, M = the forward pass on |W|, |b|, |x| without ReLU): logits and values within u (4 M + F) of a float64
+    emulation of the split arithmetic, F the inputs whose lo half is an f16 subnormal (0 < h < 2^-3) forward-propagated through |W|; against
+    the float64 module add the propagated split error (|v - hi - lo| <= 2^-22 |v| + 2^-25).  tests/test_policy_tc_envelope.py derives both."""
 
     def __init__(self, policy: torch.nn.Module, max_batch: int, device=None, with_value: bool = True):
         if not torch.cuda.is_available():

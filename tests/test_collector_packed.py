@@ -160,55 +160,57 @@ def test_twisted_collect_step_matches_gather(name, deterministic):
     assert stepped > B
 
 
-def reenact(ro, spec, tcp, act_perms, obs_perms, seed, first, T, B, gamma, lam):
-    """The rollout re-enacted with the oracle: resets, (twisted) observations, samples from the recomputed tensor-core probabilities, rewards, GAE."""
+def reenact(ro, spec, tcp, act_perms, obs_perms, seed, first, T, B, gamma, lam, rows=None):
+    """The rollout re-enacted with the oracle: resets, (twisted) observations, samples from the recomputed tensor-core probabilities, rewards, GAE.
+    rows: re-enact only these envs (envs are independent by (seed, env id)); all B by default."""
     from qiskit_gym_b200.collector import decision_seed
     kind, n, gs, ekw = spec
-    refs = [orc.OracleEnv(kind, n, gs, **ekw) for _ in range(B)]
-    ticks = np.zeros(B, np.int64)
-    acts, pacts = ro.actions.cpu().numpy(), ro.policy_actions.cpu().numpy()
-    rew, dones, succ = ro.rewards.cpu().numpy(), ro.dones.cpu().numpy(), ro.successes.cpu().numpy()
-    obs = ro.unpack_obs().cpu().numpy()
+    rows = list(range(B)) if rows is None else [int(b) for b in rows]
+    refs = [orc.OracleEnv(kind, n, gs, **ekw) for _ in rows]
+    ticks = np.zeros(len(rows), np.int64)
+    acts, pacts = ro.actions.cpu().numpy()[:, rows], ro.policy_actions.cpu().numpy()[:, rows]
+    rew, dones, succ = ro.rewards.cpu().numpy()[:, rows], ro.dones.cpu().numpy()[:, rows], ro.successes.cpu().numpy()[:, rows]
+    obs = ro.unpack_obs().cpu().numpy()[:, rows]
     size = obs.shape[-1]
-    tw = None if ro.twist is None else ro.twist.cpu().numpy()
+    tw = None if ro.twist is None else ro.twist.cpu().numpy()[:, rows]
     K = len(obs_perms) if obs_perms is not None else 1
     n_resets = 0
     for t in range(T):
         s = decision_seed(seed, t)
-        probs = tcp.forward_bits(ro.obs_bits[t].contiguous()).cpu().numpy()
-        for b, r in enumerate(refs):
+        probs = tcp.forward_bits(ro.obs_bits[t].contiguous()).cpu().numpy()[rows]
+        for i, (b, r) in enumerate(zip(rows, refs)):
             if r.is_final():
                 r.reset(seed=s, env_id=first + b)
-                ticks[b] = 0
+                ticks[i] = 0
                 n_resets += 1
             want = dense(r.observe(), size)
             if tw is not None:
-                k = int(tw[t, b])
+                k = int(tw[t, i])
                 assert k == mulhi(orc.philox_draw(s, first + b, 0, STREAM_TWIST), K)
                 tmp = np.zeros(size, np.float32)
                 tmp[np.asarray(obs_perms[k])] = want
                 want = tmp
-            assert np.array_equal(obs[t, b], want), (t, b)
+            assert np.array_equal(obs[t, i], want), (t, b)
             if r.is_final():
-                assert acts[t, b] == -1
+                assert acts[t, i] == -1
                 continue
-            w = probs[b] if tw is None else probs[b][np.asarray(act_perms[int(tw[t, b])])]
-            a = cpu_pick(w, orc.philox_draw(s, first + b, int(ticks[b]), STREAM_SAMPLE), False)
-            assert acts[t, b] == a, (t, b)
-            assert pacts[t, b] == (a if tw is None else act_perms[int(tw[t, b])][a])
+            w = probs[i] if tw is None else probs[i][np.asarray(act_perms[int(tw[t, i])])]
+            a = cpu_pick(w, orc.philox_draw(s, first + b, int(ticks[i]), STREAM_SAMPLE), False)
+            assert acts[t, i] == a, (t, b)
+            assert pacts[t, i] == (a if tw is None else act_perms[int(tw[t, i])][a])
             r.step(a)
-            ticks[b] += 1
-            assert np.float32(r.reward()).view(np.uint32) == rew[t, b].view(np.uint32)
-            assert bool(dones[t, b]) == r.is_final() and bool(succ[t, b]) == r.success()
-    assert n_resets > B
+            ticks[i] += 1
+            assert np.float32(r.reward()).view(np.uint32) == rew[t, i].view(np.uint32)
+            assert bool(dones[t, i]) == r.is_final() and bool(succ[t, i]) == r.success()
+    assert n_resets > len(rows) if len(rows) == B else n_resets >= len(rows)
     valid = acts >= 0
-    assert np.array_equal(ro.valid.cpu().numpy(), valid)
-    ra, rr = cpu_gae(rew, ro.values.cpu().numpy(), dones, valid, gamma, lam)
-    assert np.array_equal(ro.advantages.cpu().numpy().view(np.uint32), ra.view(np.uint32))
-    assert np.array_equal(ro.returns.cpu().numpy().view(np.uint32), rr.view(np.uint32))
-    lp = np.log(np.take_along_axis(np.stack([tcp.forward_bits(ro.obs_bits[t].contiguous()).cpu().numpy() for t in range(T)]),
+    assert np.array_equal(ro.valid.cpu().numpy()[:, rows], valid)
+    ra, rr = cpu_gae(rew, ro.values.cpu().numpy()[:, rows], dones, valid, gamma, lam)
+    assert np.array_equal(ro.advantages.cpu().numpy()[:, rows].view(np.uint32), ra.view(np.uint32))
+    assert np.array_equal(ro.returns.cpu().numpy()[:, rows].view(np.uint32), rr.view(np.uint32))
+    lp = np.log(np.take_along_axis(np.stack([tcp.forward_bits(ro.obs_bits[t].contiguous()).cpu().numpy()[rows] for t in range(T)]),
                                    np.maximum(pacts, 0)[..., None].astype(np.int64), axis=2)[..., 0])
-    assert np.allclose(ro.logp.cpu().numpy()[valid], lp[valid], rtol=1e-5, atol=1e-6)
+    assert np.allclose(ro.logp.cpu().numpy()[:, rows][valid], lp[valid], rtol=1e-5, atol=1e-6)
 
 
 def rollout_fields(ro):
