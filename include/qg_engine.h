@@ -389,6 +389,17 @@ QG_API int qg_policy_tc_forward_bits(qg_policy_tc* p, const uint32_t* obs_bits_d
 QG_API int qg_policy_tc_load_weights_dev(qg_policy_tc* p, int32_t obs_size, int32_t num_layers, const int32_t* out_features,
                                          const float* const* weights_dev, const float* const* biases_dev,
                                          const float* value_weight_dev, const float* value_bias_dev, qg_stream stream);
+/* Training on the tensor cores.  enable_training allocates, once, what the backward pass needs for up to max_batch rows (dZ images of every
+ * layer, transposed weight images, split-K partials); later weight loads keep them current.  generation() counts forwards.  backward
+ * differentiates the handle's latest forward, which must have run one kernel per layer (qg_policy_tc_set_mode(p, 1)) with `batch` rows and
+ * have been generation `generation` (QG_ERR_INVALID otherwise): dlogits_dev float[batch][num_actions], dvalues_dev float[batch] (NULL = 0)
+ * -> grad_w_dev[l] float[out][in], grad_b_dev[l] float[out], grad_vw_dev float[in of the last layer], grad_vb_dev float[1], OVERWRITTEN.
+ * Same split-f16 arithmetic as the forward; the head's gradient is scaled by a power of two chosen on the device; weight gradients are
+ * summed over 1024-row chunks and the chunks in a fixed order, so they are bit-reproducible.  Stream-ordered, allocates nothing. */
+QG_API int qg_policy_tc_enable_training(qg_policy_tc* p);
+QG_API int64_t qg_policy_tc_generation(const qg_policy_tc* p);
+QG_API int qg_policy_tc_backward(qg_policy_tc* p, int64_t generation, int64_t batch, const float* dlogits_dev, const float* dvalues_dev,
+                                 float* const* grad_w_dev, float* const* grad_b_dev, float* grad_vw_dev, float* grad_vb_dev, qg_stream stream);
 
 /* The whole rollout search in ONE launch: every CTA owns 8 rollouts and loops  policy (packed observation -> action weights) ->
  * sample / arg-max + fused step -> next packed observation  until its rollouts are final or max_decisions decisions were taken;

@@ -126,6 +126,9 @@ struct LayerArgs {
     float* logits; float* probs; float* values;      // last layer outputs (each may be null)
     int a_terms, Kb, NT, n_tiles, m_tiles, out_Kb, relu, num_actions, has_value, stages;
     long long batch;
+    // dgrad (k_tc_layer<1>): Y = mask(X W) 2^(sexp[s_out] - sexp[s_in]); mask = the ReLU mask read from the images of the layer input,
+    // [m_tiles][mask_Kb][2][8][128][8] (an entry is kept where its hi or lo half is non-zero)
+    const __half* mask; const int* sexp; int s_in, s_out, mask_Kb;
 };
 
 struct SmemPlan { uint32_t a_off[kStages][2], b_off[kStages][2], bar_off, stage_off, total; };
@@ -145,6 +148,9 @@ __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepc
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;\n" ::: "memory"); }
 __device__ __forceinline__ void epilogue_sync() { asm volatile("bar.sync 1, 128;\n" ::: "memory"); }      // the 4 epilogue warps
 
+// kMode 0: the forward layer.  kMode 1: the dgrad of the backward pass (qg_policy_tc_backward): X = the layer's dZ images, W = its transposed
+// weight images, the epilogue applies the ReLU mask of the layer's input and the power-of-two rescale instead of bias / ReLU
+template <int kMode>
 __global__ void __launch_bounds__(kThreads, 1) k_tc_layer(const __grid_constant__ LayerArgs a) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const SmemPlan sp = plan_smem(a.a_terms, a.NT, a.stages, a.Y ? 0 : kM * a.num_actions);
@@ -234,7 +240,36 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_layer(const __grid_constant_
             tc_fence_after();
             const uint32_t taddr = tmem_base + as * acc_cols + ((uint32_t)(q * 32) << 16);
             const long long grow = (long long)mt * kM + row;
-            if (a.Y) {
+            if constexpr (kMode == 1) {
+                const float f = ldexpf(1.0f, __ldg(a.sexp + a.s_out) - __ldg(a.sexp + a.s_in));
+                for (int c0 = 0; c0 < a.NT; c0 += 16) {
+                    uint32_t v[16];
+                    tmem_ld16(taddr + (uint32_t)c0, v);
+                    const int n0 = nt * a.NT + c0;
+                    const int okb = n0 >> 6, ch = (n0 & 63) >> 3;
+                    const size_t at = ((size_t)ch * kM + row) * 8;
+                    const __half* mimg = a.mask + (((size_t)mt * a.mask_Kb + okb) * 2) * kImgA;
+                    const uint4* m_hi = reinterpret_cast<const uint4*>(mimg + at);
+                    const uint4* m_lo = reinterpret_cast<const uint4*>(mimg + kImgA + at);
+                    const uint4 h0 = m_hi[0], h1 = m_hi[kM], l0 = m_lo[0], l1 = m_lo[kM];
+                    const uint32_t mw[8] = {h0.x | l0.x, h0.y | l0.y, h0.z | l0.z, h0.w | l0.w, h1.x | l1.x, h1.y | l1.y, h1.z | l1.z, h1.w | l1.w};
+                    uint32_t hi[8], lo[8];
+#pragma unroll
+                    for (int i = 0; i < 16; i += 2) {
+                        const float x0 = (mw[i >> 1] & 0xFFFFu) ? __uint_as_float(v[i]) * f : 0.0f;
+                        const float x1 = (mw[i >> 1] >> 16) ? __uint_as_float(v[i + 1]) * f : 0.0f;
+                        const __half hh0 = __float2half_rn(x0), hh1 = __float2half_rn(x1);
+                        const __half ll0 = __float2half_rn(x0 - __half2float(hh0)), ll1 = __float2half_rn(x1 - __half2float(hh1));
+                        hi[i >> 1] = (uint32_t)__half_as_ushort(hh0) | ((uint32_t)__half_as_ushort(hh1) << 16);
+                        lo[i >> 1] = (uint32_t)__half_as_ushort(ll0) | ((uint32_t)__half_as_ushort(ll1) << 16);
+                    }
+                    __half* img = a.Y + (((size_t)mt * a.out_Kb + okb) * 2) * kImgA;
+                    uint4* p_hi = reinterpret_cast<uint4*>(img + at);
+                    uint4* p_lo = reinterpret_cast<uint4*>(img + kImgA + at);
+                    p_hi[0] = make_uint4(hi[0], hi[1], hi[2], hi[3]); p_hi[kM] = make_uint4(hi[4], hi[5], hi[6], hi[7]);
+                    p_lo[0] = make_uint4(lo[0], lo[1], lo[2], lo[3]); p_lo[kM] = make_uint4(lo[4], lo[5], lo[6], lo[7]);
+                }
+            } else if (a.Y) {
                 for (int c0 = 0; c0 < a.NT; c0 += 16) {
                     uint32_t v[16];
                     tmem_ld16(taddr + (uint32_t)c0, v);
@@ -818,6 +853,275 @@ __global__ void k_tc_load_layer(const float* __restrict__ W, const float* __rest
     }
 }
 
+// ---- the backward pass (qg_policy_tc_backward) ----------------------------------------------------------------------------------------------
+// dZ of every layer is carried like an activation: hi / lo images [m_tiles][KbZ][2][8][128][8], KbZ even (wgrad reads 128 columns per tile),
+// scaled by 2^sexp[l] so that the halves of PPO's ~1e-6 mean-loss gradients are not f16 subnormals.  sexp comes from a device-side amax of the
+// head's gradient and, layer by layer, from the bound max|dZ_(l-1)| <= max|dZ_l| colsum_l (colsum_l = max_k sum_n |W_l[n][k]|, computed when
+// the weights are loaded): every scaled value stays below 2^15, no host synchronisation, no second pass.
+constexpr int kChunkTiles = 8;       // wgrad's split-K chunk: 8 row tiles = 1024 rows, whatever the handle's capacity or the SM count
+
+__device__ __forceinline__ uint32_t f32_abs_bits(float x) { return __float_as_uint(x) & 0x7FFFFFFFu; }
+__device__ __forceinline__ int scale_exp(float b) {        // the largest s with b 2^s < 2^15 (0 for a zero or non-finite bound)
+    if (!(b > 0.0f) || !isfinite(b)) return 0;
+    int e; frexpf(b, &e);                                   // b < 2^e
+    return max(-100, min(100, 15 - e));
+}
+__device__ __forceinline__ void atomic_max_bits(uint32_t* dst, uint32_t v) {
+#pragma unroll
+    for (int o = 16; o; o >>= 1) v = max(v, __shfl_xor_sync(0xFFFFFFFFu, v, o));
+    if ((threadIdx.x & 31) == 0 && v) atomicMax(dst, v);
+}
+// amax[0] = max |dlogits|, |dvalues| (as f32 bits: non-negative floats order like their bits; a NaN compares above +inf)
+__global__ void k_tc_amax(const float* __restrict__ dl, long long n_dl, const float* __restrict__ dv, long long n_dv, uint32_t* amax) {
+    uint32_t m = 0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_dl + n_dv; i += (long long)gridDim.x * blockDim.x)
+        m = max(m, f32_abs_bits(i < n_dl ? dl[i] : dv[i - n_dl]));
+    atomic_max_bits(amax, m);
+}
+// colsum[l] (as f32 bits) = max over input columns k of sum_n |hi + lo| of the layer's forward weight images, inflated by 2^-9 (hi + lo is w to
+// 2^-22; the bound must not be below the true one)
+__global__ void k_tc_colsum(const __half* __restrict__ img, int N, int K, int NT, int n_tiles, int Kb, uint32_t* out) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    float s = 0.0f;
+    if (k < K) {
+        const long long term = (long long)n_tiles * Kb * NT * kKB;
+        const int kb = k / kKB, kl = k - kb * kKB;
+        for (int n = 0; n < N; ++n) {
+            const int nt = n / NT, nl = n - nt * NT;
+            const long long at = ((long long)nt * Kb + kb) * NT * kKB + ((long long)(kl >> 3) * NT + nl) * 8 + (kl & 7);
+            s += fabsf(__half2float(img[at]) + __half2float(img[term + at]));
+        }
+        s *= 1.0f + 1.0f / 512.0f;
+    }
+    atomic_max_bits(out, __float_as_uint(s));
+}
+__global__ void k_tc_scales(const uint32_t* __restrict__ amax, const uint32_t* __restrict__ colsum, int L, int* sexp) {
+    float b = __uint_as_float(amax[0]);
+    for (int l = L - 1; l >= 0; --l) {
+        sexp[l] = scale_exp(b);
+        b *= __uint_as_float(colsum[l]);
+    }
+}
+// the forward weight images of one layer (rows n < N, columns k < K) -> its dgrad operand: [term][nt over K, NTd wide][kb over n][n/8][k][n%8]
+__global__ void k_tc_transpose_w(const __half* __restrict__ img, int N, int K, int NT, int n_tiles, int Kb, __half* __restrict__ wt, int NTd,
+                                 int ntd_tiles, int KbN) {
+    const long long total = (long long)N * K, term = (long long)n_tiles * Kb * NT * kKB, term_t = (long long)ntd_tiles * KbN * NTd * kKB;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int n = (int)(i / K), k = (int)(i - (long long)n * K);
+        const int nt = n / NT, nl = n - nt * NT, kb = k / kKB, kl = k - kb * kKB;
+        const long long at = ((long long)nt * Kb + kb) * NT * kKB + ((long long)(kl >> 3) * NT + nl) * 8 + (kl & 7);
+        const int td = k / NTd, kd = k - td * NTd, nb = n / kKB, nn = n - nb * kKB;
+        const long long att = ((long long)td * KbN + nb) * NTd * kKB + ((long long)(nn >> 3) * NTd + kd) * 8 + (nn & 7);
+        wt[att] = img[at];
+        wt[term_t + att] = img[term + at];
+    }
+}
+// the head's dZ: dlogits [batch][A] and dvalues [batch] (column A) -> hi / lo images scaled by 2^sexp[0]; zero past the batch and past A (+ 1)
+__global__ void k_tc_head_grad(const float* __restrict__ dl, const float* __restrict__ dv, int A, long long batch, int KbZ, const int* __restrict__ sexp,
+                               __half* __restrict__ Z, long long total) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const int row = (int)(i % kM);
+    long long r = i / kM;
+    const int ch = (int)(r % 8); r /= 8;
+    const int kb = (int)(r % KbZ);
+    const long long mt = r / KbZ;
+    const long long grow = mt * kM + row;
+    const int s = __ldg(sexp);
+    uint32_t hi[4], lo[4];
+#pragma unroll
+    for (int j = 0; j < 8; j += 2) {
+        float x[2];
+#pragma unroll
+        for (int t = 0; t < 2; ++t) {
+            const int c = kb * kKB + ch * 8 + j + t;
+            float v = 0.0f;
+            if (grow < batch) {
+                if (c < A) v = dl[grow * A + c];
+                else if (c == A && dv) v = dv[grow];
+            }
+            x[t] = ldexpf(v, s);
+        }
+        const __half h0 = __float2half_rn(x[0]), h1 = __float2half_rn(x[1]);
+        const __half l0 = __float2half_rn(x[0] - __half2float(h0)), l1 = __float2half_rn(x[1] - __half2float(h1));
+        hi[j >> 1] = (uint32_t)__half_as_ushort(h0) | ((uint32_t)__half_as_ushort(h1) << 16);
+        lo[j >> 1] = (uint32_t)__half_as_ushort(l0) | ((uint32_t)__half_as_ushort(l1) << 16);
+    }
+    __half* img = Z + ((size_t)mt * KbZ + kb) * 2 * kImgA + ((size_t)ch * kM + row) * 8;
+    *reinterpret_cast<uint4*>(img) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+    *reinterpret_cast<uint4*>(img + kImgA) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+}
+
+// wgrad:  part[chunk][o][i] = sum over the chunk's rows of dZ[row][o] H[row][i]  (scaled by 2^sexp), tcgen05 with K = rows.
+// Both operands are read in place from their images, MN-major: in an image [c/8][row][c%8] a core matrix is 8 rows (K) x 8 contiguous
+// columns (MN); K groups of 8 rows are 128 bytes apart (leading byte offset), MN groups of 8 columns 128 x 16 = 2048 bytes (stride byte
+// offset).  The two dZ images of a 128-column M tile sit back to back in shared memory, so the MN stride stays 2048 across them.
+// Tile = 128 output features (o) x 64 input features (i, one H image); a stage = one 128-row tile: dZ hi / lo of both K blocks (64 KB) + H hi
+// (/ lo) (16 / 32 KB); 2 stages.  Products dZ_hi H_hi + dZ_hi H_lo + dZ_lo H_hi (layer 1: H is 0 / 1, exact in hi: two products).
+struct WgradArgs {
+    const __half* Z; const __half* H; float* part;
+    int KbZ, KbH, h_terms, mo_tiles, chunks, m_tiles;
+    long long ldp, part_stride;
+};
+constexpr int kWStages = 2;
+constexpr uint32_t kWStageBytes = 6u * kImgA * 2;           // 4 dZ images + 2 H images
+constexpr uint32_t kWSmem = kWStages * kWStageBytes + 128;
+// MN-major operand descriptor: leading byte offset = K-group stride, stride byte offset = MN-group stride (cute::UMMA canonical INTERLEAVE
+// MN-major layout ((8,m),(8,k)) : ((1,SBO),(8,LBO)) in elements)
+__host__ __device__ constexpr uint32_t instr_desc_mn(int n) { return instr_desc(n) | (1u << 15) | (1u << 16); }
+
+__global__ void __launch_bounds__(kThreads, 1) k_tc_wgrad(const __grid_constant__ WgradArgs a) {
+    extern __shared__ __align__(1024) uint8_t smem[];
+    uint64_t* const full = reinterpret_cast<uint64_t*>(smem + kWStages * kWStageBytes);
+    uint64_t* const empty = full + kWStages;
+    uint64_t* const acc_full = empty + kWStages;
+    uint64_t* const acc_empty = acc_full + 2;
+    uint32_t* const tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int ni_tiles = a.KbH, items = a.chunks * a.mo_tiles * ni_tiles;
+    const uint32_t acc_cols = 64;
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < kWStages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
+        for (int s = 0; s < 2; ++s) { mbar_init(acc_full + s, 1); mbar_init(acc_empty + s, 4); }
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    if (warp == 1) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n" ::"r"(smem_u32(tmem_slot)), "r"(2 * acc_cols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem_base = *tmem_slot;
+    pdl_launch_dependents();
+    pdl_wait();
+    // item t -> (chunk, o tile, i tile); the chunk's row tiles [c * kChunkTiles, ..)
+    auto decode = [&](int t, int& c, int& mo, int& ni) { ni = t % ni_tiles; t /= ni_tiles; mo = t % a.mo_tiles; c = t / a.mo_tiles; };
+    if (warp == 0) {
+        if (lane == 0) {
+            uint32_t stage = 0, phase = 0;
+            const uint32_t bytes = (4u + (uint32_t)a.h_terms) * kImgA * 2;
+            for (int t = blockIdx.x; t < items; t += gridDim.x) {
+                int c, mo, ni; decode(t, c, mo, ni);
+                const int mt1 = min(a.m_tiles, (c + 1) * kChunkTiles);
+                for (int mt = c * kChunkTiles; mt < mt1; ++mt) {
+                    mbar_wait(empty + stage, phase ^ 1u);
+                    mbar_expect_tx(full + stage, bytes);
+                    uint8_t* const sp = smem + stage * kWStageBytes;
+                    for (int term = 0; term < 2; ++term)             // [term][kb 2 mo, 2 mo + 1]: the M tile's two images back to back
+                        for (int j = 0; j < 2; ++j)
+                            bulk_g2s(sp + (term * 2 + j) * kImgA * 2, a.Z + (((size_t)mt * a.KbZ + 2 * mo + j) * 2 + term) * kImgA, kImgA * 2, full + stage);
+                    for (int term = 0; term < a.h_terms; ++term)
+                        bulk_g2s(sp + (4 + term) * kImgA * 2, a.H + (((size_t)mt * a.KbH + ni) * a.h_terms + term) * kImgA, kImgA * 2, full + stage);
+                    if (++stage == (uint32_t)kWStages) { stage = 0; phase ^= 1u; }
+                }
+            }
+        }
+    } else if (warp == 1) {
+        uint32_t stage = 0, phase = 0, as = 0, aphase = 0;
+        const uint32_t idesc = instr_desc_mn(64), lbo = 128, sbo = 128 * 16;
+        for (int t = blockIdx.x; t < items; t += gridDim.x) {
+            int c, mo, ni; decode(t, c, mo, ni);
+            const int mt1 = min(a.m_tiles, (c + 1) * kChunkTiles);
+            mbar_wait(acc_empty + as, aphase ^ 1u);
+            tc_fence_after();
+            const uint32_t d = tmem_base + as * acc_cols;
+            for (int mt = c * kChunkTiles; mt < mt1; ++mt) {
+                mbar_wait(full + stage, phase);
+                tc_fence_after();
+                const uint32_t sp = smem_u32(smem + stage * kWStageBytes);
+                const uint32_t z_hi = sp, z_lo = sp + 2 * kImgA * 2, h_hi = sp + 4 * kImgA * 2, h_lo = sp + 5 * kImgA * 2;
+#pragma unroll
+                for (int k = 0; k < kM / 16; ++k) {                    // K = 16 rows: two 8-row groups, 256 bytes
+                    const uint32_t o = 256u * k;
+                    umma_f16_w(d, smem_desc(z_hi + o, lbo, sbo), smem_desc(h_hi + o, lbo, sbo), idesc, (mt > c * kChunkTiles || k) ? 1u : 0u);
+                    if (a.h_terms == 2) umma_f16_w(d, smem_desc(z_hi + o, lbo, sbo), smem_desc(h_lo + o, lbo, sbo), idesc, 1u);
+                    umma_f16_w(d, smem_desc(z_lo + o, lbo, sbo), smem_desc(h_hi + o, lbo, sbo), idesc, 1u);
+                }
+                umma_commit_w(empty + stage);
+                if (++stage == (uint32_t)kWStages) { stage = 0; phase ^= 1u; }
+            }
+            umma_commit_w(acc_full + as);
+            if (++as == 2) { as = 0; aphase ^= 1u; }
+        }
+    } else {
+        const int q = warp & 3, row = q * 32 + lane;
+        uint32_t as = 0, aphase = 0;
+        for (int t = blockIdx.x; t < items; t += gridDim.x) {
+            int c, mo, ni; decode(t, c, mo, ni);
+            mbar_wait(acc_full + as, aphase);
+            tc_fence_after();
+            const uint32_t taddr = tmem_base + as * acc_cols + ((uint32_t)(q * 32) << 16);
+            float* dst = a.part + (size_t)c * a.part_stride + (size_t)(mo * kM + row) * a.ldp + (size_t)ni * kKB;
+            for (int c0 = 0; c0 < 64; c0 += 16) {
+                uint32_t v[16];
+                tmem_ld16(taddr + (uint32_t)c0, v);
+#pragma unroll
+                for (int i = 0; i < 16; i += 4)
+                    *reinterpret_cast<float4*>(dst + c0 + i) = make_float4(__uint_as_float(v[i]), __uint_as_float(v[i + 1]), __uint_as_float(v[i + 2]), __uint_as_float(v[i + 3]));
+            }
+            tc_fence_before();
+            __syncwarp();
+            if (lane == 0) mbar_arrive(acc_empty + as);
+            if (++as == 2) { as = 0; aphase ^= 1u; }
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(tmem_base), "r"(2 * acc_cols) : "memory");
+}
+
+// db partials: bpart[chunk][o] = sum over the chunk's rows of dZ[row][o] (hi + lo, scaled).  Block = (chunk, K block of dZ), thread = row of a
+// tile: 8 tiles in order, then a fixed tree over the 128 rows
+__global__ void __launch_bounds__(128) k_tc_bias_partial(const __half* __restrict__ Z, int KbZ, int m_tiles, float* __restrict__ bpart, int ldb) {
+    __shared__ float red[128][65];
+    const int c = blockIdx.x, kb = blockIdx.y, row = threadIdx.x;
+    float s[64];
+#pragma unroll
+    for (int j = 0; j < 64; ++j) s[j] = 0.0f;
+    const int mt1 = min(m_tiles, (c + 1) * kChunkTiles);
+    for (int mt = c * kChunkTiles; mt < mt1; ++mt) {
+        const __half* img = Z + ((size_t)mt * KbZ + kb) * 2 * kImgA;
+#pragma unroll
+        for (int ch = 0; ch < 8; ++ch) {
+            const uint4 h = *reinterpret_cast<const uint4*>(img + ((size_t)ch * kM + row) * 8);
+            const uint4 l = *reinterpret_cast<const uint4*>(img + kImgA + ((size_t)ch * kM + row) * 8);
+            const uint32_t hw[4] = {h.x, h.y, h.z, h.w}, lw[4] = {l.x, l.y, l.z, l.w};
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const float2 fh = __half22float2(*reinterpret_cast<const __half2*>(&hw[j])), fl = __half22float2(*reinterpret_cast<const __half2*>(&lw[j]));
+                s[ch * 8 + 2 * j] += fh.x + fl.x;
+                s[ch * 8 + 2 * j + 1] += fh.y + fl.y;
+            }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < 64; ++j) red[row][j] = s[j];
+    __syncthreads();
+    for (int w = 64; w >= 1; w >>= 1) {
+        if (row < w)
+            for (int j = 0; j < 64; ++j) red[row][j] += red[row + w][j];
+        __syncthreads();
+    }
+    if (row < 64) bpart[(size_t)c * ldb + kb * kKB + row] = red[0][row];
+}
+// partials -> gradients: sum over the chunks in order, times 2^-sexp.  Entry (o, i) of a [rows][ld] partial; o == nrows (the head's column A)
+// goes to the value head's gradient
+__global__ void k_tc_reduce(const float* __restrict__ part, int chunks, long long stride, long long ld, int nrows, int K, int vrow,
+                            const int* __restrict__ sexp, float* __restrict__ out, float* __restrict__ vout) {
+    const long long total = (long long)(nrows + vrow) * K;
+    const int s = -__ldg(sexp);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int o = (int)(i / K), k = (int)(i - (long long)o * K);
+        const float* p = part + (size_t)o * ld + k;
+        float acc = 0.0f;
+        for (int c = 0; c < chunks; ++c) acc += p[(size_t)c * stride];
+        acc = ldexpf(acc, s);
+        if (o < nrows) out[i] = acc;
+        else vout[k] = acc;
+    }
+}
+
 }  // namespace tc
 }  // namespace qg
 
@@ -835,6 +1139,16 @@ struct qg_policy_tc {
     long long max_batch = 0; int m_tiles = 0;
     std::vector<TcLayer> layers;
     std::vector<__half*> acts;     // acts[l] = X images of layer l
+    // the last forward (qg_policy_tc_backward refers to it): its generation, batch and whether it ran per layer (acts[] hold its inputs)
+    long long generation = 0, fwd_batch = -1; bool fwd_layers = false;
+    // qg_policy_tc_enable_training
+    bool training = false;
+    std::vector<__half*> dz;       // dz[l] = dZ images of layer l [m_tiles][kbz[l]][2][8][128][8]
+    std::vector<__half*> wt;       // wt[l] (l >= 1) = the transposed weight images the dgrad reads
+    std::vector<int> kbz, ntd;     // dZ K blocks (even) / the dgrad's column tile width of layer l
+    float* part = nullptr; float* bpart = nullptr;    // wgrad / db split-K partials
+    uint32_t* stats = nullptr;     // [0] amax of the head gradient, [1 + l] colsum of layer l (f32 bits)
+    int* sexp = nullptr;           // [l] the power-of-two scale of dZ_l
 };
 
 namespace {
@@ -847,6 +1161,23 @@ namespace {
         }                                                                                      \
     } while (0)
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
+inline unsigned grid_for(const qg_policy_tc* p, long long total) { return (unsigned)std::max<long long>(1, std::min<long long>((total + 255) / 256, (long long)p->num_sms * 8)); }
+
+// the dgrad's transposed weight images and the column sums of the scale bound, from the forward weight images (same halves)
+int refresh_training_images(qg_policy_tc* p, cudaStream_t st) {
+    const int L = (int)p->layers.size();
+    TC_CUDA_OK(cudaMemsetAsync(p->stats + 1, 0, sizeof(uint32_t) * L, st));
+    for (int l = 0; l < L; ++l) {
+        const TcLayer& T = p->layers[l];
+        tc::k_tc_colsum<<<(unsigned)((T.K + 255) / 256), 256, 0, st>>>(T.W, T.N, T.K, T.NT, T.n_tiles, T.Kb, p->stats + 1 + l);
+        TC_CUDA_OK(cudaGetLastError());
+        if (l == 0) continue;
+        const int ntd_tiles = p->layers[l - 1].Npad / p->ntd[l];
+        tc::k_tc_transpose_w<<<grid_for(p, (long long)T.N * T.K), 256, 0, st>>>(T.W, T.N, T.K, T.NT, T.n_tiles, T.Kb, p->wt[l], p->ntd[l], ntd_tiles, p->kbz[l]);
+        TC_CUDA_OK(cudaGetLastError());
+    }
+    return QG_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -856,6 +1187,12 @@ void qg_policy_tc_destroy(qg_policy_tc* p) {
     for (auto& l : p->layers) { if (l.W) cudaFree(l.W); if (l.bias) cudaFree(l.bias); }
     for (auto* a : p->acts) if (a) cudaFree(a);
     if (p->W2_fused) cudaFree(p->W2_fused);
+    for (auto* a : p->dz) if (a) cudaFree(a);
+    for (auto* a : p->wt) if (a) cudaFree(a);
+    if (p->part) cudaFree(p->part);
+    if (p->bpart) cudaFree(p->bpart);
+    if (p->stats) cudaFree(p->stats);
+    if (p->sexp) cudaFree(p->sexp);
     delete p;
 }
 
@@ -938,7 +1275,7 @@ int qg_policy_tc_create(int32_t device, int32_t obs_size, int32_t num_layers, co
         while (L.stages > 1 && tc::plan_smem(L.a_terms, L.NT, L.stages, L.staging).total > 220 * 1024) --L.stages;
         max_smem = std::max<size_t>(max_smem, tc::plan_smem(L.a_terms, L.NT, L.stages, L.staging).total);
     }
-    cudaError_t ce = cudaFuncSetAttribute(tc::k_tc_layer, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem);
+    cudaError_t ce = cudaFuncSetAttribute(tc::k_tc_layer<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem);
     if (ce != cudaSuccess) { set_error(std::string("qg_policy_tc_create: ") + cudaGetErrorString(ce)); return fail(QG_ERR_CUDA); }
     // the one-kernel path: embeddings (a multiple of 128 wide after padding) -> one common layer (<= 256) -> head
     if (num_layers == 3 && p->layers[0].Npad % 128 == 0 && p->layers[0].Npad <= 512 && p->layers[0].NT == 128 && p->layers[1].Npad <= 256) {
@@ -995,7 +1332,7 @@ int qg_policy_tc_load_weights_dev(qg_policy_tc* p, int32_t obs_size, int32_t num
                                                                                        L1.Npad, 1, L1.Kb, p->W2_fused, nullptr);
         TC_CUDA_OK(cudaGetLastError());
     }
-    return QG_OK;
+    return p->training ? refresh_training_images(p, st) : QG_OK;
 }
 
 int32_t qg_policy_tc_num_actions(const qg_policy_tc* p) { return p ? p->num_actions : 0; }
@@ -1010,6 +1347,7 @@ int qg_policy_tc_forward_bits(qg_policy_tc* p, const uint32_t* obs_bits_dev, int
     if (!p || !obs_bits_dev) { set_error("null argument"); return QG_ERR_INVALID; }
     if (batch < 0 || batch > p->max_batch) { set_error("qg_policy_tc_forward_bits: batch larger than the handle was created for"); return QG_ERR_INVALID; }
     if (values_dev && !p->has_value) { set_error("qg_policy_tc_forward_bits: the policy has no value head"); return QG_ERR_INVALID; }
+    ++p->generation; p->fwd_batch = batch; p->fwd_layers = !(p->fused && !p->force_layers);
     if (batch == 0) return QG_OK;
     TC_CUDA_OK(cudaSetDevice(p->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -1055,7 +1393,114 @@ int qg_policy_tc_forward_bits(qg_policy_tc* p, const uint32_t* obs_bits_dev, int
         cudaLaunchAttribute at[1];
         at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[0].val.programmaticStreamSerializationAllowed = 1;
         lc.attrs = at; lc.numAttrs = 1;
-        TC_CUDA_OK(cudaLaunchKernelEx(&lc, tc::k_tc_layer, a));
+        TC_CUDA_OK(cudaLaunchKernelEx(&lc, tc::k_tc_layer<0>, a));
+    }
+    return QG_OK;
+}
+
+int64_t qg_policy_tc_generation(const qg_policy_tc* p) { return p ? p->generation : 0; }
+
+int qg_policy_tc_enable_training(qg_policy_tc* p) {
+    if (!p) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (p->training) return QG_OK;
+    TC_CUDA_OK(cudaSetDevice(p->device));
+    const int L = (int)p->layers.size();
+    const int chunks = (p->m_tiles + tc::kChunkTiles - 1) / tc::kChunkTiles;
+    p->dz.assign(L, nullptr); p->wt.assign(L, nullptr); p->kbz.assign(L, 0); p->ntd.assign(L, 0);
+    size_t part_floats = 0, bpart_floats = 0;
+    for (int l = 0; l < L; ++l) {
+        const TcLayer& T = p->layers[l];
+        p->kbz[l] = round_up((T.Npad + tc::kKB - 1) / tc::kKB, 2);
+        const size_t zbytes = (size_t)p->m_tiles * p->kbz[l] * 2 * tc::kImgA * sizeof(__half);
+        TC_CUDA_OK(cudaMalloc(&p->dz[l], zbytes));
+        TC_CUDA_OK(cudaMemset(p->dz[l], 0, zbytes));      // (K blocks past the layer's width are never written: they stay zero)
+        part_floats = std::max(part_floats, (size_t)chunks * p->kbz[l] * tc::kKB * T.Kb * tc::kKB);
+        bpart_floats = std::max(bpart_floats, (size_t)chunks * p->kbz[l] * tc::kKB);
+        if (l == 0) continue;
+        const int kpad = p->layers[l - 1].Npad;             // the dgrad's output columns: layer l's input, padded to 64
+        p->ntd[l] = kpad % 128 == 0 ? 128 : 64;
+        const size_t wbytes = (size_t)2 * (kpad / p->ntd[l]) * p->kbz[l] * p->ntd[l] * tc::kKB * sizeof(__half);
+        TC_CUDA_OK(cudaMalloc(&p->wt[l], wbytes));
+        TC_CUDA_OK(cudaMemset(p->wt[l], 0, wbytes));
+    }
+    TC_CUDA_OK(cudaFuncSetAttribute(tc::k_tc_layer<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::plan_smem(2, 128, tc::kStages, 0).total));
+    TC_CUDA_OK(cudaMalloc(&p->part, part_floats * sizeof(float)));
+    TC_CUDA_OK(cudaMalloc(&p->bpart, bpart_floats * sizeof(float)));
+    TC_CUDA_OK(cudaMalloc(&p->stats, sizeof(uint32_t) * (1 + L)));
+    TC_CUDA_OK(cudaMalloc(&p->sexp, sizeof(int) * L));
+    TC_CUDA_OK(cudaFuncSetAttribute(tc::k_tc_wgrad, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::kWSmem));
+    p->training = true;
+    const int rc = refresh_training_images(p, nullptr);
+    if (rc != QG_OK) return rc;
+    TC_CUDA_OK(cudaDeviceSynchronize());
+    return QG_OK;
+}
+
+int qg_policy_tc_backward(qg_policy_tc* p, int64_t generation, int64_t batch, const float* dlogits_dev, const float* dvalues_dev, float* const* grad_w_dev,
+                          float* const* grad_b_dev, float* grad_vw_dev, float* grad_vb_dev, qg_stream stream) {
+    if (!p || !dlogits_dev || !grad_w_dev || !grad_b_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (!p->training) { set_error("qg_policy_tc_backward: qg_policy_tc_enable_training was not called"); return QG_ERR_INVALID; }
+    if (generation != p->generation || batch != p->fwd_batch || !p->fwd_layers) {
+        set_error("qg_policy_tc_backward: not the handle's latest forward (a newer forward ran, or the latest ran the fused kernel)");
+        return QG_ERR_INVALID;
+    }
+    if (p->has_value && (!grad_vw_dev || !grad_vb_dev)) { set_error("qg_policy_tc_backward: the value head's gradient buffers are missing"); return QG_ERR_INVALID; }
+    const int L = (int)p->layers.size();
+    for (int l = 0; l < L; ++l) if (!grad_w_dev[l] || !grad_b_dev[l]) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (batch == 0) return QG_OK;
+    TC_CUDA_OK(cudaSetDevice(p->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const int m_tiles = (int)((batch + tc::kM - 1) / tc::kM);
+    const int chunks = (m_tiles + tc::kChunkTiles - 1) / tc::kChunkTiles;
+    const int A = p->num_actions;
+    // scales: amax of the head's gradient, then the bound chain (k_tc_scales)
+    TC_CUDA_OK(cudaMemsetAsync(p->stats, 0, sizeof(uint32_t), st));
+    const long long n_dl = batch * A, n_dv = dvalues_dev ? batch : 0;
+    tc::k_tc_amax<<<grid_for(p, n_dl + n_dv), 256, 0, st>>>(dlogits_dev, n_dl, dvalues_dev, n_dv, p->stats);
+    TC_CUDA_OK(cudaGetLastError());
+    tc::k_tc_scales<<<1, 1, 0, st>>>(p->stats, p->stats + 1, L, p->sexp);
+    TC_CUDA_OK(cudaGetLastError());
+    {
+        const long long total = (long long)m_tiles * p->kbz[L - 1] * 8 * tc::kM;
+        tc::k_tc_head_grad<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(dlogits_dev, p->has_value ? dvalues_dev : nullptr, A, batch, p->kbz[L - 1],
+                                                                             p->sexp + (L - 1), p->dz[L - 1], total);
+        TC_CUDA_OK(cudaGetLastError());
+    }
+    // dgrad, layers L .. 2: dZ_(l-1) = mask_l (dZ_l W_l) 2^(s_(l-1) - s_l)
+    for (int l = L - 1; l >= 1; --l) {
+        const int kpad = p->layers[l - 1].Npad, NT = p->ntd[l];
+        tc::LayerArgs a{};
+        a.X = p->dz[l]; a.W = p->wt[l]; a.bias = nullptr; a.Y = p->dz[l - 1];
+        a.a_terms = 2; a.Kb = p->kbz[l]; a.NT = NT; a.n_tiles = kpad / NT; a.m_tiles = m_tiles; a.out_Kb = p->kbz[l - 1];
+        a.relu = 0; a.num_actions = A; a.has_value = 0; a.batch = batch; a.stages = tc::kStages;
+        a.mask = p->acts[l]; a.sexp = p->sexp; a.s_in = l; a.s_out = l - 1; a.mask_Kb = p->layers[l].Kb;
+        cudaLaunchConfig_t lc{};
+        lc.gridDim = dim3((unsigned)std::min(m_tiles * a.n_tiles, p->num_sms)); lc.blockDim = dim3(tc::kThreads);
+        lc.dynamicSmemBytes = tc::plan_smem(2, NT, tc::kStages, 0).total; lc.stream = st;
+        TC_CUDA_OK(cudaLaunchKernelEx(&lc, tc::k_tc_layer<1>, a));
+    }
+    // wgrad and db of every layer: split-K partials per 1024-row chunk, reduced in chunk order
+    for (int l = 0; l < L; ++l) {
+        const TcLayer& T = p->layers[l];
+        const bool last = l == L - 1;
+        const int nrows = T.N - (last ? p->has_value : 0), vrow = last ? p->has_value : 0;
+        tc::WgradArgs w{};
+        w.Z = p->dz[l]; w.H = p->acts[l]; w.part = p->part;
+        w.KbZ = p->kbz[l]; w.KbH = T.Kb; w.h_terms = T.a_terms; w.mo_tiles = p->kbz[l] / 2; w.chunks = chunks; w.m_tiles = m_tiles;
+        w.ldp = (long long)T.Kb * tc::kKB; w.part_stride = (long long)p->kbz[l] * tc::kKB * w.ldp;
+        const int items = chunks * w.mo_tiles * w.KbH;
+        cudaLaunchConfig_t lc{};
+        lc.gridDim = dim3((unsigned)std::min(items, p->num_sms)); lc.blockDim = dim3(tc::kThreads);
+        lc.dynamicSmemBytes = tc::kWSmem; lc.stream = st;
+        TC_CUDA_OK(cudaLaunchKernelEx(&lc, tc::k_tc_wgrad, w));
+        tc::k_tc_reduce<<<grid_for(p, (long long)T.N * T.K), 256, 0, st>>>(p->part, chunks, w.part_stride, w.ldp, nrows, T.K, vrow, p->sexp + l,
+                                                                           grad_w_dev[l], grad_vw_dev);
+        TC_CUDA_OK(cudaGetLastError());
+        const int ldb = p->kbz[l] * tc::kKB;
+        tc::k_tc_bias_partial<<<dim3((unsigned)chunks, (unsigned)p->kbz[l]), 128, 0, st>>>(p->dz[l], p->kbz[l], m_tiles, p->bpart, ldb);
+        TC_CUDA_OK(cudaGetLastError());
+        tc::k_tc_reduce<<<grid_for(p, T.N), 256, 0, st>>>(p->bpart, chunks, ldb, 1, nrows, 1, vrow, p->sexp + l, grad_b_dev[l], grad_vb_dev);
+        TC_CUDA_OK(cudaGetLastError());
     }
     return QG_OK;
 }

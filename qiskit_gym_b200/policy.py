@@ -110,7 +110,8 @@ class TensorCorePolicy:
     emulation of the split arithmetic, F the inputs whose lo half is an f16 subnormal (0 < h < 2^-3) forward-propagated through |W|; against
     the float64 module add the propagated split error (|v - hi - lo| <= 2^-22 |v| + 2^-25).  tests/test_policy_tc_envelope.py derives both."""
 
-    def __init__(self, policy: torch.nn.Module, max_batch: int, device=None, with_value: bool = True):
+    def __init__(self, policy: torch.nn.Module, max_batch: int, device=None, with_value: bool = True, training: bool = False):
+        """training: also allocate the backward pass (forward_train); the handle then runs one kernel per layer."""
         if not torch.cuda.is_available():
             raise RuntimeError("qiskit_gym_b200 needs a CUDA device (no CPU fallback)")
         self.device_index = torch.cuda.current_device() if device is None else (device.index if isinstance(device, torch.device) else int(device))
@@ -140,6 +141,12 @@ class TensorCorePolicy:
         check(lib().qg_policy_tc_create(self.device_index, self.obs_size, n, widths, wp, bp, vw, C.c_float(vb), self.max_batch, C.byref(h)))
         self._h = h
         self.out_features = [int(w.shape[0]) for w in ws]
+        self.training = bool(training)
+        if self.training:
+            if not self.has_value:
+                raise NotImplementedError("TensorCorePolicy(training=True) needs the value head (with_value=True)")
+            check(lib().qg_policy_tc_enable_training(self._h))
+            self.set_per_layer(True)
 
     def _device_params(self, policy: torch.nn.Module):
         """The module's action-path weights / biases (and value head) when they can be read in place: f32, contiguous, on this device, with the
@@ -206,6 +213,50 @@ class TensorCorePolicy:
         st = C.c_void_p(torch.cuda.current_stream(obs_bits.device).cuda_stream)
         check(lib().qg_policy_tc_forward_bits(self._h, _dptr(obs_bits), B, _dptr(probs), _dptr(logits), _dptr(values), st))
         return probs if probs is not None else (logits if logits is not None else values)
+
+
+    def forward_train(self, policy: torch.nn.Module, obs_bits: torch.Tensor):
+        """Differentiable forward of `policy` on packed observation bits int32 [B, obs_words] -> (logits [B, A], values [B, 1]), like
+        policy(dense) for a BasicPolicy.  The handle's weights are refreshed from the module first (load_weights) when they changed.
+        backward() writes the gradients of exactly the parameters of action_layers and simple_value_head, computed by the tcgen05 backward
+        pass (qg_policy_tc_backward); autograd accumulates them into .grad.  A backward after a newer forward on this handle raises."""
+        if not self.training:
+            raise ValueError("forward_train needs a handle created with training=True")
+        if self.version != weights_version(policy):
+            self.load_weights(policy)
+        layers = action_layers(policy)
+        head = simple_value_head(policy)
+        params = [l.weight for l in layers] + [l.bias for l in layers] + [head.weight, head.bias]
+        return _TensorCoreTrain.apply(self, obs_bits, *params)
+
+
+class _TensorCoreTrain(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, tcp, obs_bits, *params):
+        B = obs_bits.shape[0]
+        if B > tcp.max_batch:
+            raise ValueError(f"forward_train: {B} rows exceed the handle's max_batch {tcp.max_batch}")
+        logits = torch.empty((B, tcp.num_actions), dtype=torch.float32, device=obs_bits.device)
+        values = torch.empty((B,), dtype=torch.float32, device=obs_bits.device)
+        tcp.forward_bits(obs_bits, logits=logits, values=values)
+        ctx.tcp, ctx.generation, ctx.B = tcp, int(lib().qg_policy_tc_generation(tcp._h)), B
+        ctx.shapes = [p.shape for p in params]
+        return logits, values.reshape(B, 1)
+
+    @staticmethod
+    def backward(ctx, dlogits, dvalues):
+        tcp, B = ctx.tcp, ctx.B
+        dev = tcp.device
+        dl = dlogits.float().contiguous() if dlogits is not None else torch.zeros((B, tcp.num_actions), dtype=torch.float32, device=dev)
+        dv = dvalues.float().reshape(B).contiguous() if dvalues is not None else None
+        grads = [torch.empty(s, dtype=torch.float32, device=dev) for s in ctx.shapes]
+        n = len(tcp.out_features)
+        gw = (C.c_void_p * n)(*[g.data_ptr() for g in grads[:n]])
+        gb = (C.c_void_p * n)(*[g.data_ptr() for g in grads[n:2 * n]])
+        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        check(lib().qg_policy_tc_backward(tcp._h, ctx.generation, B, _dptr(dl), _dptr(dv), gw, gb, C.c_void_p(grads[2 * n].data_ptr()),
+                                          C.c_void_p(grads[2 * n + 1].data_ptr()), st))
+        return (None, None, *grads)
 
 
 def pack_obs_bits(obs: torch.Tensor) -> torch.Tensor:

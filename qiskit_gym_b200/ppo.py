@@ -295,13 +295,20 @@ class PPO(Trainer):
     algorithm = "PPO"
 
     def __init__(self, env_kind: int, num_qubits: int, gateset, policy: torch.nn.Module, config: dict | None = None, device=None,
-                 seed: int = 0, use_twists: bool = True, minibatch_size: int | None = None, matmul_precision: str = "f32", **env_kwargs):
+                 seed: int = 0, use_twists: bool = True, minibatch_size: int | None = None, matmul_precision: str = "f32",
+                 update_precision: str = "f32", **env_kwargs):
         """matmul_precision: "f32" (default), "tf32" or "bf16" run the policy in PyTorch on dense observations (RolloutCollector.collect);
         "tensor_core" collects with packed-bit observations and the tcgen05 policy (RolloutCollector.collect_packed, twists included) and
         the update unpacks each minibatch's observations from the bits.  "tensor_core" raises NotImplementedError where that path cannot run
-        (more than 127 actions, a value head that is not one Linear, a device that is not sm_100)."""
+        (more than 127 actions, a value head that is not one Linear, a device that is not sm_100).
+        update_precision: "f32" (default) runs the update's forward and backward in PyTorch; "tensor_core" runs them on the tcgen05 kernels
+        (TensorCorePolicy.forward_train) from the packed rollout's bits, so it needs matmul_precision="tensor_core".  The loss is the same code."""
         if matmul_precision not in ("f32", "tf32", "bf16", "tensor_core"):
             raise ValueError(f"matmul_precision must be one of f32, tf32, bf16, tensor_core (got {matmul_precision!r})")
+        if update_precision not in ("f32", "tensor_core"):
+            raise ValueError(f"update_precision must be f32 or tensor_core (got {update_precision!r})")
+        if update_precision == "tensor_core" and matmul_precision != "tensor_core":
+            raise ValueError('update_precision="tensor_core" trains on the packed rollout\'s bits: it needs matmul_precision="tensor_core"')
         super().__init__(env_kind, num_qubits, gateset, policy, config, device=device, seed=seed, minibatch_size=minibatch_size, **env_kwargs)
         self.tensor_core = matmul_precision == "tensor_core"
         self.collector = RolloutCollector(self.env, self.policy, gamma=self.cfg["collecting"]["gamma"], lam=self.cfg["collecting"]["lambda"],
@@ -309,6 +316,8 @@ class PPO(Trainer):
                                           matmul_precision="f32" if self.tensor_core else matmul_precision)
         if self.tensor_core:
             self.collector.tensor_core_policy()          # fails here, not in the first iteration, where the tensor-core policy cannot run
+        self.update_tc = update_precision == "tensor_core"
+        self._train_tcp = None
 
     def iterate(self) -> dict:
         steps = self._episode_steps()
@@ -330,6 +339,8 @@ class PPO(Trainer):
         else:
             obs = ro.obs.reshape((-1,) + tuple(ro.obs.shape[2:]))[idx]
             obs_of = lambda sel: obs[sel]                                                         # noqa: E731
+        forward = (lambda sel: self._train_policy(int(bits[sel].shape[0])).forward_train(self.policy, bits[sel])) if self.update_tc \
+            else (lambda sel: self.policy(obs_of(sel)))                                           # noqa: E731
         act = ro.policy_actions.reshape(-1)[idx]
         logp_old = ro.logp.reshape(-1)[idx]
         adv = ro.advantages.reshape(-1)[idx]
@@ -342,7 +353,7 @@ class PPO(Trainer):
         stats = {}
         for _ in range(int(t["num_epochs"])):
             for sel in self._minibatches(n):
-                logits, value = self.policy(obs_of(sel))
+                logits, value = forward(sel)
                 logp_all = torch.log_softmax(logits.float(), dim=-1)
                 logp = logp_all.gather(1, act[sel][:, None]).squeeze(1)
                 ratio = torch.exp(logp - logp_old[sel])
@@ -356,6 +367,15 @@ class PPO(Trainer):
                          "clip_frac": ((ratio - 1.0).abs() > clip).float().mean().detach()}
         self.policy.eval()
         return {k: float(v.item()) for k, v in stats.items()} | {"samples": n}
+
+    def _train_policy(self, rows: int):
+        """The update's training handle (TensorCorePolicy with the backward pass), grown geometrically when a minibatch outgrows it."""
+        from .policy import TensorCorePolicy
+        tcp = self._train_tcp
+        if tcp is None or tcp.max_batch < rows:
+            cap = max(rows, 2 * tcp.max_batch) if tcp is not None else rows
+            tcp = self._train_tcp = TensorCorePolicy(self.policy, max_batch=cap, device=self.device, with_value=True, training=True)
+        return tcp
 
 
 class AlphaZero(Trainer):

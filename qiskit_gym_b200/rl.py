@@ -134,22 +134,28 @@ class RLSynthesis:
         if actions is not None:
             return self.env.build_circuit_from_solution(actions, input)
 
-    def learn(self, initial_difficulty=1, num_iterations=int(1e10), tb_path=None, log=None, seed: int = 0, matmul_precision: str = "f32"):
+    def learn(self, initial_difficulty=1, num_iterations=int(1e10), tb_path=None, log=None, seed: int = 0, matmul_precision: str = "f32",
+              update_precision: str = "f32"):
         """rl/synthesis.py:128-139: PPO (`twisterl.rl.PPO`) or AlphaZero (`twisterl.rl.AZ`) on the device (ppo.py).  The trained
         policy is `self.policy` (searches built before the call are dropped so that `synth` uses the new weights).
         matmul_precision (PPO): how the collector runs the policy — "f32" (the reference's arithmetic, the default), "tf32", "bf16", or
-        "tensor_core" (packed observations and the tcgen05 policy: RolloutCollector.collect_packed)."""
+        "tensor_core" (packed observations and the tcgen05 policy: RolloutCollector.collect_packed).
+        update_precision (PPO): "f32" (the default) or "tensor_core" (the update's forward and backward on the tcgen05 kernels; needs
+        matmul_precision="tensor_core")."""
         from . import ppo
         algo = self.algorithm_cls.split(".")[-1]
         if algo not in ("PPO", "AZ"):
             raise NotImplementedError(f"algorithm class {self.algorithm_cls} is not supported (twisterl.rl.PPO, twisterl.rl.AZ)")
         if algo == "AZ" and matmul_precision != "f32":
             raise NotImplementedError("matmul_precision applies to PPO only (AlphaZero evaluates its policy inside the tree search)")
+        if algo == "AZ" and update_precision != "f32":
+            raise NotImplementedError("update_precision applies to PPO only (the AlphaZero update runs in f32 PyTorch)")
         cfg = dict(self.env_config)
         kind = _ENV_KINDS[self.env.cls_name]
         kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset")}
         if algo == "PPO":
             kw["matmul_precision"] = matmul_precision
+            kw["update_precision"] = update_precision
         trainer = (ppo.PPO if algo == "PPO" else ppo.AlphaZero)(kind, cfg["num_qubits"], cfg["gateset"], self.policy, self.rl_config, device=self.device, seed=seed, **kw)
         if hasattr(self.env, "difficulty"):
             self.env.difficulty = initial_difficulty                # rl/synthesis.py:129 (a reference *Gym object; a SynthSpec owns no env)
