@@ -129,6 +129,11 @@ QG_API int32_t qg_get_difficulty(const qg_engine* e);                /* Env::get
  * `count` envs (synth search).  depth := max_depth, internals reset. */
 QG_API int qg_set_state(qg_engine* e, const int64_t* states_host, int64_t stride, int64_t first,
                         int64_t count, int32_t broadcast, qg_stream stream);
+/* Env::set_state for groups of envs (a search over many targets): payload p (at states_host + p*stride) is loaded into envs
+ * [p*group, (p+1)*group) for p < num_states; envs past num_states*group are untouched.  Each payload is packed once on the host.
+ * QG_ERR_INVALID for group <= 0 or num_states*group outside the batch. */
+QG_API int qg_set_state_grouped(qg_engine* e, const int64_t* states_host, int64_t stride, int64_t num_states, int64_t group,
+                                qg_stream stream);
 /* Env::reset for every env: identity scrambled by `difficulty` random gates drawn from
  * Philox4x32-10(seed; env id, draw index) (permutation.rs:175-192, linear_function.rs:285-300,
  * clifford.rs:306-319, pauli.rs:554-586).  env ids are first_env_id + local index so a sharded batch
@@ -262,6 +267,13 @@ QG_API int qg_search_step(qg_engine* e, const float* weights_dev, int32_t determ
  * (max wins: successful first, then highest return, then lowest id).  Writes the winning key to
  * *best_key_host and the winner's local env index to *best_env_host (-1 if B == 0). */
 QG_API int qg_search_best(qg_engine* e, int64_t* best_key_host, int64_t* best_env_host, qg_stream stream);
+/* Per-target best rollout of a search over many targets (each target loaded into its own group of rollouts by qg_set_state_grouped):
+ * for every group g of envs [g*group, (g+1)*group), g < num_groups, keys_dev[g] = the largest qg_search_best key of the group, and if
+ * that rollout succeeded, actions_dev[g][0..len) its Env::solution with len_dev[g] = len (len_dev[g] = 0: no rollout of the group
+ * succeeded; -(length): the solution is longer than cap and nothing is written).  keys_dev int64[num_groups], actions_dev
+ * uint32[num_groups][cap], len_dev int32[num_groups].  One kernel, asynchronous on the stream, no host synchronisation. */
+QG_API int qg_search_best_grouped(qg_engine* e, int64_t group, int64_t num_groups, int64_t* keys_dev, uint32_t* actions_dev, int32_t cap,
+                                  int32_t* len_dev, qg_stream stream);
 QG_API int qg_read_returns(qg_engine* e, float* returns_dev, qg_stream stream);
 /* End of a search sharded over GPUs (rl/synthesis.py:112-126 `solve(..., num_searches)` with the rollouts split over ranks, each rank's
  * qg_search_begin given its first GLOBAL rollout id): the on-GPU best-rollout reduction of this rank, then — given an NCCL communicator —

@@ -34,13 +34,7 @@ __global__ void k_copy_f32(const float* src, float* dst, int64_t n) {
     if (i < n) dst[i] = src[i];
 }
 
-// ---- best-rollout reduction (synth search): arg-max of a packed key ----------------------------------
-// key = success<<62 | orderable_u32(return)<<30 | (2^30-1 - global rollout id)
-__device__ __forceinline__ unsigned long long rollout_key(bool success, float ret, int64_t gid) {
-    uint32_t u = __float_as_uint(ret);
-    u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);      // order-preserving map f32 -> u32
-    return ((unsigned long long)(success ? 1 : 0) << 62) | ((unsigned long long)u << 30) | (unsigned long long)((0x3FFFFFFFll - gid) & 0x3FFFFFFFll);
-}
+// ---- best-rollout reduction (synth search): arg-max of the packed key rollout_key (qg_kernels.cuh) ----------------------------------
 __global__ void k_best(const __grid_constant__ DevCfg c, unsigned long long* best) {
     const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     unsigned long long key = 0;

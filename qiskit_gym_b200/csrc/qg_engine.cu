@@ -184,14 +184,14 @@ int qg::launch_step(qg_engine* e, int mode, StepArgs a, cudaStream_t st, int64_t
 
 namespace {
 
-int launch_load(qg_engine* e, int64_t first, int64_t count, int broadcast, uint32_t depth_init, cudaStream_t st) {
+int launch_load(qg_engine* e, int64_t first, int64_t count, int64_t group, uint32_t depth_init, cudaStream_t st) {
     if (count <= 0) return QG_OK;
     const unsigned grid = (unsigned)((count + 255) / 256);
     switch (e->L.kind) {
-        case QG_ENV_PERMUTATION: k_load<QG_ENV_PERMUTATION><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, broadcast, depth_init); break;
-        case QG_ENV_LINEAR_FUNCTION: k_load<QG_ENV_LINEAR_FUNCTION><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, broadcast, depth_init); break;
-        case QG_ENV_CLIFFORD: k_load<QG_ENV_CLIFFORD><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, broadcast, depth_init); break;
-        default: k_load<QG_ENV_PAULI_NETWORK><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, broadcast, depth_init); break;
+        case QG_ENV_PERMUTATION: k_load<QG_ENV_PERMUTATION><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, group, depth_init); break;
+        case QG_ENV_LINEAR_FUNCTION: k_load<QG_ENV_LINEAR_FUNCTION><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, group, depth_init); break;
+        case QG_ENV_CLIFFORD: k_load<QG_ENV_CLIFFORD><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, group, depth_init); break;
+        default: k_load<QG_ENV_PAULI_NETWORK><<<grid, 256, 0, st>>>(e->dc, e->staged, e->L.PW, first, count, group, depth_init); break;
     }
     CUDA_OK(cudaGetLastError());
     return QG_OK;
@@ -396,7 +396,7 @@ int qg_create(const qg_config* cfg, int32_t device, int64_t batch, void* workspa
     // constructor state: identity, depth 1, success, reward 1.0 (permutation.rs:75-98, clifford.rs:205-236, pauli.rs:354-409)
     ce = cudaMemcpy(e->staged, ident.data(), (size_t)L.PW * 4, cudaMemcpyHostToDevice);
     if (ce != cudaSuccess) { set_error(std::string("engine init: ") + cudaGetErrorString(ce)); return fail(QG_ERR_CUDA); }
-    rc = launch_load(e, 0, batch, 1, 1u, 0);
+    rc = launch_load(e, 0, batch, batch, 1u, 0);
     if (rc != QG_OK) return fail(rc);
     ce = cudaStreamSynchronize(0);
     if (ce != cudaSuccess) { set_error(std::string("engine init: ") + cudaGetErrorString(ce)); return fail(QG_ERR_CUDA); }
@@ -439,12 +439,11 @@ int qg_set_difficulty(qg_engine* e, int32_t difficulty) {
 }
 int32_t qg_get_difficulty(const qg_engine* e) { return e ? e->cfg.difficulty : 0; }
 
-int qg_set_state(qg_engine* e, const int64_t* states_host, int64_t stride, int64_t first, int64_t count, int32_t broadcast, qg_stream stream) {
-    if (!e || !states_host) { set_error("null argument"); return QG_ERR_INVALID; }
-    if (first < 0 || count < 0 || first + count > e->B) { set_error("set_state: env range outside the batch"); return QG_ERR_INVALID; }
+namespace {
+// `payloads` payloads packed once each, env first + i loads payload i / group
+int set_state_impl(qg_engine* e, const int64_t* states_host, int64_t stride, int64_t first, int64_t count, int64_t payloads, int64_t group, qg_stream stream) {
     if (count == 0) return QG_OK;
     CUDA_OK(cudaSetDevice(e->device));
-    const int64_t payloads = broadcast ? 1 : count;
     int rc = ensure_host_staging(e, payloads * e->L.PW);
     if (rc != QG_OK) return rc;
     for (int64_t i = 0; i < payloads; ++i) {
@@ -455,10 +454,26 @@ int qg_set_state(qg_engine* e, const int64_t* states_host, int64_t stride, int64
     }
     cudaStream_t st = (cudaStream_t)stream;
     CUDA_OK(cudaMemcpyAsync(e->staged, e->h_staged, (size_t)payloads * e->L.PW * 4, cudaMemcpyHostToDevice, st));
-    rc = launch_load(e, first, count, broadcast ? 1 : 0, (uint32_t)e->cfg.max_depth, st);
+    rc = launch_load(e, first, count, group, (uint32_t)e->cfg.max_depth, st);
     if (rc != QG_OK) return rc;
     CUDA_OK(cudaStreamSynchronize(st));   // the pinned staging buffer is reused by the next call
     return QG_OK;
+}
+}  // namespace
+
+int qg_set_state(qg_engine* e, const int64_t* states_host, int64_t stride, int64_t first, int64_t count, int32_t broadcast, qg_stream stream) {
+    if (!e || !states_host) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (first < 0 || count < 0 || first + count > e->B) { set_error("set_state: env range outside the batch"); return QG_ERR_INVALID; }
+    // broadcast: one payload read by all `count` envs; otherwise one payload per env
+    return set_state_impl(e, states_host, stride, first, count, broadcast ? 1 : count, broadcast ? count : 1, stream);
+}
+
+int qg_set_state_grouped(qg_engine* e, const int64_t* states_host, int64_t stride, int64_t num_states, int64_t group, qg_stream stream) {
+    if (!e || !states_host) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (group <= 0 || num_states < 0 || num_states > e->B / group) {
+        set_error("set_state_grouped: group must be >= 1 and num_states * group within the batch"); return QG_ERR_INVALID;
+    }
+    return set_state_impl(e, states_host, stride, 0, num_states * group, num_states, group, stream);
 }
 
 namespace {

@@ -23,8 +23,7 @@ namespace qg {
 
 // ---- Env::solution for many envs ------------------------------------------------------------------------------------------------
 // One thread per env walks its column of the slot-major log sol[slot][env] (consecutive threads read consecutive addresses) and writes its
-// env-major row.  Entries logged while the env was inverted carry bit 31 (LinearFunction / Clifford / Permutation): they follow the others,
-// in reverse order (clifford.rs:376-381).  PauliNetwork words are emitted as logged (bit 31 there is ROTATION_MARKER, pauli.rs:685-719).
+// env-major row (write_solution, qg_kernels.cuh).
 __global__ void k_solutions(const __grid_constant__ DevCfg c, int64_t first, int64_t count, uint32_t* __restrict__ out, int cap, int32_t* __restrict__ len) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
@@ -32,15 +31,36 @@ __global__ void k_solutions(const __grid_constant__ DevCfg c, int64_t first, int
     const int n = (int)(c.rec[(size_t)HD_FLAGS * c.Bpad + env] >> FL_LEN_SHIFT);
     if (n > cap) { len[i] = -n; return; }
     len[i] = n;
-    uint32_t* row = out + (size_t)i * cap;
-    const uint32_t* col = c.sol + env;
-    if (c.kind == QG_ENV_PAULI_NETWORK) {
-        for (int k = 0; k < n; ++k) row[k] = col[(size_t)k * c.Bpad];
-        return;
+    write_solution(c, env, n, out + (size_t)i * cap);
+}
+
+// ---- per-target winners of a multi-target search --------------------------------------------------------------------------------------
+// One warp per group g of `group` consecutive envs: the lanes stride over the group's rollouts, a shuffle reduction finds the largest
+// rollout_key (keys are unique, so the result does not depend on the order), and lane 0 writes the key and, if the winner succeeded, its
+// Env::solution (len = 0: no success; len = -(length): longer than cap, nothing written).
+constexpr int kGroupWarps = 8;
+__global__ void __launch_bounds__(kGroupWarps * 32) k_best_grouped(const __grid_constant__ DevCfg c, int64_t group, int64_t num_groups,
+                                                                    int64_t* __restrict__ keys, uint32_t* __restrict__ actions, int cap,
+                                                                    int32_t* __restrict__ len) {
+    const int64_t g = (int64_t)blockIdx.x * kGroupWarps + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (g >= num_groups) return;
+    const int64_t e0 = g * group;
+    unsigned long long key = 0;
+    for (int64_t j = lane; j < group; j += 32) {
+        const int64_t env = e0 + j;
+        const unsigned long long k = rollout_key((c.rec[(size_t)HD_FLAGS * c.Bpad + env] & FL_SUCCESS) != 0, c.ret[env], c.first_id + env);
+        key = k > key ? k : key;
     }
-    int w = 0;
-    for (int k = 0; k < n; ++k) { const uint32_t v = col[(size_t)k * c.Bpad]; if (!(v & 0x80000000u)) row[w++] = v; }
-    for (int k = n - 1; k >= 0; --k) { const uint32_t v = col[(size_t)k * c.Bpad]; if (v & 0x80000000u) row[w++] = v & 0x7FFFFFFFu; }
+    for (int o = 16; o > 0; o >>= 1) { const unsigned long long other = __shfl_xor_sync(0xFFFFFFFFu, key, o); key = other > key ? other : key; }
+    if (lane != 0) return;
+    keys[g] = (int64_t)key;
+    if (!((key >> 62) & 1ull)) { len[g] = 0; return; }
+    const int64_t env = (0x3FFFFFFFll - (int64_t)(key & 0x3FFFFFFFull)) - c.first_id;
+    const int n = (int)(c.rec[(size_t)HD_FLAGS * c.Bpad + env] >> FL_LEN_SHIFT);
+    if (n > cap) { len[g] = -n; return; }
+    len[g] = n;
+    write_solution(c, env, n, actions + (size_t)g * cap);
 }
 
 // ---- end of a sharded search -------------------------------------------------------------------------------------------------------
@@ -55,15 +75,8 @@ __global__ void k_pack_winner(const __grid_constant__ DevCfg c, const unsigned l
     if (env < 0 || env >= c.B) return;
     const int n = (int)(c.rec[(size_t)HD_FLAGS * c.Bpad + env] >> FL_LEN_SHIFT);
     if (n > cap) return;
-    const uint32_t* col = c.sol + env;
-    uint32_t* out = row + kFinHdr;
-    int w = 0;
-    if (c.kind == QG_ENV_PAULI_NETWORK) { for (int k = 0; k < n; ++k) out[w++] = col[(size_t)k * c.Bpad]; }
-    else {
-        for (int k = 0; k < n; ++k) { const uint32_t v = col[(size_t)k * c.Bpad]; if (!(v & 0x80000000u)) out[w++] = v; }
-        for (int k = n - 1; k >= 0; --k) { const uint32_t v = col[(size_t)k * c.Bpad]; if (v & 0x80000000u) out[w++] = v & 0x7FFFFFFFu; }
-    }
-    row[2] = (uint32_t)w;
+    write_solution(c, env, n, row + kFinHdr);
+    row[2] = (uint32_t)n;
 }
 // rows [world][row_words] -> the row with the largest key into out (keys are unique: they embed the global rollout id)
 __global__ void k_pick_winner(const uint32_t* __restrict__ rows, int world, int row_words, uint32_t* __restrict__ out) {
@@ -220,6 +233,21 @@ int qg_solutions_host(qg_engine* e, int64_t first, int64_t count, uint32_t* out_
     CUDA_OK(cudaMemcpyAsync(len_host, e->bulk_len, (size_t)count * 4, cudaMemcpyDeviceToHost, st));
     CUDA_OK(cudaMemcpyAsync(out_host, e->bulk_sol, (size_t)count * cap * 4, cudaMemcpyDeviceToHost, st));
     CUDA_OK(cudaStreamSynchronize(st));
+    return QG_OK;
+}
+
+int qg_search_best_grouped(qg_engine* e, int64_t group, int64_t num_groups, int64_t* keys_dev, uint32_t* actions_dev, int32_t cap, int32_t* len_dev,
+                           qg_stream stream) {
+    if (!e) { set_error("null engine"); return QG_ERR_INVALID; }
+    if (group <= 0 || num_groups < 0 || num_groups > e->B / group || cap < 1) {
+        set_error("qg_search_best_grouped: group must be >= 1, num_groups * group within the batch and cap >= 1"); return QG_ERR_INVALID;
+    }
+    if (num_groups == 0) return QG_OK;
+    if (!keys_dev || !actions_dev || !len_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    CUDA_OK(cudaSetDevice(e->device));
+    k_best_grouped<<<(unsigned)((num_groups + kGroupWarps - 1) / kGroupWarps), kGroupWarps * 32, 0, (cudaStream_t)stream>>>(e->dc, group, num_groups, keys_dev,
+                                                                                                                          actions_dev, cap, len_dev);
+    CUDA_OK(cudaGetLastError());
     return QG_OK;
 }
 
@@ -490,13 +518,7 @@ namespace qg {
 __global__ void k_best_key(const __grid_constant__ DevCfg c, unsigned long long* best) {
     const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     unsigned long long key = 0;
-    if (env < c.B) {
-        const uint32_t f = c.rec[(size_t)HD_FLAGS * c.Bpad + env];
-        uint32_t u = __float_as_uint(c.ret[env]);
-        u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);      // order-preserving map f32 -> u32 (qg_aux_kernels.cuh rollout_key)
-        const int64_t gid = c.first_id + env;
-        key = ((unsigned long long)((f & FL_SUCCESS) ? 1 : 0) << 62) | ((unsigned long long)u << 30) | (unsigned long long)((0x3FFFFFFFll - gid) & 0x3FFFFFFFll);
-    }
+    if (env < c.B) key = rollout_key((c.rec[(size_t)HD_FLAGS * c.Bpad + env] & FL_SUCCESS) != 0, c.ret[env], c.first_id + env);
     for (int o = 16; o > 0; o >>= 1) { const unsigned long long other = __shfl_xor_sync(0xFFFFFFFFu, key, o); key = other > key ? other : key; }
     if ((threadIdx.x & 31) == 0 && key) atomicMax(best, key);
 }

@@ -1163,13 +1163,14 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, INV == 32 ? 8 : 16) k_step(
 }
 
 // ---- load (set_state / constructor) --------------------------------------------------------------
-// staged: [count][PW] words per env = state words (+ PauliNetwork extras); broadcast: every env reads payload 0.
+// staged: payloads of PW words = state words (+ PauliNetwork extras); env first + i reads payload i / group (group = 1: one payload per
+// env; group = count: every env reads payload 0; qg_set_state_grouped: one payload per group of rollouts).
 template <int KIND>
-__global__ void k_load(const __grid_constant__ DevCfg c, const uint32_t* __restrict__ staged, int PW, int64_t first, int64_t count, int broadcast, uint32_t depth_init) {
+__global__ void k_load(const __grid_constant__ DevCfg c, const uint32_t* __restrict__ staged, int PW, int64_t first, int64_t count, int64_t group, uint32_t depth_init) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
     const int64_t env = first + i;
-    const uint32_t* src = staged + (size_t)(broadcast ? 0 : i) * PW;
+    const uint32_t* src = staged + (size_t)(i / group) * PW;
     auto put = [&](int w, uint32_t v) { c.rec[(size_t)w * c.Bpad + env] = v; };
     bool ok = true;
     if (KIND == QG_ENV_PERMUTATION) {
@@ -1190,6 +1191,27 @@ __global__ void k_load(const __grid_constant__ DevCfg c, const uint32_t* __restr
     put(HD_NCNOTS, 0); put(HD_NGATES, 0); put(HD_LAYERS, 0);
     put(HD_REWARD, __float_as_uint(ok ? 1.0f : 0.0f));
     put(HD_TICK, 0);
+}
+
+// ---- read-out of a search (k_best, k_best_grouped, k_solutions, k_pack_winner) ------------------------------------------------------
+// key = success<<62 | orderable_u32(return)<<30 | (2^30-1 - global rollout id): the largest key is the best rollout
+__device__ __forceinline__ unsigned long long rollout_key(bool success, float ret, int64_t gid) {
+    uint32_t u = __float_as_uint(ret);
+    u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);      // order-preserving map f32 -> u32
+    return ((unsigned long long)(success ? 1 : 0) << 62) | ((unsigned long long)u << 30) | (unsigned long long)((0x3FFFFFFFll - gid) & 0x3FFFFFFFll);
+}
+// Env::solution of `env` (its n logged entries) into row[0..n): the column of the slot-major log sol[slot][env], entries logged while the
+// env was inverted (bit 31: LinearFunction / Clifford / Permutation) after the others, in reverse order (clifford.rs:376-381); PauliNetwork
+// words as logged (bit 31 there is ROTATION_MARKER, pauli.rs:685-719).
+__device__ __forceinline__ void write_solution(const DevCfg& c, int64_t env, int n, uint32_t* __restrict__ row) {
+    const uint32_t* col = c.sol + env;
+    if (c.kind == QG_ENV_PAULI_NETWORK) {
+        for (int k = 0; k < n; ++k) row[k] = col[(size_t)k * c.Bpad];
+        return;
+    }
+    int w = 0;
+    for (int k = 0; k < n; ++k) { const uint32_t v = col[(size_t)k * c.Bpad]; if (!(v & 0x80000000u)) row[w++] = v; }
+    for (int k = n - 1; k >= 0; --k) { const uint32_t v = col[(size_t)k * c.Bpad]; if (v & 0x80000000u) row[w++] = v & 0x7FFFFFFFu; }
 }
 
 // ---- reset (Permutation / LinearFunction / Clifford): identity scrambled by `difficulty` Philox-drawn gates

@@ -105,23 +105,34 @@ class BatchedEnv:
         return self._twists
 
     # ------------------------------------------------------------------ state in
+    @staticmethod
+    def _payload_rows(states) -> np.ndarray:
+        """A sequence / int64 array of payloads -> int64 [count, stride], shorter payloads zero-padded."""
+        if isinstance(states, np.ndarray) and states.ndim == 2:
+            return np.ascontiguousarray(states, dtype=np.int64)
+        arr = np.zeros((len(states), max((len(s) for s in states), default=1)), dtype=np.int64)
+        for i, s in enumerate(states):
+            arr[i, : len(s)] = s
+        return arr
+
     def set_state(self, states, first: int = 0):
         """Env::set_state.  `states`: one payload (list[int]) => loaded into every env, or a sequence /
         int64 array of per-env payloads."""
-        if isinstance(states, np.ndarray) and states.ndim == 2:
-            arr = np.ascontiguousarray(states, dtype=np.int64)
+        if (isinstance(states, np.ndarray) and states.ndim == 2) or (len(states) > 0 and isinstance(states[0], (list, tuple, np.ndarray))):
+            arr = self._payload_rows(states)
             count, stride, bcast = arr.shape[0], arr.shape[1], 0
-        elif len(states) > 0 and isinstance(states[0], (list, tuple, np.ndarray)):
-            stride = max(len(s) for s in states)
-            arr = np.zeros((len(states), stride), dtype=np.int64)
-            for i, s in enumerate(states):
-                arr[i, : len(s)] = s
-            count, bcast = len(states), 0
         else:
             arr = np.asarray(list(states), dtype=np.int64).reshape(1, -1)
             count, stride, bcast = self.batch - first, arr.shape[1], 1
         with torch.cuda.device(self.device):
             check(lib().qg_set_state(self._h, arr.ctypes.data_as(C.c_void_p), stride, first, count, bcast, self._stream()))
+
+    def set_state_grouped(self, states, group: int):
+        """Env::set_state for groups of envs (qg_set_state_grouped): payload p of `states` (a sequence / int64 array of payloads) goes
+        to envs [p * group, (p + 1) * group); envs past len(states) * group are untouched."""
+        arr = self._payload_rows(states)
+        with torch.cuda.device(self.device):
+            check(lib().qg_set_state_grouped(self._h, arr.ctypes.data_as(C.c_void_p), arr.shape[1], arr.shape[0], int(group), self._stream()))
 
     def reset(self, seed: int = 0, first_env_id: int = 0):
         check(lib().qg_reset(self._h, C.c_uint64(seed & (2**64 - 1)), first_env_id, self._stream()))
@@ -467,6 +478,20 @@ class BatchedEnv:
         key, env = C.c_int64(), C.c_int64()
         check(lib().qg_search_best(self._h, C.byref(key), C.byref(env), self._stream()))
         return key.value, env.value
+
+    def search_best_grouped(self, group: int, num_groups: int, cap: int | None = None, out: torch.Tensor | None = None):
+        """Best rollout of each group of `group` consecutive envs (qg_search_best_grouped), on the device and without a host
+        synchronisation: (keys int64 [num_groups], lens int32 [num_groups], actions int32 [num_groups, cap]); lens[g] = 0 when no rollout
+        of group g succeeded, -(length) when its solution is longer than cap.  `out`: an 8-byte aligned int32 device tensor of at least
+        num_groups * (3 + cap) elements that the three are views of (so that one copy brings all of them to the host)."""
+        if cap is None:
+            cap = max(int(self.cfg.solution_capacity) or (int(self.cfg.max_depth) + 16), 1)
+        G, need = int(num_groups), int(num_groups) * (3 + int(cap))
+        flat = torch.empty(max(need, 2), dtype=torch.int32, device=self.device) if out is None else out
+        assert flat.dtype == torch.int32 and flat.is_cuda and flat.is_contiguous() and flat.numel() >= need and flat.data_ptr() % 8 == 0
+        keys, lens, actions = flat[: 2 * G].view(torch.int64), flat[2 * G: 3 * G], flat[3 * G: need].view(G, int(cap))
+        check(lib().qg_search_best_grouped(self._h, int(group), G, _dptr(keys), _dptr(actions), int(cap), _dptr(lens), self._stream()))
+        return keys, lens, actions
 
     def returns(self):
         out = torch.zeros(self.batch, dtype=torch.float32, device=self.device)

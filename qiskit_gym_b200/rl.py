@@ -16,7 +16,7 @@ import json
 
 import torch
 
-from .search import BasicPolicy, RolloutSearch
+from .search import BasicPolicy, RolloutSearch, chunk_plan
 from .specs import SynthSpec
 
 _ENV_KINDS = {"PermutationEnv": 0, "LinearFunctionEnv": 1, "CliffordEnv": 2, "PauliNetworkEnv": 3}
@@ -81,19 +81,26 @@ class RLSynthesis:
                 torch.save(self.policy.state_dict(), f)
 
     # ---- synthesis ------------------------------------------------------------------------------------
-    def _search(self, num_searches: int) -> RolloutSearch:
+    def _search(self, num_searches: int, targets_per_launch: int | None = None) -> RolloutSearch:
+        """The cached search of `num_searches` rollouts per target: the single-target one, or with targets_per_launch the one solve_many
+        uses (rebuilt only when a call needs more targets per launch than it holds)."""
         from .policy import weights_version
-        rs = self._searches.get(num_searches)
+        key = num_searches if targets_per_launch is None else ("many", num_searches)
+        rs = self._searches.get(key)
         if rs is not None and getattr(rs, "fused", None) is not None and rs.fused.version != weights_version(self.policy):
             rs = None                                    # the cached search captured older weights (load_state_dict after the first synth)
+        if rs is not None and targets_per_launch is not None and rs.targets_per_launch < targets_per_launch:
+            rs = None
         if rs is None:
+            self._searches.pop(key, None)                # (frees the old engine before the new one allocates)
             cfg = dict(self.env_config)
             kind = _ENV_KINDS[self.env.cls_name]
             kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset", "max_depth", "add_perms")}
 
             def make(backend):
                 return RolloutSearch(kind, cfg["num_qubits"], cfg["gateset"], self.policy, num_searches, device=self.device,
-                                     max_depth=cfg.get("max_depth", 128), add_perms=False, policy_backend=backend, **kw)
+                                     max_depth=cfg.get("max_depth", 128), add_perms=False, policy_backend=backend,
+                                     targets_per_launch=targets_per_launch or 1, **kw)
             try:
                 rs = make("persistent")
                 rs.check_supported()
@@ -101,7 +108,7 @@ class RLSynthesis:
                 # outside the one-launch search's limits (Permutation wider than 64 qubits, a layer wider than 1024, policy + env larger
                 # than one SM's shared memory): the PyTorch policy on dense observations has none of them
                 rs = make("torch")
-            self._searches[num_searches] = rs
+            self._searches[key] = rs
         return rs
 
     def _mcts(self, num_searches: int, num_mcts_searches: int, C: float):
@@ -125,6 +132,39 @@ class RLSynthesis:
                 raise NotImplementedError("max_expand_depth != 1 is not supported by the device tree search (mcts.py)")
             return self._mcts(int(num_searches), int(num_mcts_searches), float(C)).solve(state, deterministic=deterministic, seed=seed).actions
         return self._search(int(num_searches)).solve(state, deterministic=deterministic, seed=seed).actions
+
+    def solve_many(self, states, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
+                   max_rollouts: int = 65536):
+        """`solve` for many targets in few launches: a list with, for each state, the action list of its best successful rollout or None.
+        Target t's result is that of solve(states[t]) on rollout ids t*num_searches .. (t+1)*num_searches - 1 (search.RolloutSearch.solve_many),
+        so solve_many([x])[0] == solve(x).  Up to max_rollouts rollouts run per launch (the one-launch search keeps ~4 KB of first-layer
+        accumulators per rollout at the default network: 65 536 rollouts ~ 256 MB)."""
+        if num_mcts_searches:
+            raise NotImplementedError("solve_many runs rollout searches only (num_mcts_searches = 0): use solve() for the tree search")
+        states = list(states)
+        num_searches = int(num_searches)
+        if num_searches < 1:
+            raise ValueError("num_searches must be >= 1")
+        chunk_plan(len(states), 1, num_searches)         # ValueError for targets x rollouts >= 2^30, before anything is allocated
+        if not states:
+            return []
+        tpl = min(len(states), max(1, int(max_rollouts) // num_searches))
+        res = self._search(num_searches, tpl).solve_many(states, deterministic=deterministic, seed=seed)
+        return [r.actions for r in res]
+
+    def synth_many(self, inputs, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
+                   max_rollouts: int = 65536):
+        """`synth` for many inputs (solve_many): a list of circuits (or gate lists), None where a target has no successful rollout."""
+        inputs = list(inputs)
+        actions = self.solve_many([self.env.get_state(x) for x in inputs], deterministic, num_searches, num_mcts_searches, seed, max_rollouts)
+        out = []
+        for x, a in zip(inputs, actions):
+            if a is None:
+                out.append(None)
+                continue
+            self.env.get_state(x)                        # the env object's per-target state (PauliNetwork rotation parameters), as synth leaves it
+            out.append(self.env.build_circuit_from_solution(a, x))
+        return out
 
     def synth(self, input, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
               max_expand_depth: int = 1, seed: int = 0):

@@ -16,8 +16,10 @@ from __future__ import annotations
 import time
 from dataclasses import dataclass
 
+import numpy as np
 import torch
 
+from . import _abi
 from .engine import BatchedEnv
 
 KEY_SUCCESS_BIT = 62
@@ -73,6 +75,24 @@ def decode_key(key: int):
     return bool((key >> KEY_SUCCESS_BIT) & 1), KEY_ID_MASK - (key & KEY_ID_MASK)
 
 
+def chunk_plan(num_targets: int, targets_per_launch: int, num_rollouts: int):
+    """How solve_many splits its targets: [(first target, targets in the chunk, first global rollout id)]; a chunk pads
+    targets_per_launch - count slots.  Rollout ids must fit the key's 30-bit id field: num_targets * num_rollouts < 2^30."""
+    if num_targets * num_rollouts >= 1 << 30:
+        raise ValueError(f"{num_targets} targets x {num_rollouts} rollouts do not fit the 30-bit rollout id of the search key (< 2^30 needed)")
+    return [(s, min(targets_per_launch, num_targets - s), s * num_rollouts) for s in range(0, num_targets, targets_per_launch)]
+
+
+def identity_payload(env_kind: int, num_qubits: int) -> list[int]:
+    """The env kind's identity as a set_state payload: a target that is solved when loaded (solve_many pads short chunks with it)."""
+    n = int(num_qubits)
+    if env_kind == _abi.ENV_PERMUTATION:
+        return list(range(n))
+    d = n if env_kind == _abi.ENV_LINEAR_FUNCTION else 2 * n
+    eye = np.eye(d, dtype=np.int64).ravel().tolist()
+    return [0] + eye if env_kind == _abi.ENV_PAULI_NETWORK else eye
+
+
 def reduce_best(local_key: int, local_solution, group=None, device=None):
     """Cross-rank best-rollout reduction in two collectives: an all-gather of (packed key, solution length) — the owner of the winning
     rollout is the rank holding the largest key; keys are unique, they embed the global rollout id — then the owner broadcasts its action
@@ -104,13 +124,20 @@ class RolloutSearch:
     """Device-resident `solve`: owns a BatchedEnv of `num_rollouts` rollouts on one GPU."""
 
     def __init__(self, env_kind, num_qubits, gateset, policy: torch.nn.Module, num_rollouts: int, device=None,
-                 max_depth: int = 128, use_cuda_graph: bool = True, policy_backend: str = "persistent", **env_kwargs):
+                 max_depth: int = 128, use_cuda_graph: bool = True, policy_backend: str = "persistent", targets_per_launch: int = 1,
+                 **env_kwargs):
         """policy_backend: "persistent" = the whole search in ONE kernel launch (qg_search_run: every CTA loops policy -> sample ->
         step for its 8 rollouts); "fused" = two launches per decision (policy.FusedPolicy + qg_search_step_bits) in a CUDA graph;
         "torch" = dense f32 observations + the PyTorch module (cuBLAS GEMMs, softmax).  "persistent" and "fused" take identical
-        decisions (same kernels' device code, same bits)."""
+        decisions (same kernels' device code, same bits).
+        targets_per_launch: solve_many searches that many targets together, each with its own `num_rollouts` rollouts (the engine
+        holds targets_per_launch * num_rollouts); solve() needs targets_per_launch == 1."""
         env_kwargs.setdefault("add_perms", False)
-        self.env = BatchedEnv(env_kind, num_qubits, gateset, num_rollouts, device=device, max_depth=max_depth, **env_kwargs)
+        if targets_per_launch < 1:
+            raise ValueError("targets_per_launch must be >= 1")
+        self.env_kind, self.num_qubits = env_kind, num_qubits
+        self.R, self.targets_per_launch = num_rollouts, targets_per_launch
+        self.env = BatchedEnv(env_kind, num_qubits, gateset, targets_per_launch * num_rollouts, device=device, max_depth=max_depth, **env_kwargs)
         self.policy = policy.to(self.env.device).eval()
         assert policy_backend in ("persistent", "fused", "torch")
         self.backend = policy_backend
@@ -119,7 +146,7 @@ class RolloutSearch:
             self.fused = FusedPolicy(self.policy, device=self.env.device)
             self.obs_bits = self.env.new_obs_bits()
         self.max_depth = max_depth
-        self.B = num_rollouts
+        self.B = targets_per_launch * num_rollouts
         dev = self.env.device
         self.probs = torch.zeros((self.B, self.env.num_actions()), dtype=torch.float32, device=dev)
         self.num_active = torch.zeros(1, dtype=torch.int32, device=dev)
@@ -150,9 +177,11 @@ class RolloutSearch:
         else:
             self.env.observe()
 
-    def _graph(self, deterministic):
-        g = self._graphs.get(deterministic)
-        if g is None:
+    def _graph(self, deterministic, params):
+        """The CUDA graph of one iteration.  Its launches carry the engine's seed and first rollout id as they were at capture (the
+        step kernel takes them by value), so a graph serves only searches with the same (seed, first rollout id): `params`."""
+        g, captured = self._graphs.get(deterministic, (None, None))
+        if g is None or captured != params:
             # warm-up outside capture (cuBLAS workspaces, lazy module init), on a scratch copy of the state
             self.env.snapshot()
             for _ in range(2):
@@ -163,7 +192,7 @@ class RolloutSearch:
             with torch.cuda.graph(g, stream=self._stream):
                 self._iteration(deterministic)
             self.env.restore()
-            self._graphs[deterministic] = g
+            self._graphs[deterministic] = (g, params)
         return g
 
     def _local_best(self, comm):
@@ -177,39 +206,90 @@ class RolloutSearch:
         ok, rid = decode_key(key)
         return key, (env.solution(idx) if (ok and idx >= 0) else None), False
 
+    def _search(self, load, deterministic, seed, first_rollout_id, check_every):
+        """One search on self._stream (the caller enters it): load() puts the targets into the rollouts, then the decisions run.
+        Returns the number of decision steps, or None for the one-launch search (its CTAs' counts are in self._decisions)."""
+        env = self.env
+        if self.backend == "persistent":
+            load()
+            env.search_begin(seed, first_rollout_id)
+            self._observe()
+            env.search_run(self.fused, self.obs_bits, self.probs, self.max_depth, deterministic=deterministic, decisions=self._decisions)
+            return None
+        load()
+        if self.use_graph:
+            env.search_begin(seed, first_rollout_id)        # (what the captured launches see)
+            g = self._graph(deterministic, (seed, first_rollout_id))
+            load()
+        env.search_begin(seed, first_rollout_id)
+        self._observe()
+        its = 0
+        while its < self.max_depth:
+            if self.use_graph:
+                g.replay()
+            else:
+                self._iteration(deterministic)
+            its += 1
+            if its % check_every == 0 and int(self.num_active.item()) == 0:
+                break
+        return its
+
     def solve(self, state, deterministic: bool = False, seed: int = 0, first_rollout_id: int = 0, check_every: int = 8,
               group=None, comm=None) -> SearchResult:
         """group: torch.distributed group for the Python-side cross-rank reduction (reduce_best); comm: an ncclComm_t handle for the
         C-side one (qg_search_finish); with neither, and torch.distributed initialised, the default group is used."""
+        if self.targets_per_launch != 1:
+            raise ValueError("solve() searches one target: use solve_many() on a search built with targets_per_launch > 1")
         env = self.env
         t0 = time.perf_counter()
-        if self.backend == "persistent":
-            with torch.cuda.stream(self._stream):
-                env.set_state(state)
-                env.search_begin(seed, first_rollout_id)
-                self._observe()
-                env.search_run(self.fused, self.obs_bits, self.probs, self.max_depth, deterministic=deterministic, decisions=self._decisions)
-                key, sol, reduced = self._local_best(comm)
-                its = int(self._decisions.max().item())
-            return self._finish(key, sol, its, t0, group, reduced)
         with torch.cuda.stream(self._stream):
-            env.set_state(state)                         # broadcast: every rollout starts from the target
-            if self.use_graph:
-                g = self._graph(deterministic)
-                env.set_state(state)
-            env.search_begin(seed, first_rollout_id)
-            self._observe()
-            its = 0
-            while its < self.max_depth:
-                if self.use_graph:
-                    g.replay()
-                else:
-                    self._iteration(deterministic)
-                its += 1
-                if its % check_every == 0 and int(self.num_active.item()) == 0:
-                    break
+            # broadcast: every rollout starts from the target
+            its = self._search(lambda: env.set_state(state), deterministic, seed, first_rollout_id, check_every)
             key, sol, reduced = self._local_best(comm)
+            if its is None:
+                its = int(self._decisions.max().item())
         return self._finish(key, sol, its, t0, group, reduced)
+
+    def solve_many(self, states, deterministic: bool = False, seed: int = 0, check_every: int = 8) -> list[SearchResult]:
+        """solve() for many targets, targets_per_launch of them per search.  Target t gets global rollout ids t*R .. t*R + R - 1
+        (R = num_rollouts), so its result equals solve(states[t], deterministic, seed, first_rollout_id=t*R) of a single-target search
+        with the same policy and backend, whatever targets_per_launch is.  A short last chunk fills its free slots with the env kind's
+        identity, which is final when loaded.  Each chunk: grouped load, the search, the per-target winner reduction on the device and
+        one device-to-host copy.  SearchResult.seconds is the chunk's wall time, .rollouts = R."""
+        states = list(states)
+        T, R = self.targets_per_launch, self.R
+        plan = chunk_plan(len(states), T, R)
+        env = self.env
+        cap = max(int(env.cfg.solution_capacity) or (self.max_depth + 16), 1)
+        words = T * (3 + cap) + 1                           # keys (2 words each), lengths, action rows, decision count
+        if getattr(self, "_win", None) is None or self._win.numel() != words:
+            self._win = torch.zeros(words, dtype=torch.int32, device=env.device)
+            self._win_host = torch.zeros(words, dtype=torch.int32, pin_memory=True)
+        pad = identity_payload(self.env_kind, self.num_qubits)
+        out = []
+        for start, count, first_id in plan:
+            t0 = time.perf_counter()
+            chunk = states[start: start + count] + [pad] * (T - count)
+            with torch.cuda.stream(self._stream):
+                its = self._search(lambda: env.set_state_grouped(chunk, R), deterministic, seed, first_id, check_every)
+                env.search_best_grouped(R, T, cap, out=self._win[: words - 1])
+                if its is None:
+                    torch.amax(self._decisions, dim=0, keepdim=True, out=self._win[words - 1:])
+                self._win_host.copy_(self._win, non_blocking=True)
+                self._stream.synchronize()
+            h = self._win_host.numpy()
+            keys, lens, rows = h[: 2 * T].view(np.int64), h[2 * T: 3 * T], h[3 * T: words - 1].view(np.uint32).reshape(T, cap)
+            if its is None:
+                its = int(h[words - 1])
+            dt = time.perf_counter() - t0
+            for j in range(count):
+                key = int(keys[j])
+                ok, rid = decode_key(key)
+                if ok and lens[j] < 0:
+                    raise ValueError(f"a solution is longer than cap={cap}")
+                out.append(SearchResult(actions=rows[j, : lens[j]].astype(np.int64).tolist() if ok else None, key=key, rollout_id=rid,
+                                        success=ok, iterations=its, seconds=dt, rollouts=R))
+        return out
 
     def _finish(self, key, sol, its, t0, group, reduced=False):
         env = self.env
