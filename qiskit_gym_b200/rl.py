@@ -16,7 +16,7 @@ import json
 
 import torch
 
-from .search import BasicPolicy, RolloutSearch, chunk_plan
+from .search import BasicPolicy, RolloutSearch, check_tensor_core_search, chunk_plan
 from .specs import SynthSpec
 
 _ENV_KINDS = {"PermutationEnv": 0, "LinearFunctionEnv": 1, "CliffordEnv": 2, "PauliNetworkEnv": 3}
@@ -81,11 +81,14 @@ class RLSynthesis:
                 torch.save(self.policy.state_dict(), f)
 
     # ---- synthesis ------------------------------------------------------------------------------------
-    def _search(self, num_searches: int, targets_per_launch: int | None = None) -> RolloutSearch:
+    def _search(self, num_searches: int, targets_per_launch: int | None = None, matmul_precision: str = "f32") -> RolloutSearch:
         """The cached search of `num_searches` rollouts per target: the single-target one, or with targets_per_launch the one solve_many
-        uses (rebuilt only when a call needs more targets per launch than it holds)."""
+        uses (rebuilt only when a call needs more targets per launch than it holds).  matmul_precision="tensor_core": the "tensor_core"
+        backend, cached under its own key (it never replaces the f32 search) and with no fall-back; it refreshes its weights itself."""
         from .policy import weights_version
         key = num_searches if targets_per_launch is None else ("many", num_searches)
+        if matmul_precision == "tensor_core":
+            key = ("tensor_core", key)
         rs = self._searches.get(key)
         if rs is not None and getattr(rs, "fused", None) is not None and rs.fused.version != weights_version(self.policy):
             rs = None                                    # the cached search captured older weights (load_state_dict after the first synth)
@@ -101,13 +104,16 @@ class RLSynthesis:
                 return RolloutSearch(kind, cfg["num_qubits"], cfg["gateset"], self.policy, num_searches, device=self.device,
                                      max_depth=cfg.get("max_depth", 128), add_perms=False, policy_backend=backend,
                                      targets_per_launch=targets_per_launch or 1, **kw)
-            try:
-                rs = make("persistent")
-                rs.check_supported()
-            except NotImplementedError:
-                # outside the one-launch search's limits (Permutation wider than 64 qubits, a layer wider than 1024, policy + env larger
-                # than one SM's shared memory): the PyTorch policy on dense observations has none of them
-                rs = make("torch")
+            if matmul_precision == "tensor_core":
+                rs = make("tensor_core")
+            else:
+                try:
+                    rs = make("persistent")
+                    rs.check_supported()
+                except NotImplementedError:
+                    # outside the one-launch search's limits (Permutation wider than 64 qubits, a layer wider than 1024, policy + env larger
+                    # than one SM's shared memory): the PyTorch policy on dense observations has none of them
+                    rs = make("torch")
             self._searches[key] = rs
         return rs
 
@@ -134,29 +140,38 @@ class RLSynthesis:
         return self._search(int(num_searches)).solve(state, deterministic=deterministic, seed=seed).actions
 
     def solve_many(self, states, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
-                   max_rollouts: int = 65536):
+                   max_rollouts: int = 65536, matmul_precision: str = "f32"):
         """`solve` for many targets in few launches: a list with, for each state, the action list of its best successful rollout or None.
         Target t's result is that of solve(states[t]) on rollout ids t*num_searches .. (t+1)*num_searches - 1 (search.RolloutSearch.solve_many),
         so solve_many([x])[0] == solve(x).  Up to max_rollouts rollouts run per launch (the one-launch search keeps ~4 KB of first-layer
-        accumulators per rollout at the default network: 65 536 rollouts ~ 256 MB)."""
+        accumulators per rollout at the default network: 65 536 rollouts ~ 256 MB).
+        matmul_precision: "f32" (the default: the searches of solve) or "tensor_core" (RolloutSearch's "tensor_core" backend: the policy on
+        tcgen05 tensor cores, for large launches).  The two round differently, so "tensor_core" results equal a single-target "tensor_core"
+        search, not solve(); it raises NotImplementedError where it cannot run (more than 127 actions, a Permutation wider than 64 qubits, a
+        device that is not sm_100) instead of falling back to another arithmetic."""
         if num_mcts_searches:
             raise NotImplementedError("solve_many runs rollout searches only (num_mcts_searches = 0): use solve() for the tree search")
+        if matmul_precision not in ("f32", "tensor_core"):
+            raise ValueError(f"matmul_precision must be f32 or tensor_core (got {matmul_precision!r})")
         states = list(states)
         num_searches = int(num_searches)
         if num_searches < 1:
             raise ValueError("num_searches must be >= 1")
         chunk_plan(len(states), 1, num_searches)         # ValueError for targets x rollouts >= 2^30, before anything is allocated
+        if matmul_precision == "tensor_core":
+            check_tensor_core_search(_ENV_KINDS[self.env.cls_name], self.env_config["num_qubits"], self.env.num_actions(), self.device)
         if not states:
             return []
         tpl = min(len(states), max(1, int(max_rollouts) // num_searches))
-        res = self._search(num_searches, tpl).solve_many(states, deterministic=deterministic, seed=seed)
+        res = self._search(num_searches, tpl, matmul_precision).solve_many(states, deterministic=deterministic, seed=seed)
         return [r.actions for r in res]
 
     def synth_many(self, inputs, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
-                   max_rollouts: int = 65536):
+                   max_rollouts: int = 65536, matmul_precision: str = "f32"):
         """`synth` for many inputs (solve_many): a list of circuits (or gate lists), None where a target has no successful rollout."""
         inputs = list(inputs)
-        actions = self.solve_many([self.env.get_state(x) for x in inputs], deterministic, num_searches, num_mcts_searches, seed, max_rollouts)
+        actions = self.solve_many([self.env.get_state(x) for x in inputs], deterministic, num_searches, num_mcts_searches, seed, max_rollouts,
+                                  matmul_precision)
         out = []
         for x, a in zip(inputs, actions):
             if a is None:

@@ -93,6 +93,19 @@ def identity_payload(env_kind: int, num_qubits: int) -> list[int]:
     return [0] + eye if env_kind == _abi.ENV_PAULI_NETWORK else eye
 
 
+def check_tensor_core_search(env_kind: int, num_qubits: int, num_actions: int, device=None):
+    """Raises NotImplementedError where the "tensor_core" search backend cannot run: more than 127 actions (the tensor-core head), a
+    Permutation wider than 64 qubits (no packed observations), a device that is not sm_100 (tcgen05)."""
+    if num_actions > 127:
+        raise NotImplementedError(f"the tensor-core search supports up to 127 actions (got {num_actions})")
+    if env_kind == _abi.ENV_PERMUTATION and num_qubits > 64:
+        raise NotImplementedError(f"the tensor-core search needs packed observations: a Permutation of {num_qubits} > 64 qubits has none")
+    if not torch.cuda.is_available():
+        raise RuntimeError("qiskit_gym_b200 needs a CUDA device (no CPU fallback)")
+    if torch.cuda.get_device_capability(device)[0] != 10:
+        raise NotImplementedError("the tensor-core search needs an sm_100 device (tcgen05)")
+
+
 def reduce_best(local_key: int, local_solution, group=None, device=None):
     """Cross-rank best-rollout reduction in two collectives: an all-gather of (packed key, solution length) — the owner of the winning
     rollout is the rank holding the largest key; keys are unique, they embed the global rollout id — then the owner broadcasts its action
@@ -130,27 +143,41 @@ class RolloutSearch:
         step for its 8 rollouts); "fused" = two launches per decision (policy.FusedPolicy + qg_search_step_bits) in a CUDA graph;
         "torch" = dense f32 observations + the PyTorch module (cuBLAS GEMMs, softmax).  "persistent" and "fused" take identical
         decisions (same kernels' device code, same bits).
+        "tensor_core" = the "fused" decision with the policy on tcgen05 tensor cores (policy.TensorCorePolicy with max_batch = the
+        engine's rollouts, no value head): observe bits -> qg_policy_tc_forward_bits -> qg_search_step_bits, in a CUDA graph.  It is
+        built for large batches (solve_many at tens of thousands of rollouts per launch) and is opt-in: its f16 hi+lo split arithmetic
+        rounds differently from the f32 backends, so its decisions are not theirs (the probabilities are within TensorCorePolicy's error
+        bound of the float64 module).  Each row's probabilities are bit-identical whatever the batch size and the other rows, so the
+        solve_many contract below holds among "tensor_core" searches.  NotImplementedError where it cannot run: more than 127 actions,
+        a Permutation wider than 64 qubits (no packed observations), a device that is not sm_100.  A weight update of `policy` (optimizer
+        step, load_state_dict) is copied into the handle in place before the next search (captured graphs stay valid).
         targets_per_launch: solve_many searches that many targets together, each with its own `num_rollouts` rollouts (the engine
         holds targets_per_launch * num_rollouts); solve() needs targets_per_launch == 1."""
         env_kwargs.setdefault("add_perms", False)
         if targets_per_launch < 1:
             raise ValueError("targets_per_launch must be >= 1")
+        assert policy_backend in ("persistent", "fused", "torch", "tensor_core")
         self.env_kind, self.num_qubits = env_kind, num_qubits
         self.R, self.targets_per_launch = num_rollouts, targets_per_launch
         self.env = BatchedEnv(env_kind, num_qubits, gateset, targets_per_launch * num_rollouts, device=device, max_depth=max_depth, **env_kwargs)
         self.policy = policy.to(self.env.device).eval()
-        assert policy_backend in ("persistent", "fused", "torch")
         self.backend = policy_backend
-        if policy_backend in ("fused", "persistent"):
-            from .policy import FusedPolicy
-            self.fused = FusedPolicy(self.policy, device=self.env.device)
-            self.obs_bits = self.env.new_obs_bits()
         self.max_depth = max_depth
         self.B = targets_per_launch * num_rollouts
         dev = self.env.device
+        if policy_backend in ("fused", "persistent"):
+            from .policy import FusedPolicy
+            self.fused = FusedPolicy(self.policy, device=dev)
+        if policy_backend == "tensor_core":
+            from .policy import TensorCorePolicy
+            check_tensor_core_search(env_kind, num_qubits, self.env.num_actions(), dev)
+            self.tcp = TensorCorePolicy(self.policy, max_batch=self.B, device=dev, with_value=False)
+        if policy_backend != "torch":
+            self.obs_bits = self.env.new_obs_bits()
         self.probs = torch.zeros((self.B, self.env.num_actions()), dtype=torch.float32, device=dev)
         self.num_active = torch.zeros(1, dtype=torch.int32, device=dev)
         self.use_graph = use_cuda_graph
+        self.hook = None            # tests: hook(probs, obs_bits) sees every decision's policy output before the step reads it (no graph)
         self._graphs = {}
         self._stream = torch.cuda.Stream(device=dev)
         self._decisions = torch.zeros((self.B + 7) // 8, dtype=torch.int32, device=dev)
@@ -162,8 +189,10 @@ class RolloutSearch:
             self.env.search_run(self.fused, self.obs_bits, self.probs, 0, deterministic=True, decisions=self._decisions)
 
     def _iteration(self, deterministic):
-        if self.backend == "fused":
-            self.fused.forward_bits(self.obs_bits, probs=self.probs)
+        if self.backend in ("fused", "tensor_core"):
+            (self.fused if self.backend == "fused" else self.tcp).forward_bits(self.obs_bits, probs=self.probs)
+            if self.hook is not None:
+                self.hook(self.probs, self.obs_bits)
             self.env.search_step_bits(self.probs, self.obs_bits, deterministic=deterministic, num_active=self.num_active)
             return
         with torch.no_grad():
@@ -172,10 +201,24 @@ class RolloutSearch:
         self.env.search_step(self.probs, deterministic=deterministic, obs=True, num_active=self.num_active)
 
     def _observe(self):
-        if self.backend in ("fused", "persistent"):
+        if self.backend != "torch":
             self.env.observe_bits(self.obs_bits)
         else:
             self.env.observe()
+
+    def _refresh_weights(self):
+        """"tensor_core": copies a weight update of self.policy into the handle in place, after the caller's stream's pending work (captured
+        graphs stay valid); a module of another shape, or whose parameters cannot be read in place, gets a new handle and new graphs."""
+        if self.backend != "tensor_core":
+            return
+        from .policy import TensorCorePolicy, weights_version
+        if not self.tcp.can_load(self.policy):
+            self._graphs = {}
+            self.tcp = TensorCorePolicy(self.policy, max_batch=self.B, device=self.env.device, with_value=False)
+        elif self.tcp.version != weights_version(self.policy):
+            self._stream.wait_stream(torch.cuda.current_stream(self.env.device))
+            with torch.cuda.stream(self._stream):
+                self.tcp.load_weights(self.policy)
 
     def _graph(self, deterministic, params):
         """The CUDA graph of one iteration.  Its launches carry the engine's seed and first rollout id as they were at capture (the
@@ -217,7 +260,8 @@ class RolloutSearch:
             env.search_run(self.fused, self.obs_bits, self.probs, self.max_depth, deterministic=deterministic, decisions=self._decisions)
             return None
         load()
-        if self.use_graph:
+        use_graph = self.use_graph and self.hook is None
+        if use_graph:
             env.search_begin(seed, first_rollout_id)        # (what the captured launches see)
             g = self._graph(deterministic, (seed, first_rollout_id))
             load()
@@ -225,7 +269,7 @@ class RolloutSearch:
         self._observe()
         its = 0
         while its < self.max_depth:
-            if self.use_graph:
+            if use_graph:
                 g.replay()
             else:
                 self._iteration(deterministic)
@@ -242,6 +286,7 @@ class RolloutSearch:
             raise ValueError("solve() searches one target: use solve_many() on a search built with targets_per_launch > 1")
         env = self.env
         t0 = time.perf_counter()
+        self._refresh_weights()
         with torch.cuda.stream(self._stream):
             # broadcast: every rollout starts from the target
             its = self._search(lambda: env.set_state(state), deterministic, seed, first_rollout_id, check_every)
@@ -266,6 +311,7 @@ class RolloutSearch:
             self._win = torch.zeros(words, dtype=torch.int32, device=env.device)
             self._win_host = torch.zeros(words, dtype=torch.int32, pin_memory=True)
         pad = identity_payload(self.env_kind, self.num_qubits)
+        self._refresh_weights()
         out = []
         for start, count, first_id in plan:
             t0 = time.perf_counter()
