@@ -463,6 +463,17 @@ QG_API int qg_mcts_backup(const qg_mcts_tree* t, const float* prior_dev, const f
                           const uint8_t* done_dev, qg_stream stream);
 /* weights_dev float[num_trees][num_actions] = root visit counts / their sum (all zero for a tree without simulations). */
 QG_API int qg_mcts_root_weights(const qg_mcts_tree* t, float* weights_dev, qg_stream stream);
+/* Tree reuse between decisions (protocol in csrc/qg_mcts.cu), after the rollouts' qg_search_step with chosen_dev int32[num_trees]: tree i
+ * is re-rooted at c = child[0][chosen[i]] when chosen[i] >= 0, that child exists and its record in `pool` (slot i * node_cap + c) equals env
+ * i's record in `rollouts` (solution-log length masked).  It then keeps the first keep_nodes (1..node_cap) nodes of c's subtree in creation
+ * order, renumbered in that order (c becomes node 0), with their pool records; an edge whose child was dropped keeps N / W and gets child
+ * -1.  reused_dev uint8[num_trees] receives 1 for a re-rooted tree, 0 otherwise (the tree is left for qg_mcts_begin_keep to start
+ * afresh).  Uses path_node as scratch (it is free between decisions).  `pool` and `rollouts` share env kind, qubits, gateset and device. */
+QG_API int qg_mcts_reroot(const qg_mcts_tree* t, qg_engine* pool, const qg_engine* rollouts, const int32_t* chosen_dev, int32_t keep_nodes,
+                          uint8_t* reused_dev, qg_stream stream);
+/* qg_mcts_begin for the trees with reused_dev[i] == 0; re-rooted trees (reused_dev[i] != 0) are left untouched, root prior included. */
+QG_API int qg_mcts_begin_keep(const qg_mcts_tree* t, const float* root_prior_dev, const uint8_t* root_final_dev, const uint8_t* reused_dev,
+                              qg_stream stream);
 
 #ifdef __cplusplus
 }

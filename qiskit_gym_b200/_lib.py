@@ -28,7 +28,8 @@ SYMBOLS = [
     "qg_obs_words", "qg_step_bits", "qg_replay_bits", "qg_observe_bits", "qg_search_step_bits",
     "qg_policy_create", "qg_policy_create_value", "qg_policy_destroy", "qg_policy_num_actions", "qg_policy_has_value", "qg_policy_forward_bits",
     "qg_policy_forward_bits_value",
-    "qg_step_slots", "qg_copy_records", "qg_mcts_begin", "qg_mcts_select", "qg_mcts_backup", "qg_mcts_root_weights", "qg_search_run",
+    "qg_step_slots", "qg_copy_records", "qg_mcts_begin", "qg_mcts_select", "qg_mcts_backup", "qg_mcts_root_weights", "qg_mcts_reroot", "qg_mcts_begin_keep",
+    "qg_search_run",
     "qg_solutions", "qg_solutions_host", "qg_replay_host_packed", "qg_replay_host_packed_async", "qg_replay_packed", "qg_host_alloc", "qg_host_free", "qg_bind_thread_to_device",
     "qg_dlpack_obs", "qg_search_finish", "qg_nccl_unique_id", "qg_nccl_comm_create", "qg_nccl_comm_destroy",
     "qg_policy_tc_create", "qg_policy_tc_destroy", "qg_policy_tc_num_actions", "qg_policy_tc_forward_bits", "qg_policy_tc_set_mode",
@@ -133,6 +134,8 @@ def lib():
     L.qg_mcts_select.argtypes = [treep, C.c_float, vp, vp, vp, vp]
     L.qg_mcts_backup.argtypes = [treep, vp, vp, vp, vp, vp]
     L.qg_mcts_root_weights.argtypes = [treep, vp, vp]
+    L.qg_mcts_reroot.argtypes = [treep, vp, vp, vp, i32, vp, vp]
+    L.qg_mcts_begin_keep.argtypes = [treep, vp, vp, vp, vp]
     L.qg_search_run.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp]
     L.qg_solutions.argtypes = [vp, i64, i64, vp, i32, vp, vp]
     L.qg_solutions_host.argtypes = [vp, i64, i64, vp, i32, vp, vp]

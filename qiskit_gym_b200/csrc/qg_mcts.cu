@@ -12,6 +12,15 @@
 //                the new node gets the policy's priors for its observation; its value v is the value head's output, 0 if final;
 //                back up  G <- reward(child) + G  from the leaf (G = v) to the root, N(a) += 1, W(a) += G on every edge.
 //   decision:    action weights = N(a) / sum N at the root (arg-max or Philox sample by qg_search_step).
+//   tree reuse (opt-in, MCTSSearch(reuse_tree=True); node_cap = 2S + 1 for S simulations per decision): after the rollouts' step,
+//                tree i is re-rooted (qg_mcts_reroot) when the rollout played an action a >= 0 (chosen[i]), the root has a child
+//                c = child[0][a], and the pool record of c equals the rollout's record word for word (the solution-log length of
+//                HD_FLAGS masked as k_copy_records masks it).  With add_inverts the pool and the rollout draw their own coins, so c is one
+//                sample of a stochastic step: the record test keeps it only when the rollout reached the same env.  A re-rooted tree
+//                keeps the first K = node_cap - S nodes of c's subtree in creation order (a prefix in creation order holds every kept
+//                node's parent), renumbered in that order so that c becomes node 0; prior, N, W, remapped children, reward, final flag
+//                and pool record move with each node.  An edge whose child was dropped keeps N and W and gets child = -1.  The root keeps
+//                its stored prior (qg_mcts_begin_keep skips it); every other tree starts fresh.  The decision then adds S simulations.
 // Every f32 operation is rounded on its own (no FMA contraction) so the CPU restatement reproduces each argmax.
 //
 // Decomposition: one warp per tree; lanes stride over the actions of a node for the PUCT arg-max and for initialising a
@@ -19,7 +28,7 @@
 #include <algorithm>
 #include <string>
 
-#include "qg_host.hpp"
+#include "qg_engine_priv.hpp"
 
 namespace qg {
 
@@ -32,9 +41,7 @@ __device__ __forceinline__ void warp_argmax(float& s, int& a) {
     }
 }
 
-__global__ void k_mcts_begin(const qg_mcts_tree t, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final) {
-    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-    if (tree >= t.num_trees) return;
+__device__ __forceinline__ void begin_tree(const qg_mcts_tree& t, int tree, int lane, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final) {
     const size_t base = (size_t)tree * t.node_cap;
     for (int a = lane; a < t.num_actions; a += 32) {
         const size_t k = base * t.num_actions + a;
@@ -42,6 +49,75 @@ __global__ void k_mcts_begin(const qg_mcts_tree t, const float* __restrict__ roo
         t.visits[k] = 0; t.value_sum[k] = 0.0f; t.child[k] = -1;
     }
     if (lane == 0) { t.node_count[tree] = 1; t.node_reward[base] = 0.0f; t.node_final[base] = root_final[tree] ? 1 : 0; t.path_len[tree] = 0; t.new_node[tree] = -1; }
+}
+
+__global__ void k_mcts_begin(const qg_mcts_tree t, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final) {
+    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (tree >= t.num_trees) return;
+    begin_tree(t, tree, lane, root_prior, root_final);
+}
+
+__global__ void k_mcts_begin_keep(const qg_mcts_tree t, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final,
+                                  const uint8_t* __restrict__ reused) {
+    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (tree >= t.num_trees || reused[tree]) return;
+    begin_tree(t, tree, lane, root_prior, root_final);
+}
+
+// Re-rooting (protocol above).  path_node of tree i holds the old -> new node id map: >= 0 kept under that id, -2 a member of c's subtree
+// that is not kept (yet), -1 not a member.  Pass 1 walks nodes c .. node_count-1 in creation order; a member takes the next new id and marks
+// its children, so a node's mark is final before the walk reaches it (children are created after their parent).  Pass 2 moves the kept
+// nodes in ascending old-id order in place: new id <= old id and every lane moves the same entries of every row, so no row is written
+// before it has been read.
+__global__ void k_mcts_reroot(const qg_mcts_tree t, uint32_t* pool_rec, int64_t pool_bpad, const uint32_t* __restrict__ roll_rec, int64_t roll_bpad,
+                              int W, const int32_t* __restrict__ chosen, int keep, uint8_t* __restrict__ reused) {
+    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (tree >= t.num_trees) return;
+    const size_t base = (size_t)tree * t.node_cap;
+    const int A = t.num_actions, a = chosen[tree];
+    const int c = (a >= 0 && a < A) ? t.child[base * A + a] : -1;
+    bool diff = c < 0;
+    if (c >= 0) {
+        const uint32_t len_mask = (1u << FL_LEN_SHIFT) - 1u;
+        for (int w = lane; w < W; w += 32) {
+            const uint32_t m = w == HD_FLAGS ? len_mask : 0xFFFFFFFFu;
+            diff |= ((pool_rec[(size_t)w * pool_bpad + base + c] ^ roll_rec[(size_t)w * roll_bpad + tree]) & m) != 0u;
+        }
+    }
+    diff = __any_sync(0xFFFFFFFFu, diff);
+    if (lane == 0) reused[tree] = diff ? 0 : 1;
+    if (diff) return;
+    volatile int32_t* map = t.path_node + base;
+    const int count = t.node_count[tree];
+    for (int j = c + lane; j < count; j += 32) map[j] = -1;
+    __syncwarp();
+    int kept = 0;
+    for (int j = c; j < count && kept < keep; ++j) {
+        if (j != c && map[j] == -1) continue;
+        if (lane == 0) map[j] = kept;
+        ++kept;
+        for (int b = lane; b < A; b += 32) {
+            const int ch = t.child[(base + j) * A + b];
+            if (ch >= 0) map[ch] = -2;
+        }
+        __syncwarp();
+    }
+    for (int j = c, moved = 0; moved < kept; ++j) {
+        const int nj = map[j];
+        if (nj < 0) continue;
+        ++moved;
+        const size_t src = (base + j) * A, dst = (base + nj) * A;
+        for (int b = lane; b < A; b += 32) {
+            const int ch = t.child[src + b];
+            const int nc = ch >= 0 ? map[ch] : -1;
+            const float p = t.prior[src + b], s = t.value_sum[src + b];
+            const int n = t.visits[src + b];
+            t.prior[dst + b] = p; t.visits[dst + b] = n; t.value_sum[dst + b] = s; t.child[dst + b] = nc >= 0 ? nc : -1;
+        }
+        for (int w = lane; w < W; w += 32) pool_rec[(size_t)w * pool_bpad + base + nj] = pool_rec[(size_t)w * pool_bpad + base + j];
+        if (lane == 0) { t.node_reward[base + nj] = t.node_reward[base + j]; t.node_final[base + nj] = t.node_final[base + j]; }
+    }
+    if (lane == 0) t.node_count[tree] = kept;
 }
 
 __global__ void k_mcts_select(const qg_mcts_tree t, float c_puct, int32_t* __restrict__ src_slot, int32_t* __restrict__ dst_slot, int32_t* __restrict__ action) {
@@ -191,6 +267,37 @@ int qg_mcts_root_weights(const qg_mcts_tree* t, float* weights_dev, qg_stream st
     if (!weights_dev) { set_error("null argument"); return QG_ERR_INVALID; }
     if (t->num_trees == 0) return QG_OK;
     k_mcts_root_weights<<<tree_grid(t), 128, 0, (cudaStream_t)stream>>>(*t, weights_dev);
+    MCTS_LAUNCHED();
+    return QG_OK;
+}
+
+int qg_mcts_reroot(const qg_mcts_tree* t, qg_engine* pool, const qg_engine* rollouts, const int32_t* chosen_dev, int32_t keep_nodes,
+                   uint8_t* reused_dev, qg_stream stream) {
+    const int rc = check_tree(t);
+    if (rc != QG_OK) return rc;
+    if (!pool || !rollouts || !chosen_dev || !reused_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (pool->L.kind != rollouts->L.kind || pool->L.n != rollouts->L.n || pool->L.W != rollouts->L.W || pool->L.A != rollouts->L.A ||
+        pool->device != rollouts->device || t->num_actions != pool->L.A) {
+        set_error("qg_mcts_reroot: the engines must share env kind, qubits, gateset size and device with the trees"); return QG_ERR_INVALID;
+    }
+    if (rollouts->B < t->num_trees || pool->B < (int64_t)t->num_trees * t->node_cap) {
+        set_error("qg_mcts_reroot: the rollout engine needs one env per tree and the pool node_cap slots per tree"); return QG_ERR_INVALID;
+    }
+    if (keep_nodes < 1 || keep_nodes > t->node_cap) { set_error("qg_mcts_reroot: keep_nodes must be in 1..node_cap"); return QG_ERR_INVALID; }
+    if (t->num_trees == 0) return QG_OK;
+    CUDA_OK(cudaSetDevice(pool->device));
+    k_mcts_reroot<<<tree_grid(t), 128, 0, (cudaStream_t)stream>>>(*t, pool->dc.rec, pool->Bpad, rollouts->dc.rec, rollouts->Bpad, pool->L.W, chosen_dev,
+                                                                  keep_nodes, reused_dev);
+    MCTS_LAUNCHED();
+    return QG_OK;
+}
+
+int qg_mcts_begin_keep(const qg_mcts_tree* t, const float* root_prior_dev, const uint8_t* root_final_dev, const uint8_t* reused_dev, qg_stream stream) {
+    const int rc = check_tree(t);
+    if (rc != QG_OK) return rc;
+    if (!root_prior_dev || !root_final_dev || !reused_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (t->num_trees == 0) return QG_OK;
+    k_mcts_begin_keep<<<tree_grid(t), 128, 0, (cudaStream_t)stream>>>(*t, root_prior_dev, root_final_dev, reused_dev);
     MCTS_LAUNCHED();
     return QG_OK;
 }

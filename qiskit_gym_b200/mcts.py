@@ -8,6 +8,9 @@ instead of the raw policy output.  The tree bookkeeping (PUCT descent, node crea
 a child node's env is the parent's record cloned and stepped in one pass through a pool of record slots
 (`qg_step_slots`); the policy evaluates all new leaves of a simulation round in one batch.
 
+With `reuse_tree=True` a decision starts from the subtree below the action the rollout played (AlphaGo Zero's tree reuse), kept
+when the tree's node for it holds the env the rollout reached (csrc/qg_mcts.cu states the rule).
+
 twisterl's own tree search is not in the reference tree: the protocol (stated in csrc/qg_mcts.cu) is this engine's, and
 `max_expand_depth` — whose exact meaning cannot be recovered from the reference — is accepted and must be 1.
 """
@@ -54,23 +57,36 @@ class TreeArrays:
         check(lib().qg_mcts_root_weights(C.byref(self.c), _dptr(out), self._st()))
         return out
 
+    def reroot(self, pool, rollouts, chosen, keep_nodes, reused):
+        check(lib().qg_mcts_reroot(C.byref(self.c), pool._h, rollouts._h, _dptr(chosen), int(keep_nodes), _dptr(reused), self._st()))
+
+    def begin_keep(self, root_prior, root_final, reused):
+        check(lib().qg_mcts_begin_keep(C.byref(self.c), _dptr(root_prior), _dptr(root_final), _dptr(reused), self._st()))
+
 
 class MCTSSearch:
     """`solve` with a tree search per decision.  Owns the rollout engine (R envs, solutions tracked) and a slot-pool engine of
-    R * (num_mcts_searches + 1) records for the tree nodes."""
+    R * node_cap records for the tree nodes (node_cap = num_mcts_searches + 1, or 2 * num_mcts_searches + 1 with reuse_tree)."""
 
     def __init__(self, env_kind, num_qubits, gateset, policy: torch.nn.Module, num_rollouts: int, num_mcts_searches: int, C: float = 2 ** 0.5,
-                 device=None, max_depth: int = 128, use_cuda_graph: bool = True, policy_backend: str = "auto", **env_kwargs):
+                 device=None, max_depth: int = 128, use_cuda_graph: bool = True, policy_backend: str = "auto", reuse_tree: bool = False,
+                 **env_kwargs):
         """use_cuda_graph: a decision's launches (root evaluation, then per simulation PUCT descent -> clone + step -> policy -> back-up)
         are captured once and replayed: the whole decision as one graph up to 128 simulations, one graph per simulation beyond.
         policy_backend: "fused" = priors and values of the root / the leaves from packed observations in one kernel (policy.FusedPolicy
         with the value head; re-created whenever the module's weights change), "torch" = the PyTorch module on dense observations, "auto" =
-        fused when the policy has the simple head layout and the env can pack its observations."""
+        fused when the policy has the simple head layout and the env can pack its observations.
+        reuse_tree: each decision after the first of a `solve` keeps up to num_mcts_searches + 1 nodes of the subtree below the action
+        the rollout played, with their statistics, and adds num_mcts_searches simulations to them (qg_mcts_reroot).  The rollout's
+        action must then reach `decide` through `chosen` (solve does it; a caller driving decide itself passes chosen=self.chosen
+        to search_step).  `reused[i]` tells whether tree i was kept at the last decision."""
         assert num_mcts_searches >= 1 and policy_backend in ("auto", "fused", "torch")
         env_kwargs.setdefault("add_perms", False)
         self.env = BatchedEnv(env_kind, num_qubits, gateset, num_rollouts, device=device, max_depth=max_depth, **env_kwargs)
         pool_kwargs = dict(env_kwargs, track_solution=False)
-        self.S, self.NC, self.R = int(num_mcts_searches), int(num_mcts_searches) + 1, int(num_rollouts)
+        self.reuse = bool(reuse_tree)
+        self.S, self.R = int(num_mcts_searches), int(num_rollouts)
+        self.NC = (2 * self.S + 1) if self.reuse else (self.S + 1)
         self.pool = BatchedEnv(env_kind, num_qubits, gateset, self.R * self.NC, device=self.env.device_index, max_depth=max_depth, **pool_kwargs)
         self.policy = policy.to(self.env.device).eval()
         self.c_puct, self.max_depth = float(C), int(max_depth)
@@ -84,6 +100,9 @@ class MCTSSearch:
         self.leaf_reward = torch.zeros(self.R, dtype=torch.float32, device=dev)
         self.leaf_done = torch.zeros(self.R, dtype=torch.bool, device=dev)
         self.weights = torch.zeros((self.R, A), dtype=torch.float32, device=dev)
+        self.chosen = torch.full((self.R,), -1, dtype=i32, device=dev)        # the rollouts' last actions (-1: none, fresh trees)
+        self.reused = torch.zeros(self.R, dtype=torch.uint8, device=dev)       # 1: tree i was re-rooted at the last decision
+        self._fresh = True          # chosen is all -1: the next decision starts every tree afresh
         self.num_active = torch.zeros(1, dtype=torch.int32, device=dev)
         self.hook = None            # tests: hook(kind, decision, simulation, tensors...) sees the policy outputs the trees consumed
         from .policy import simple_value_head
@@ -118,6 +137,8 @@ class MCTSSearch:
 
     def _root(self, decision: int = 0):
         env, pool, tree = self.env, self.pool, self.tree
+        if self.reuse:
+            tree.reroot(pool, env, self.chosen, self.NC - self.S, self.reused)
         _, done, _, _ = env.status()
         if self.backend == "fused":
             env.observe_bits(self.root_bits)
@@ -128,8 +149,11 @@ class MCTSSearch:
             prior, _ = self._policy(env.obs)
         if self.hook:
             self.hook("root", decision, -1, prior, None)
-        pool.copy_records_from(env, self.root_slots)
-        tree.begin(prior, done)
+        pool.copy_records_from(env, self.root_slots)          # (a re-rooted tree's root record already equals it)
+        if self.reuse:
+            tree.begin_keep(prior, done, self.reused)
+        else:
+            tree.begin(prior, done)
 
     def _simulation(self, decision: int = 0, s: int = 0):
         pool, tree = self.pool, self.tree
@@ -153,7 +177,8 @@ class MCTSSearch:
 
     def _capture(self):
         """Graphs of one decision.  The search reads the rollout engine and writes only the slot pool, the trees and self.weights, so
-        the warm-up runs (cuBLAS workspaces, lazy initialisation) leave the rollouts untouched."""
+        the warm-up runs (cuBLAS workspaces, lazy initialisation) leave the rollouts untouched.  With reuse_tree they would overwrite
+        trees that the next decision keeps: decide() captures only while every tree starts afresh (chosen all -1)."""
         dev = self.env.device
         for _ in range(2):
             self._root()
@@ -178,9 +203,12 @@ class MCTSSearch:
         """One decision's tree search for every rollout; leaves the root visit weights in self.weights."""
         if self.backend == "fused":
             self._fused_policy()
+        fresh, self._fresh = self._fresh, False
         if not self.use_graph or self.hook is not None:
             return self._decide_eager(decision)
         if self._graphs is None or self._graph_policy is not self.policy:      # (a graph holds the policy's parameter tensors)
+            if self.reuse and not fresh:
+                return self._decide_eager(decision)
             self._capture()
         root, sim, whole = self._graphs
         if whole is not None:
@@ -196,10 +224,12 @@ class MCTSSearch:
         t0 = time.perf_counter()
         env.set_state(state)
         env.search_begin(seed, first_rollout_id)
+        self.chosen.fill_(-1)
+        self._fresh = True
         its = 0
         while its < self.max_depth:
             self.decide(its)
-            env.search_step(self.weights, deterministic=deterministic, obs=False, num_active=self.num_active)
+            env.search_step(self.weights, deterministic=deterministic, obs=False, chosen=self.chosen, num_active=self.num_active)
             its += 1
             if its % check_every == 0 and int(self.num_active.item()) == 0:
                 break

@@ -117,26 +117,30 @@ class RLSynthesis:
             self._searches[key] = rs
         return rs
 
-    def _mcts(self, num_searches: int, num_mcts_searches: int, C: float):
+    def _mcts(self, num_searches: int, num_mcts_searches: int, C: float, reuse_tree: bool = False):
         from .mcts import MCTSSearch
-        key = ("mcts", num_searches, num_mcts_searches, C)
+        key = ("mcts", num_searches, num_mcts_searches, C, reuse_tree)
         ms = self._searches.get(key)
         if ms is None:
             cfg = dict(self.env_config)
             kind = _ENV_KINDS[self.env.cls_name]
             kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset", "max_depth", "add_perms")}
             ms = MCTSSearch(kind, cfg["num_qubits"], cfg["gateset"], self.policy, num_searches, num_mcts_searches, C=C, device=self.device,
-                            max_depth=cfg.get("max_depth", 128), add_perms=False, **kw)
+                            max_depth=cfg.get("max_depth", 128), add_perms=False, reuse_tree=reuse_tree, **kw)
             self._searches[key] = ms
         return ms
 
     def solve(self, state, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
-              max_expand_depth: int = 1, seed: int = 0):
-        """twisterl `Algorithm.solve`: the action list of the best successful rollout, or None."""
+              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False):
+        """twisterl `Algorithm.solve`: the action list of the best successful rollout, or None.
+        reuse_tree (tree search only): every decision but the first starts from the subtree below the action played (mcts.MCTSSearch)."""
+        if reuse_tree and not num_mcts_searches:
+            raise ValueError("reuse_tree needs a tree search (num_mcts_searches > 0)")
         if num_mcts_searches:
             if max_expand_depth != 1:
                 raise NotImplementedError("max_expand_depth != 1 is not supported by the device tree search (mcts.py)")
-            return self._mcts(int(num_searches), int(num_mcts_searches), float(C)).solve(state, deterministic=deterministic, seed=seed).actions
+            return self._mcts(int(num_searches), int(num_mcts_searches), float(C), bool(reuse_tree)).solve(state, deterministic=deterministic,
+                                                                                                             seed=seed).actions
         return self._search(int(num_searches)).solve(state, deterministic=deterministic, seed=seed).actions
 
     def solve_many(self, states, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
@@ -182,10 +186,10 @@ class RLSynthesis:
         return out
 
     def synth(self, input, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
-              max_expand_depth: int = 1, seed: int = 0):
+              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False):
         """rl/synthesis.py:112-126.  Returns the synthesised circuit (QuantumCircuit with Qiskit, else a gate list) or None."""
         state = self.env.get_state(input)
-        actions = self.solve(state, deterministic, num_searches, num_mcts_searches, C, max_expand_depth, seed=seed)
+        actions = self.solve(state, deterministic, num_searches, num_mcts_searches, C, max_expand_depth, seed=seed, reuse_tree=reuse_tree)
         if actions is not None:
             return self.env.build_circuit_from_solution(actions, input)
 
