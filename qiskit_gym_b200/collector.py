@@ -182,19 +182,19 @@ class RolloutCollector:
             return torch.softmax(logits.float(), dim=-1), value.float().reshape(-1)
 
     def tensor_core_policy(self):
-        """The collect_packed policy handle (policy.TensorCorePolicy) for the current weights.  A weight update (optimizer step, load_state_dict)
-        is copied into the existing handle in place (TensorCorePolicy.load_weights: captured rollout graphs stay valid); the handle is rebuilt —
-        and the graphs dropped — only for a new shape, parameters that are not f32 / contiguous on the device, or a larger batch.
+        """The collect_packed policy handle (policy.TensorCorePolicy) refreshed from self.policy (TensorCorePolicy.refresh): a weight update
+        (optimizer step, load_state_dict) is copied into the handle in place, so captured rollout graphs stay valid; they are dropped when the
+        handle is recreated (another module that cannot be loaded in place) or rebuilt for a larger batch.
         Raises NotImplementedError where the tensor-core policy cannot run (more than 127 actions, a value head that is not one Linear,
         a device that is not sm_100)."""
-        from .policy import TensorCorePolicy, weights_version
+        from .policy import TensorCorePolicy
         B = self.env.batch
         tcp = getattr(self, "_tcp", None)
-        if tcp is None or tcp.max_batch < B or not tcp.can_load(self.policy):
+        if tcp is None or tcp.max_batch < B:
             tcp = self._tcp = TensorCorePolicy(self.policy, max_batch=B, device=self.env.device, with_value=True)
             self._packed = {}
-        elif tcp.version != weights_version(self.policy):
-            tcp.load_weights(self.policy)
+        elif tcp.refresh(self.policy):
+            self._packed = {}
         return tcp
 
     def collect_packed(self, num_steps: int, deterministic: bool = False, use_cuda_graph: bool = True) -> Rollout:

@@ -24,7 +24,7 @@ import torch
 from . import _abi
 from ._lib import check, lib
 from .engine import BatchedEnv, _dptr
-from .search import SearchResult, decode_key, reduce_best
+from .search import SearchResult, best_rollout, search_result
 
 
 class TreeArrays:
@@ -74,7 +74,7 @@ class MCTSSearch:
         """use_cuda_graph: a decision's launches (root evaluation, then per simulation PUCT descent -> clone + step -> policy -> back-up)
         are captured once and replayed: the whole decision as one graph up to 128 simulations, one graph per simulation beyond.
         policy_backend: "fused" = priors and values of the root / the leaves from packed observations in one kernel (policy.FusedPolicy
-        with the value head; re-created whenever the module's weights change), "torch" = the PyTorch module on dense observations, "auto" =
+        with the value head, refreshed from `policy` before every decision), "torch" = the PyTorch module on dense observations, "auto" =
         fused when the policy has the simple head layout and the env can pack its observations.
         reuse_tree: each decision after the first of a `solve` keeps up to num_mcts_searches + 1 nodes of the subtree below the action
         the rollout played, with their statistics, and adds num_mcts_searches simulations to them (qg_mcts_reroot).  The rollout's
@@ -105,7 +105,7 @@ class MCTSSearch:
         self._fresh = True          # chosen is all -1: the next decision starts every tree afresh
         self.num_active = torch.zeros(1, dtype=torch.int32, device=dev)
         self.hook = None            # tests: hook(kind, decision, simulation, tensors...) sees the policy outputs the trees consumed
-        from .policy import simple_value_head
+        from .policy import FusedPolicy, simple_value_head
         can_fuse = simple_value_head(self.policy) is not None and not (env_kind == 0 and num_qubits > 64)      # (no packed observations for n > 64 permutations)
         if policy_backend == "fused" and not can_fuse:
             raise NotImplementedError("policy_backend='fused' needs single-Linear action / value heads")
@@ -116,24 +116,15 @@ class MCTSSearch:
             self.leaf_bits = torch.zeros((self.R, self.env.obs_words()), dtype=torch.int32, device=dev)
             self.pri = torch.zeros((self.R, A), dtype=torch.float32, device=dev)
             self.val = torch.zeros(self.R, dtype=torch.float32, device=dev)
+            self.fused = FusedPolicy(self.policy, device=dev, with_value=True)
         self.use_graph = bool(use_cuda_graph)
-        self._graphs = None         # (root graph or None, simulation graph or None, whole-decision graph or None)
-        self._graph_policy = None
-        self._fused_for = None
+        self._graphs = None         # (module captured, root graph or None, simulation graph or None, whole-decision graph or None)
         self._stream = torch.cuda.Stream(device=dev)
 
     def _policy(self, obs):
         with torch.no_grad():
             logits, value = self.policy(obs)
             return torch.softmax(logits.float(), dim=-1).contiguous(), value.float().reshape(-1).contiguous()
-
-    def _fused_policy(self):
-        from .policy import FusedPolicy, weights_version
-        if self.fused is None or self.fused.version != weights_version(self.policy) or self._fused_for is not self.policy:
-            self.fused = FusedPolicy(self.policy, device=self.env.device, with_value=True)
-            self._fused_for = self.policy
-            self._graphs = None                    # a graph holds the old handle
-        return self.fused
 
     def _root(self, decision: int = 0):
         env, pool, tree = self.env, self.pool, self.tree
@@ -189,28 +180,28 @@ class MCTSSearch:
             whole = torch.cuda.CUDAGraph()
             with torch.cuda.graph(whole, stream=self._stream):
                 self._decide_eager()
-            self._graphs = (None, None, whole)
+            self._graphs = (self.policy, None, None, whole)
         else:
             root, sim = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
             with torch.cuda.graph(root, stream=self._stream):
                 self._root()
             with torch.cuda.graph(sim, stream=self._stream):
                 self._simulation()
-            self._graphs = (root, sim, None)
-        self._graph_policy = self.policy
+            self._graphs = (self.policy, root, sim, None)
 
     def decide(self, decision: int = 0):
         """One decision's tree search for every rollout; leaves the root visit weights in self.weights."""
-        if self.backend == "fused":
-            self._fused_policy()
+        # a graph holds the policy handle and the module's parameter tensors
+        if (self.fused is not None and self.fused.refresh(self.policy)) or (self._graphs is not None and self._graphs[0] is not self.policy):
+            self._graphs = None
         fresh, self._fresh = self._fresh, False
         if not self.use_graph or self.hook is not None:
             return self._decide_eager(decision)
-        if self._graphs is None or self._graph_policy is not self.policy:      # (a graph holds the policy's parameter tensors)
+        if self._graphs is None:
             if self.reuse and not fresh:
                 return self._decide_eager(decision)
             self._capture()
-        root, sim, whole = self._graphs
+        _, root, sim, whole = self._graphs
         if whole is not None:
             whole.replay()
             return self.weights
@@ -233,14 +224,5 @@ class MCTSSearch:
             its += 1
             if its % check_every == 0 and int(self.num_active.item()) == 0:
                 break
-        key, idx = env.search_best()
-        ok, rid = decode_key(key)
-        sol = env.solution(idx) if (ok and idx >= 0) else None
-        world = 1
-        import torch.distributed as dist
-        if dist.is_available() and dist.is_initialized():
-            world = dist.get_world_size(group)
-            key, sol = reduce_best(key, sol, group=group, device=env.device if dist.get_backend(group) == "nccl" else None)
-            ok, rid = decode_key(key)
-        return SearchResult(actions=sol if ok else None, key=key, rollout_id=rid, success=ok, iterations=its,
-                            seconds=time.perf_counter() - t0, rollouts=self.R * world)
+        key, sol = best_rollout(env)
+        return search_result(env, key, sol, its, t0, self.R, group)

@@ -225,8 +225,7 @@ class Trainer:
             ms = self._eval_mcts.get(key)
             if ms is None:
                 kind, n, gs, kw = self.spec
-                kw = {k: v for k, v in kw.items() if k != "max_depth"}
-                ms = MCTSSearch(kind, n, gs, self.policy, E, sims, C=float(ev["C"]), device=self.device.index, max_depth=int(self.env.cfg.max_depth), **kw)
+                ms = MCTSSearch(kind, n, gs, self.policy, E, sims, C=float(ev["C"]), device=self.device.index, **kw)
                 self._eval_mcts[key] = ms
             ms.policy = self.policy
             env = ms.env
@@ -403,9 +402,7 @@ class AlphaZero(Trainer):
         if int(c["max_expand_depth"]) != 1:
             raise NotImplementedError("max_expand_depth != 1 is not supported by the device tree search (mcts.py)")
         kind, n, gs, kw = self.spec
-        kw = {k: v for k, v in kw.items() if k != "max_depth"}
-        self.search = self._mcts_cls(kind, n, gs, self._policy_for_env, batch, int(c["num_mcts_searches"]), C=float(c["C"]), device=device,
-                                     max_depth=int(self.spec[3].get("max_depth", 128)), **kw)
+        self.search = self._mcts_cls(kind, n, gs, self._policy_for_env, batch, int(c["num_mcts_searches"]), C=float(c["C"]), device=device, **kw)
         return self.search.env
 
     def iterate(self) -> dict:
@@ -414,7 +411,6 @@ class AlphaZero(Trainer):
         ms.policy = self.policy.eval()
         dev, A = self.device, env.num_actions()
         obs_buf = torch.empty((T, B) + tuple(env.obs_shape()), dtype=torch.float32, device=dev)
-        self._bit_shifts = torch.arange(32, dtype=torch.int32, device=dev)
         pi = torch.zeros((T, B, A), dtype=torch.float32, device=dev)
         actions = torch.full((T, B), -1, dtype=torch.int32, device=dev)
         rewards = torch.zeros((T, B), dtype=torch.float32, device=dev)
@@ -427,9 +423,7 @@ class AlphaZero(Trainer):
             if ms.backend == "fused":
                 # the fused backend observes into packed bits only (ms.root_bits): the training sample is what the root evaluation saw
                 # (for PauliNetwork with add_perms that includes the qubit permutation observe() picked)
-                bits = ms.root_bits.reshape(B, -1)
-                dense = ((bits.unsqueeze(-1) >> self._bit_shifts) & 1).reshape(B, -1)[:, :obs_buf[t].numel() // B]
-                obs_buf[t].copy_(dense.reshape(obs_buf[t].shape))
+                obs_buf[t].copy_(unpack_bits(ms.root_bits, env._obs_size).reshape(obs_buf[t].shape))
             else:
                 obs_buf[t].copy_(env.obs)
             pi[t].copy_(w)

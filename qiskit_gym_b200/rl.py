@@ -81,28 +81,29 @@ class RLSynthesis:
                 torch.save(self.policy.state_dict(), f)
 
     # ---- synthesis ------------------------------------------------------------------------------------
+    def _env_args(self, **override):
+        """(env kind, num_qubits, gateset, the env config's other entries updated with `override`): what a device engine is built from."""
+        cfg = self.env_config
+        kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset")}
+        return _ENV_KINDS[self.env.cls_name], cfg["num_qubits"], cfg["gateset"], {**kw, **override}
+
     def _search(self, num_searches: int, targets_per_launch: int | None = None, matmul_precision: str = "f32") -> RolloutSearch:
         """The cached search of `num_searches` rollouts per target: the single-target one, or with targets_per_launch the one solve_many
         uses (rebuilt only when a call needs more targets per launch than it holds).  matmul_precision="tensor_core": the "tensor_core"
-        backend, cached under its own key (it never replaces the f32 search) and with no fall-back; it refreshes its weights itself."""
-        from .policy import weights_version
+        backend, cached under its own key (it never replaces the f32 search) and with no fall-back.  A search refreshes its policy handle
+        from self.policy itself, so a weight update does not rebuild it."""
         key = num_searches if targets_per_launch is None else ("many", num_searches)
         if matmul_precision == "tensor_core":
             key = ("tensor_core", key)
         rs = self._searches.get(key)
-        if rs is not None and getattr(rs, "fused", None) is not None and rs.fused.version != weights_version(self.policy):
-            rs = None                                    # the cached search captured older weights (load_state_dict after the first synth)
         if rs is not None and targets_per_launch is not None and rs.targets_per_launch < targets_per_launch:
             rs = None
         if rs is None:
             self._searches.pop(key, None)                # (frees the old engine before the new one allocates)
-            cfg = dict(self.env_config)
-            kind = _ENV_KINDS[self.env.cls_name]
-            kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset", "max_depth", "add_perms")}
+            kind, n, gs, kw = self._env_args(add_perms=False)
 
             def make(backend):
-                return RolloutSearch(kind, cfg["num_qubits"], cfg["gateset"], self.policy, num_searches, device=self.device,
-                                     max_depth=cfg.get("max_depth", 128), add_perms=False, policy_backend=backend,
+                return RolloutSearch(kind, n, gs, self.policy, num_searches, device=self.device, policy_backend=backend,
                                      targets_per_launch=targets_per_launch or 1, **kw)
             if matmul_precision == "tensor_core":
                 rs = make("tensor_core")
@@ -122,11 +123,8 @@ class RLSynthesis:
         key = ("mcts", num_searches, num_mcts_searches, C, reuse_tree)
         ms = self._searches.get(key)
         if ms is None:
-            cfg = dict(self.env_config)
-            kind = _ENV_KINDS[self.env.cls_name]
-            kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset", "max_depth", "add_perms")}
-            ms = MCTSSearch(kind, cfg["num_qubits"], cfg["gateset"], self.policy, num_searches, num_mcts_searches, C=C, device=self.device,
-                            max_depth=cfg.get("max_depth", 128), add_perms=False, reuse_tree=reuse_tree, **kw)
+            kind, n, gs, kw = self._env_args(add_perms=False)
+            ms = MCTSSearch(kind, n, gs, self.policy, num_searches, num_mcts_searches, C=C, device=self.device, reuse_tree=reuse_tree, **kw)
             self._searches[key] = ms
         return ms
 
@@ -209,13 +207,11 @@ class RLSynthesis:
             raise NotImplementedError("matmul_precision applies to PPO only (AlphaZero evaluates its policy inside the tree search)")
         if algo == "AZ" and update_precision != "f32":
             raise NotImplementedError("update_precision applies to PPO only (the AlphaZero update runs in f32 PyTorch)")
-        cfg = dict(self.env_config)
-        kind = _ENV_KINDS[self.env.cls_name]
-        kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset")}
+        kind, n, gs, kw = self._env_args()
         if algo == "PPO":
             kw["matmul_precision"] = matmul_precision
             kw["update_precision"] = update_precision
-        trainer = (ppo.PPO if algo == "PPO" else ppo.AlphaZero)(kind, cfg["num_qubits"], cfg["gateset"], self.policy, self.rl_config, device=self.device, seed=seed, **kw)
+        trainer = (ppo.PPO if algo == "PPO" else ppo.AlphaZero)(kind, n, gs, self.policy, self.rl_config, device=self.device, seed=seed, **kw)
         if hasattr(self.env, "difficulty"):
             self.env.difficulty = initial_difficulty                # rl/synthesis.py:129 (a reference *Gym object; a SynthSpec owns no env)
         try:

@@ -133,6 +133,31 @@ def reduce_best(local_key: int, local_solution, group=None, device=None):
     return best, [int(v) for v in buf[:n].tolist()]
 
 
+def best_rollout(env: BatchedEnv):
+    """(key, solution or None) of the best rollout of this rank's engine (qg_search_best)."""
+    key, idx = env.search_best()
+    ok, rid = decode_key(key)
+    return key, (env.solution(idx) if (ok and idx >= 0) else None)
+
+
+def search_result(env: BatchedEnv, key, sol, its, t0, local_rollouts, group=None, reduced=False) -> SearchResult:
+    """The SearchResult of a search whose best local rollout is (key, sol): under torch.distributed, reduced over the ranks first
+    (reduce_best) unless `reduced` says the key already is the global one; rollouts = local_rollouts x the world size."""
+    ok, rid = decode_key(key)
+    world = 1
+    try:
+        import torch.distributed as dist
+        if dist.is_available() and dist.is_initialized():
+            world = dist.get_world_size(group)
+            if not reduced:
+                key, sol = reduce_best(key, sol, group=group, device=env.device if dist.get_backend(group) == "nccl" else None)
+            ok, rid = decode_key(key)
+    except ImportError:
+        pass
+    return SearchResult(actions=sol if ok else None, key=key, rollout_id=rid, success=ok, iterations=its,
+                        seconds=time.perf_counter() - t0, rollouts=local_rollouts * world)
+
+
 class RolloutSearch:
     """Device-resident `solve`: owns a BatchedEnv of `num_rollouts` rollouts on one GPU."""
 
@@ -149,8 +174,10 @@ class RolloutSearch:
         rounds differently from the f32 backends, so its decisions are not theirs (the probabilities are within TensorCorePolicy's error
         bound of the float64 module).  Each row's probabilities are bit-identical whatever the batch size and the other rows, so the
         solve_many contract below holds among "tensor_core" searches.  NotImplementedError where it cannot run: more than 127 actions,
-        a Permutation wider than 64 qubits (no packed observations), a device that is not sm_100.  A weight update of `policy` (optimizer
-        step, load_state_dict) is copied into the handle in place before the next search (captured graphs stay valid).
+        a Permutation wider than 64 qubits (no packed observations), a device that is not sm_100.
+        Every search starts by refreshing the policy handle from `self.policy` (policy.FusedPolicy / TensorCorePolicy.refresh): a weight
+        update (optimizer step, load_state_dict) or another module assigned to `policy` is what the next search runs.  "tensor_core" copies
+        a weight update into the handle in place (captured graphs stay valid).
         targets_per_launch: solve_many searches that many targets together, each with its own `num_rollouts` rollouts (the engine
         holds targets_per_launch * num_rollouts); solve() needs targets_per_launch == 1."""
         env_kwargs.setdefault("add_perms", False)
@@ -165,13 +192,14 @@ class RolloutSearch:
         self.max_depth = max_depth
         self.B = targets_per_launch * num_rollouts
         dev = self.env.device
+        self.handle = None          # the policy's C handle (policy.FusedPolicy / TensorCorePolicy); None for "torch"
         if policy_backend in ("fused", "persistent"):
             from .policy import FusedPolicy
-            self.fused = FusedPolicy(self.policy, device=dev)
+            self.handle = FusedPolicy(self.policy, device=dev)
         if policy_backend == "tensor_core":
             from .policy import TensorCorePolicy
             check_tensor_core_search(env_kind, num_qubits, self.env.num_actions(), dev)
-            self.tcp = TensorCorePolicy(self.policy, max_batch=self.B, device=dev, with_value=False)
+            self.handle = TensorCorePolicy(self.policy, max_batch=self.B, device=dev, with_value=False)
         if policy_backend != "torch":
             self.obs_bits = self.env.new_obs_bits()
         self.probs = torch.zeros((self.B, self.env.num_actions()), dtype=torch.float32, device=dev)
@@ -182,15 +210,19 @@ class RolloutSearch:
         self._stream = torch.cuda.Stream(device=dev)
         self._decisions = torch.zeros((self.B + 7) // 8, dtype=torch.int32, device=dev)
 
+    # the handle under the names it had per backend before `handle` (read by existing callers): None for the other backends
+    fused = property(lambda self: self.handle if self.backend in ("fused", "persistent") else None)
+    tcp = property(lambda self: self.handle if self.backend == "tensor_core" else None)
+
     def check_supported(self):
         """Raises NotImplementedError (QG_ERR_UNSUPPORTED) now rather than in the first solve() when the one-launch search cannot run
         this env / policy pair: a zero-decision qg_search_run goes through all of its checks without launching anything."""
         if self.backend == "persistent":
-            self.env.search_run(self.fused, self.obs_bits, self.probs, 0, deterministic=True, decisions=self._decisions)
+            self.env.search_run(self.handle, self.obs_bits, self.probs, 0, deterministic=True, decisions=self._decisions)
 
     def _iteration(self, deterministic):
         if self.backend in ("fused", "tensor_core"):
-            (self.fused if self.backend == "fused" else self.tcp).forward_bits(self.obs_bits, probs=self.probs)
+            self.handle.forward_bits(self.obs_bits, probs=self.probs)
             if self.hook is not None:
                 self.hook(self.probs, self.obs_bits)
             self.env.search_step_bits(self.probs, self.obs_bits, deterministic=deterministic, num_active=self.num_active)
@@ -206,19 +238,11 @@ class RolloutSearch:
         else:
             self.env.observe()
 
-    def _refresh_weights(self):
-        """"tensor_core": copies a weight update of self.policy into the handle in place, after the caller's stream's pending work (captured
-        graphs stay valid); a module of another shape, or whose parameters cannot be read in place, gets a new handle and new graphs."""
-        if self.backend != "tensor_core":
-            return
-        from .policy import TensorCorePolicy, weights_version
-        if not self.tcp.can_load(self.policy):
+    def _refresh_weights(self, caller):
+        """Brings the handle up to self.policy; runs on self._stream, whose refresh work waits for the caller's stream.  A recreated
+        handle drops the graphs captured with the old one."""
+        if self.handle is not None and self.handle.refresh(self.policy, after=caller):
             self._graphs = {}
-            self.tcp = TensorCorePolicy(self.policy, max_batch=self.B, device=self.env.device, with_value=False)
-        elif self.tcp.version != weights_version(self.policy):
-            self._stream.wait_stream(torch.cuda.current_stream(self.env.device))
-            with torch.cuda.stream(self._stream):
-                self.tcp.load_weights(self.policy)
 
     def _graph(self, deterministic, params):
         """The CUDA graph of one iteration.  Its launches carry the engine's seed and first rollout id as they were at capture (the
@@ -238,17 +262,6 @@ class RolloutSearch:
             self._graphs[deterministic] = (g, params)
         return g
 
-    def _local_best(self, comm):
-        """(key, solution or None) of this rank's rollouts — or, with an ncclComm_t of the C ABI (engine.nccl_comm_create), of ALL ranks'
-        rollouts: qg_search_finish does the cross-GPU reduction itself (one all-gather + on-GPU pick), no torch collective."""
-        env = self.env
-        if comm is not None:
-            key, ok, rid, owner, sol = env.search_finish(comm)
-            return key, sol, True
-        key, idx = env.search_best()
-        ok, rid = decode_key(key)
-        return key, (env.solution(idx) if (ok and idx >= 0) else None), False
-
     def _search(self, load, deterministic, seed, first_rollout_id, check_every):
         """One search on self._stream (the caller enters it): load() puts the targets into the rollouts, then the decisions run.
         Returns the number of decision steps, or None for the one-launch search (its CTAs' counts are in self._decisions)."""
@@ -257,7 +270,7 @@ class RolloutSearch:
             load()
             env.search_begin(seed, first_rollout_id)
             self._observe()
-            env.search_run(self.fused, self.obs_bits, self.probs, self.max_depth, deterministic=deterministic, decisions=self._decisions)
+            env.search_run(self.handle, self.obs_bits, self.probs, self.max_depth, deterministic=deterministic, decisions=self._decisions)
             return None
         load()
         use_graph = self.use_graph and self.hook is None
@@ -286,14 +299,18 @@ class RolloutSearch:
             raise ValueError("solve() searches one target: use solve_many() on a search built with targets_per_launch > 1")
         env = self.env
         t0 = time.perf_counter()
-        self._refresh_weights()
+        caller = torch.cuda.current_stream(env.device)
         with torch.cuda.stream(self._stream):
+            self._refresh_weights(caller)
             # broadcast: every rollout starts from the target
             its = self._search(lambda: env.set_state(state), deterministic, seed, first_rollout_id, check_every)
-            key, sol, reduced = self._local_best(comm)
+            if comm is not None:        # qg_search_finish reduces over ALL ranks itself (one all-gather + on-GPU pick), no torch collective
+                key, ok, rid, owner, sol = env.search_finish(comm)
+            else:
+                key, sol = best_rollout(env)
             if its is None:
                 its = int(self._decisions.max().item())
-        return self._finish(key, sol, its, t0, group, reduced)
+        return search_result(env, key, sol, its, t0, self.B, group, reduced=comm is not None)
 
     def solve_many(self, states, deterministic: bool = False, seed: int = 0, check_every: int = 8) -> list[SearchResult]:
         """solve() for many targets, targets_per_launch of them per search.  Target t gets global rollout ids t*R .. t*R + R - 1
@@ -311,7 +328,9 @@ class RolloutSearch:
             self._win = torch.zeros(words, dtype=torch.int32, device=env.device)
             self._win_host = torch.zeros(words, dtype=torch.int32, pin_memory=True)
         pad = identity_payload(self.env_kind, self.num_qubits)
-        self._refresh_weights()
+        caller = torch.cuda.current_stream(env.device)
+        with torch.cuda.stream(self._stream):
+            self._refresh_weights(caller)
         out = []
         for start, count, first_id in plan:
             t0 = time.perf_counter()
@@ -336,19 +355,3 @@ class RolloutSearch:
                 out.append(SearchResult(actions=rows[j, : lens[j]].astype(np.int64).tolist() if ok else None, key=key, rollout_id=rid,
                                         success=ok, iterations=its, seconds=dt, rollouts=R))
         return out
-
-    def _finish(self, key, sol, its, t0, group, reduced=False):
-        env = self.env
-        ok, rid = decode_key(key)
-        world = 1
-        try:
-            import torch.distributed as dist
-            if dist.is_available() and dist.is_initialized():
-                world = dist.get_world_size(group)
-                if not reduced:
-                    key, sol = reduce_best(key, sol, group=group, device=env.device if dist.get_backend(group) == "nccl" else None)
-                ok, rid = decode_key(key)
-        except ImportError:
-            pass
-        return SearchResult(actions=sol if ok else None, key=key, rollout_id=rid, success=ok, iterations=its,
-                            seconds=time.perf_counter() - t0, rollouts=self.B * world)

@@ -146,7 +146,7 @@ def test_solve_many_bit_identical_to_single_target(name, R):
     seed = 5
     for T in (1, 5, 37):
         rs = RolloutSearch(kind, n, gs, _tc_policy(name), R, max_depth=MAX_DEPTH, policy_backend="tensor_core", targets_per_launch=T, **kw)
-        assert rs.tcp.max_batch == T * R and rs.tcp.set_per_layer(False) == FUSED[name]
+        assert rs.handle.max_batch == T * R and rs.handle.set_per_layer(False) == FUSED[name]
         for det in (False, True):
             got = rs.solve_many(states[:T], deterministic=det, seed=seed)
             assert len(got) == T
@@ -287,7 +287,7 @@ def test_collector_scale_validity():
     states = [states[i] for i in rng.permutation(T)]
     pol = _policy(kind, n, gs, kw, seed=1, embedding_size=512, common_layers=(256,))
     rs = RolloutSearch(kind, n, gs, pol, R, targets_per_launch=T, policy_backend="tensor_core", **kw)
-    assert rs.env.batch == 65536 and rs.tcp.set_per_layer(False)
+    assert rs.env.batch == 65536 and rs.handle.set_per_layer(False)
     res = rs.solve_many(states, seed=17)
     solved = [t for t in range(T) if res[t].success]
     assert len(solved) > 50

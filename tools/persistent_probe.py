@@ -24,7 +24,7 @@ for emb, common in ((512, (256,)), (32, ())):
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    env.search_run(rs.fused, rs.obs_bits, rs.probs, 128, decisions=rs._decisions)
+    env.search_run(rs.handle, rs.obs_bits, rs.probs, 128, decisions=rs._decisions)
     e1.record()
     torch.cuda.synchronize()
     k_ms = e0.elapsed_time(e1)

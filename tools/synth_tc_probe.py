@@ -60,9 +60,9 @@ def split(tc, ffma, state, seed, decisions):
         tc._observe()
         ev[1].record()
         for d in range(decisions):
-            tc.tcp.forward_bits(tc.obs_bits, probs=tc.probs)
+            tc.handle.forward_bits(tc.obs_bits, probs=tc.probs)
             ev[2 + 3 * d].record()
-            ffma.fused.forward_bits(tc.obs_bits, probs=ffma.probs)          # (same observations; its output is not used)
+            ffma.handle.forward_bits(tc.obs_bits, probs=ffma.probs)          # (same observations; its output is not used)
             ev[3 + 3 * d].record()
             env.search_step_bits(tc.probs, tc.obs_bits, num_active=tc.num_active)
             ev[4 + 3 * d].record()
