@@ -355,11 +355,24 @@ QG_API int qg_search_step_bits(qg_engine* e, const float* weights_dev, int32_t d
  * action head) evaluated from packed observations in one kernel: first layer = bias + sum of the weight columns of the
  * set bits, then the Linear/ReLU chain and a softmax.  Layer l has out_features[l] outputs and consumes the
  * observation (l = 0) or layer l-1; weights_host[l] is torch's Linear.weight layout [out][in] row-major, f32; ReLU
- * follows every layer but the last.  Limits: 1..8 layers, widths <= 1024.
- * Arithmetic: the first layer's input is 0/1, so it is a sum of weight rows; it is computed EXACTLY: the weights are converted once to
- * fixed point (int32, the largest |weight| just below 2^30) and summed in 64-bit integers, then scaled back and biased in f32.  The sum
- * is therefore independent of the order of its terms, which lets qg_search_run update it from the observation entries that changed
- * instead of recomputing it, with bit-identical results.  The other layers are f32 FMA chains over ascending input index. */
+ * follows every layer but the last.  Limits: 1..8 layers, widths <= 1024 (the last layer's width counts the value column of
+ * qg_policy_create_value), and the CTA's shared-memory plan must fit 210 KB, which caps obs_size well below 65535 (QG_ERR_UNSUPPORTED).
+ * Arithmetic (tests/test_policy_fused_envelope.py restates it bit for bit):
+ * - First layer: its input is 0/1, so it is a sum of weight rows, computed EXACTLY.  The weights (with the value column when the network
+ *   has one layer) are converted once to fixed point, q = rint(w * 2^shift) with ties to even, shift = min(30 - e, 120) where
+ *   2^(e-1) <= max |w| < 2^e (shift = 30 when every weight is 0), and summed in 64-bit integers; then h = b + float(float(sum) * 2^-shift)
+ *   in f32.  The sum is independent of the order of its terms, which lets qg_search_run update it from the observation entries that
+ *   changed instead of recomputing it, with bit-identical results.
+ * - Other layers: f32 fused multiply-adds in partial chains over the inputs, combined with f32 adds in a fixed order.  The inputs are
+ *   read in tiles of kt = max(1, 8192 / stride) rows, stride = the layer's width rounded up to a multiple of 4, and split by their
+ *   position u within the tile (not by their global index):
+ *     width > 256:      2 chains, chain c takes u = c, c + 2, ..;  chain 0 starts from the bias, chain 1 from 0;  z = c0 + c1
+ *     width 65..256:    4 chains, u = c, c + 4, ..;  chain 0 starts from the bias, the others from 0;  z = ((c0 + c1) + c2) + c3
+ *     width <= 64:      16 chains, u = c, c + 16, .., all start from 0;  z = ((((0 + c0) + c1) + ..) + c15) + b
+ *   Each chain runs over the tiles in order.  The order is fixed by the shape alone, so a row's outputs do not depend on the batch,
+ *   the other rows or the launch, and qg_search_run decides exactly as the per-decision launches do.
+ * - Softmax over the A action logits (the value column is not part of it): lane l of a warp takes a = l, l + 32, .. for the max and
+ *   the sum of expf(z - max), the lanes are combined by an xor butterfly (offsets 16, 8, 4, 2, 1), p = expf(z - max) * (1 / sum). */
 QG_API int qg_policy_create(int32_t device, int32_t obs_size, int32_t num_layers, const int32_t* out_features,
                             const float* const* weights_host, const float* const* biases_host, qg_policy** out);
 /* The same with the BasicPolicy's value head (a single Linear from the last common layer to one output, examples/models/{*}.pt

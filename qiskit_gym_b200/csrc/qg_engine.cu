@@ -910,7 +910,20 @@ int qg_search_run(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t m
     a.magic_vpe = e->magic_vpe; a.magic_a4 = e->magic_a4; a.symplectic = e->all_symplectic ? 1 : 0;
     a.magic_ow = magic40(((uint32_t)e->L.obs_size + 31u) / 32u);
     const size_t step_smem = (size_t)e->sm_warp_words * 4 + 16;
-    if (policy_smem_bytes(pol->d) + step_smem > 220 * 1024) { set_error("qg_search_run: policy + env do not fit one SM's shared memory"); return QG_ERR_UNSUPPORTED; }
+    {   // the bytes launch_search_fused will request (policy + step region + the CTA's action weights + static) against the device's limit
+        size_t dyn = 0, stat = 0, limit = 0;
+        switch (e->L.kind) {
+            case QG_ENV_PERMUTATION: CUDA_OK(search_fused_smem<QG_ENV_PERMUTATION>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
+            case QG_ENV_LINEAR_FUNCTION: CUDA_OK(search_fused_smem<QG_ENV_LINEAR_FUNCTION>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
+            case QG_ENV_CLIFFORD: CUDA_OK(search_fused_smem<QG_ENV_CLIFFORD>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
+            default: CUDA_OK(search_fused_smem<QG_ENV_PAULI_NETWORK>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
+        }
+        if (dyn + stat > limit) {
+            set_error("qg_search_run: policy + env + action weights need " + std::to_string(dyn + stat) + " bytes of shared memory (" + std::to_string(dyn) +
+                      " dynamic + " + std::to_string(stat) + " static), one block may have " + std::to_string(limit));
+            return QG_ERR_UNSUPPORTED;
+        }
+    }
     if (e->B == 0 || max_decisions == 0) return QG_OK;          // (after every support check: a zero-decision call is the caller's probe)
     cudaStream_t st = (cudaStream_t)stream;
     // the policy's first-layer accumulators, one set per CTA of 8 rollouts (grown on first use; a launch in flight on another stream

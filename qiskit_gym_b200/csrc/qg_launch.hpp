@@ -27,5 +27,9 @@ cudaError_t prepare_step_kind(size_t smem_bytes);
 struct PolicyDev;
 template <int KIND>
 cudaError_t launch_search_fused(const DevCfg& c, const StepArgs& a, const PolicyDev& p, int max_decisions, int32_t* decisions_out, size_t step_smem_bytes, long long* acc0, const uint32_t* first_bits, cudaStream_t st);
+// the shared memory a launch_search_fused CTA needs (the dynamic bytes it requests, the kernel's static bytes) and the most one block
+// may have on `device`
+template <int KIND>
+cudaError_t search_fused_smem(const PolicyDev& p, size_t step_smem_bytes, int device, size_t* dynamic_bytes, size_t* static_bytes, size_t* limit);
 
 }  // namespace qg

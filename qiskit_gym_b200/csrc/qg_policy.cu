@@ -14,7 +14,8 @@
 // completing on mbarriers, three tiles in flight, one flat tile schedule across all layers so the pipeline never
 // drains at a layer boundary.  The first layer is an exact gather-sum in fixed point (layer0_fixed in qg_policy_kernels.cuh:
 // 64-bit integer accumulators, order independent), which the one-launch search updates incrementally from the observation
-// bits that changed; the dense layers sum over the input features in ascending order, in f32.
+// bits that changed; the dense layers sum over the input features in f32 FMA chains that split each weight tile's rows over 2, 4 or 16
+// thread groups and combine them in a fixed order (include/qg_engine.h, qg_policy_create, states the order).
 #include <algorithm>
 #include <cmath>
 #include <cstring>

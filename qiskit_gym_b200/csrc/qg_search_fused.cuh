@@ -71,10 +71,28 @@ __global__ void __launch_bounds__(kPolThreads) k_search_fused(const __grid_const
     if (tid == 0 && decisions_out) decisions_out[blockIdx.x] = min(it + 1, max_decisions);
 }
 
+// Dynamic shared memory one k_search_fused CTA asks for: the policy's plan, one warp region of the step kernel and the CTA's action
+// weights (s_probs, [kPolRows][A] floats).  launch_search_fused requests exactly this; search_fused_smem checks it against the device.
+inline size_t search_fused_dynamic_smem(const PolicyDev& p, size_t step_smem_bytes) {
+    return policy_smem_bytes(p) + step_smem_bytes + (size_t)kPolRows * p.num_actions * 4;
+}
+
+template <int KIND>
+cudaError_t search_fused_smem(const PolicyDev& p, size_t step_smem_bytes, int device, size_t* dynamic_bytes, size_t* static_bytes, size_t* limit) {
+    cudaFuncAttributes fa{};
+    cudaError_t e = cudaFuncGetAttributes(&fa, k_search_fused<KIND>);
+    int optin = 0;
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+    *dynamic_bytes = search_fused_dynamic_smem(p, step_smem_bytes);
+    *static_bytes = fa.sharedSizeBytes;                 // the kernel's s_active / s_ret
+    *limit = (size_t)optin;
+    return e;
+}
+
 template <int KIND>
 cudaError_t launch_search_fused(const DevCfg& c, const StepArgs& a, const PolicyDev& p, int max_decisions, int32_t* decisions_out, size_t step_smem_bytes, long long* acc0,
                                 const uint32_t* first_bits, cudaStream_t st) {
-    const size_t smem = policy_smem_bytes(p) + step_smem_bytes + (size_t)kPolRows * p.num_actions * 4;
+    const size_t smem = search_fused_dynamic_smem(p, step_smem_bytes);
     cudaError_t e = cudaFuncSetAttribute(k_search_fused<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const unsigned grid = (unsigned)((c.B + kPolRows - 1) / kPolRows);
