@@ -437,6 +437,32 @@ QG_API int qg_policy_tc_backward(qg_policy_tc* p, int64_t generation, int64_t ba
 QG_API int qg_search_run(qg_engine* e, qg_policy* policy, int32_t deterministic, int32_t max_decisions, uint32_t* obs_bits_dev,
                          float* weights_dev, int32_t* decisions_dev, qg_stream stream);
 
+/* The twisted rollout search: the policy runs in a symmetry frame of the env (its twists, qg_twists_copy of a config with add_perms = 1)
+ * drawn per rollout and decision, as the collector trains it.  Protocol: rollout i (global id g = first_rollout_id + i of qg_search_begin)
+ * decides in frame k = mulhi(philox(seed; g, tick, stream 5), num_twists), tick = its step counter at decision time (the counter that
+ * also keys the decision's sample draw), so k depends on the seed, g and the decision index only.  The policy sees the observation in
+ * frame k (entry i moves to obs_perms[k][i], as qg_twist_bits); env action a weighs probs[act_perm[k][a]] and the arg-max / inverse-CDF
+ * sum run over a in env order (as qg_collect_step_twisted_dev).  Returns, solutions (env action order), keys and the best-rollout rule are
+ * those of the untwisted search; a table holding only the identity reproduces it bit for bit.
+ * Tables (device memory, the caller's): qperm_inv_dev uint8[num_twists][num_qubits], the inverse qubit permutation of every twist (as for
+ * qg_twist_bits); act_perm_dev int32[num_twists][num_actions], the act perms; twist_dev int32[B], each rollout's frame of its current
+ * decision (written by these calls).  Permutation (<= 64 qubits), LinearFunction and Clifford; QG_ERR_UNSUPPORTED for PauliNetwork (its
+ * symmetry is applied inside the env by add_perms) and for a Permutation without packed observations.
+ * - qg_search_observe_twisted: after qg_set_state and qg_search_begin, the packed observations of the rollouts in the frame of their next
+ *   decision (drawn from their step counters) -> obs_bits_dev uint32[B][qg_obs_words], the frames -> twist_dev.
+ * - qg_search_step_twisted: the counterpart of qg_search_step_bits: picks through act_perm[twist[i]], steps, and writes the next
+ *   observation already in the frame drawn from the post-step tick, updating twist_dev.
+ * - qg_search_run_twisted: qg_search_run for the twisted search, obs_bits_dev / twist_dev as qg_search_observe_twisted left them; its
+ *   decisions are bit-identical to rounds of qg_policy_forward_bits + qg_search_step_twisted. */
+QG_API int qg_search_observe_twisted(qg_engine* e, uint32_t* obs_bits_dev, const uint8_t* qperm_inv_dev, int32_t num_twists, int32_t* twist_dev,
+                                     qg_stream stream);
+QG_API int qg_search_step_twisted(qg_engine* e, const float* weights_dev, int32_t deterministic, uint32_t* obs_bits_dev,
+                                  const uint8_t* qperm_inv_dev, const int32_t* act_perm_dev, int32_t num_twists, int32_t* twist_dev,
+                                  int32_t* chosen_dev, int32_t* num_active_dev, qg_stream stream);
+QG_API int qg_search_run_twisted(qg_engine* e, qg_policy* policy, int32_t deterministic, int32_t max_decisions, uint32_t* obs_bits_dev,
+                                 float* weights_dev, int32_t* decisions_dev, const uint8_t* qperm_inv_dev, const int32_t* act_perm_dev,
+                                 int32_t num_twists, int32_t* twist_dev, qg_stream stream);
+
 /* ---- tree search (SURVEY.md §8f row 4: num_mcts_searches > 0, rl/synthesis.py:122-124, rl/configs.py:30-42) ----------------
  * Clone + step through record slots: the engine's batch is a pool of record slots; logical env i (i < count) reads the
  * record in slot src_slot_dev[i], plays actions_dev[i] and writes the result to slot dst_slot_dev[i] (a tree-search child

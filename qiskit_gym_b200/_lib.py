@@ -35,6 +35,7 @@ SYMBOLS = [
     "qg_policy_tc_create", "qg_policy_tc_destroy", "qg_policy_tc_num_actions", "qg_policy_tc_forward_bits", "qg_policy_tc_set_mode",
     "qg_reset_select_dev", "qg_collect_step_dev", "qg_collect_step_twisted_dev", "qg_twist_bits", "qg_policy_tc_load_weights_dev",
     "qg_policy_tc_enable_training", "qg_policy_tc_generation", "qg_policy_tc_backward", "qg_set_state_grouped", "qg_search_best_grouped",
+    "qg_search_observe_twisted", "qg_search_step_twisted", "qg_search_run_twisted",
 ]
 
 
@@ -167,6 +168,9 @@ def lib():
     L.qg_policy_tc_backward.argtypes = [vp, i64, i64, vp, vp, vp, vp, vp, vp, vp]
     L.qg_set_state_grouped.argtypes = [vp, vp, i64, i64, i64, vp]
     L.qg_search_best_grouped.argtypes = [vp, i64, i64, vp, vp, i32, vp, vp]
+    L.qg_search_observe_twisted.argtypes = [vp, vp, vp, i32, vp, vp]
+    L.qg_search_step_twisted.argtypes = [vp, vp, i32, vp, vp, vp, i32, vp, vp, vp, vp]
+    L.qg_search_run_twisted.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp, vp, i32, vp, vp]
     _lib = L
     return L
 

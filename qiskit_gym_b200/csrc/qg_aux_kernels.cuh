@@ -89,10 +89,8 @@ __global__ void k_twist_gather(const float* __restrict__ in, float* __restrict__
     }
 }
 
-// Twists on packed observations (qg_twist_bits).  Every obs perm of a Permutation / LinearFunction / Clifford twist is the lift of a qubit
-// permutation p: entry (r, c) of the d x d observation (d = n or 2n) moves to (lift(r), lift(c)), lift(i) = p[i] for i < n, n + p[i - n]
-// otherwise (qg_host.cpp compute_twists).  qpinv[k] = p^-1 of twist k, so output entry (R, C) is input entry (lift^-1(R), lift^-1(C)) —
-// qg_twist_gather with the inverse obs perm, on bits, from a [K][n] byte table instead of a [K][d*d] index table.
+// Twists on packed observations (qg_twist_bits): twist_word (qg_common.cuh) with qpinv[k] = p^-1 of twist k — qg_twist_gather with the
+// inverse obs perm, on bits, from a [K][n] byte table instead of a [K][d*d] index table.
 // Thread = (env, output word).  Twist index: kidx_in[b], or drawn  mulhi(philox(*seed_dev, first + b, draw, STREAM_TWIST), K)  (the seed
 // is read at run time, so the launch can live in a CUDA graph); written to kidx_out[b] when given.
 __global__ void k_twist_bits(const uint32_t* __restrict__ in, uint32_t* __restrict__ out, int ow, int obs_size, int n, int d,
@@ -104,18 +102,36 @@ __global__ void k_twist_bits(const uint32_t* __restrict__ in, uint32_t* __restri
         const int w = (int)(i - b * ow);
         const uint32_t k = kidx_in ? (uint32_t)kidx_in[b] : __umulhi(philox_draw(*seed_dev, (uint64_t)(first + b), draw, STREAM_TWIST), K);
         if (kidx_out && w == 0) kidx_out[b] = (int32_t)k;
-        const uint8_t* const pk = qpinv + (size_t)k * n;
         const uint32_t* const row = in + (size_t)b * ow;
-        int j = w * 32, R = j / d, Cc = j - R * d;
-        uint32_t acc = 0;
-        for (int bit = 0; bit < 32 && j < obs_size; ++bit, ++j) {
-            const int sr = R < n ? (int)__ldg(pk + R) : n + (int)__ldg(pk + R - n);
-            const int sc = Cc < n ? (int)__ldg(pk + Cc) : n + (int)__ldg(pk + Cc - n);
-            const int s = sr * d + sc;
-            acc |= ((__ldg(row + (s >> 5)) >> (s & 31)) & 1u) << bit;
-            if (++Cc == d) { Cc = 0; ++R; }
+        out[i] = twist_word([&](int s) { return (__ldg(row + (s >> 5)) >> (s & 31)) & 1u; }, w, obs_size, n, d, qpinv + (size_t)k * n);
+    }
+}
+
+// The twisted search's observation (qg_search_observe_twisted, qg_search_step_twisted): the packed observation of every rollout in the
+// frame of its next decision, k = twist_draw(seed, first_id + b, HD_TICK), read straight from the records (the state bit stream of a
+// LinearFunction / Clifford IS its observation; a Permutation's is the one-hot of its bytes, bit i * n + state[i]); k goes to twist[b].
+// Thread = (rollout, output word).
+template <int KIND>
+__global__ void k_observe_twisted(const __grid_constant__ DevCfg c, uint32_t* __restrict__ out, int ow, const uint8_t* __restrict__ qpinv, uint32_t K, int d,
+                                  int32_t* __restrict__ twist) {
+    const int64_t total = c.B * (int64_t)ow;
+    const int n = c.n;
+    const uint64_t seed = seed_of(c);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t b = i / ow;
+        const int w = (int)(i - b * ow);
+        const uint32_t k = twist_draw(seed, c.first_id + b, c.rec[(size_t)HD_TICK * c.Bpad + b], K);
+        if (w == 0) twist[b] = (int32_t)k;
+        const uint32_t* const st = c.rec + (size_t)c.off_state * c.Bpad + b;         // state word v of rollout b at st[v * Bpad]
+        const uint8_t* const pk = qpinv + (size_t)k * n;
+        if (KIND == QG_ENV_PERMUTATION) {
+            out[i] = twist_word([&](int s) {
+                const int q = s / n;
+                return ((st[(size_t)(q >> 2) * c.Bpad] >> ((q & 3) * 8)) & 0xFFu) == (uint32_t)(s - q * n) ? 1u : 0u;
+            }, w, c.obs_size, n, d, pk);
+        } else {
+            out[i] = twist_word([&](int s) { return (st[(size_t)(s >> 5) * c.Bpad] >> (s & 31)) & 1u; }, w, c.obs_size, n, d, pk);
         }
-        out[i] = acc;
     }
 }
 

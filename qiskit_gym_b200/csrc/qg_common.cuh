@@ -83,6 +83,30 @@ __host__ __device__ __forceinline__ uint32_t philox_draw(uint64_t seed, uint64_t
 
 #ifdef __CUDACC__
 __device__ __forceinline__ uint64_t seed_of(const DevCfg& c) { return c.seed_dev ? *c.seed_dev : c.seed; }
+
+// ---- twists on packed observations ------------------------------------------------------------------------------------------
+// Every obs perm of a Permutation / LinearFunction / Clifford twist is the lift of a qubit permutation p: entry (r, c) of the d x d
+// observation (d = n or 2n) moves to (lift(r), lift(c)), lift(i) = p[i] for i < n, n + p[i - n] otherwise (qg_host.cpp compute_twists).
+// Word w of the observation in the frame whose inverse qubit permutation is pk = p^-1: output entry (R, C) is input entry
+// (lift^-1(R), lift^-1(C)), read through in_bit(entry index).  Every twisted bit of the engine comes from here (qg_twist_bits, the
+// twisted search's observations and the one-launch twisted search).
+template <class InBit>
+__device__ __forceinline__ uint32_t twist_word(const InBit& in_bit, int w, int obs_size, int n, int d, const uint8_t* __restrict__ pk) {
+    int j = w * 32, R = j / d, Cc = j - R * d;
+    uint32_t acc = 0;
+    for (int bit = 0; bit < 32 && j < obs_size; ++bit, ++j) {
+        const int sr = R < n ? (int)__ldg(pk + R) : n + (int)__ldg(pk + R - n);
+        const int sc = Cc < n ? (int)__ldg(pk + Cc) : n + (int)__ldg(pk + Cc - n);
+        acc |= (uint32_t)in_bit(sr * d + sc) << bit;
+        if (++Cc == d) { Cc = 0; ++R; }
+    }
+    return acc;
+}
+// The twist frame of a rollout's decision in the twisted search: mulhi(philox(seed; global rollout id, tick, STREAM_TWIST), K), keyed on
+// the step counter HD_TICK like the decision's sample draw.
+__device__ __forceinline__ uint32_t twist_draw(uint64_t seed, int64_t id, uint32_t tick, uint32_t K) {
+    return __umulhi(philox_draw(seed, (uint64_t)id, tick, STREAM_TWIST), K);
+}
 // ---- per-thread word array living in shared memory with stride EPC (bank == lane, conflict free
 //      for any per-thread dynamic index) ------------------------------------------------------------
 template <int EPC>

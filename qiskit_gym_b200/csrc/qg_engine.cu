@@ -896,8 +896,13 @@ int qg_copy_records(qg_engine* dst, const int32_t* dst_slot_dev, qg_engine* src,
     return QG_OK;
 }
 
-int qg_search_run(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t max_decisions, uint32_t* obs_bits_dev, float* weights_dev,
-                  int32_t* decisions_dev, qg_stream stream) {
+}  // extern "C"
+
+namespace {
+
+// qg_search_run and qg_search_run_twisted (tw: the twisted search's tables, a.act_perm = act_perm_dev; null: untwisted)
+int search_run(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t max_decisions, uint32_t* obs_bits_dev, float* weights_dev,
+               int32_t* decisions_dev, const SearchTwist* tw, const int32_t* act_perm_dev, qg_stream stream) {
     if (!e || !pol || !obs_bits_dev || !weights_dev) { set_error("null argument"); return QG_ERR_INVALID; }
     if (pol->device != e->device) { set_error("qg_search_run: policy and engine live on different devices"); return QG_ERR_INVALID; }
     if (pol->d.obs_size != e->L.obs_size || pol->d.num_actions != e->L.A) { set_error("qg_search_run: the policy's observation size / action count do not match the env"); return QG_ERR_INVALID; }
@@ -905,6 +910,7 @@ int qg_search_run(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t m
     if (max_decisions < 0) { set_error("qg_search_run: negative decision budget"); return QG_ERR_INVALID; }
     CUDA_OK(cudaSetDevice(e->device));
     StepArgs a{}; a.weights = weights_dev; a.deterministic = deterministic;      // (no packed-observation output: the kernel keeps the bit stream on chip)
+    if (tw) { a.act_perm = act_perm_dev; a.twist = tw->twist; }
     a.nsteps = 1; a.ring = 1; a.pdl_mode = 0; a.num_sms = e->num_sms;
     a.sm_warp_words = e->sm_warp_words; a.sm_scr = e->sm_scr; a.sm_obs = e->sm_obs; a.sm_cat = -1; a.sm_wts = -1; a.magic_obs = e->magic_obs; a.magic_A = e->magic_A;
     a.magic_vpe = e->magic_vpe; a.magic_a4 = e->magic_a4; a.symplectic = e->all_symplectic ? 1 : 0;
@@ -913,10 +919,14 @@ int qg_search_run(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t m
     {   // the bytes launch_search_fused will request (policy + step region + the CTA's action weights + static) against the device's limit
         size_t dyn = 0, stat = 0, limit = 0;
         switch (e->L.kind) {
-            case QG_ENV_PERMUTATION: CUDA_OK(search_fused_smem<QG_ENV_PERMUTATION>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
-            case QG_ENV_LINEAR_FUNCTION: CUDA_OK(search_fused_smem<QG_ENV_LINEAR_FUNCTION>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
-            case QG_ENV_CLIFFORD: CUDA_OK(search_fused_smem<QG_ENV_CLIFFORD>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
-            default: CUDA_OK(search_fused_smem<QG_ENV_PAULI_NETWORK>(pol->d, step_smem, e->device, &dyn, &stat, &limit)); break;
+            case QG_ENV_PERMUTATION: CUDA_OK((tw ? search_fused_smem<QG_ENV_PERMUTATION, true>(pol->d, step_smem, e->device, &dyn, &stat, &limit)
+                                                        : search_fused_smem<QG_ENV_PERMUTATION, false>(pol->d, step_smem, e->device, &dyn, &stat, &limit))); break;
+            case QG_ENV_LINEAR_FUNCTION: CUDA_OK((tw ? search_fused_smem<QG_ENV_LINEAR_FUNCTION, true>(pol->d, step_smem, e->device, &dyn, &stat, &limit)
+                                                        : search_fused_smem<QG_ENV_LINEAR_FUNCTION, false>(pol->d, step_smem, e->device, &dyn, &stat, &limit))); break;
+            case QG_ENV_CLIFFORD: CUDA_OK((tw ? search_fused_smem<QG_ENV_CLIFFORD, true>(pol->d, step_smem, e->device, &dyn, &stat, &limit)
+                                                        : search_fused_smem<QG_ENV_CLIFFORD, false>(pol->d, step_smem, e->device, &dyn, &stat, &limit))); break;
+            default: CUDA_OK((tw ? search_fused_smem<QG_ENV_PAULI_NETWORK, true>(pol->d, step_smem, e->device, &dyn, &stat, &limit)
+                                                        : search_fused_smem<QG_ENV_PAULI_NETWORK, false>(pol->d, step_smem, e->device, &dyn, &stat, &limit))); break;
         }
         if (dyn + stat > limit) {
             set_error("qg_search_run: policy + env + action weights need " + std::to_string(dyn + stat) + " bytes of shared memory (" + std::to_string(dyn) +
@@ -935,12 +945,78 @@ int qg_search_run(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t m
         pol->acc0_ctas = ctas;
     }
     switch (e->L.kind) {
-        case QG_ENV_PERMUTATION: CUDA_OK(launch_search_fused<QG_ENV_PERMUTATION>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, st)); break;
-        case QG_ENV_LINEAR_FUNCTION: CUDA_OK(launch_search_fused<QG_ENV_LINEAR_FUNCTION>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, st)); break;
-        case QG_ENV_CLIFFORD: CUDA_OK(launch_search_fused<QG_ENV_CLIFFORD>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, st)); break;
-        default: CUDA_OK(launch_search_fused<QG_ENV_PAULI_NETWORK>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, st)); break;
+        case QG_ENV_PERMUTATION: CUDA_OK(launch_search_fused<QG_ENV_PERMUTATION>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, tw, st)); break;
+        case QG_ENV_LINEAR_FUNCTION: CUDA_OK(launch_search_fused<QG_ENV_LINEAR_FUNCTION>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, tw, st)); break;
+        case QG_ENV_CLIFFORD: CUDA_OK(launch_search_fused<QG_ENV_CLIFFORD>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, tw, st)); break;
+        default: CUDA_OK(launch_search_fused<QG_ENV_PAULI_NETWORK>(e->dc, a, pol->d, max_decisions, decisions_dev, step_smem, pol->acc0, obs_bits_dev, tw, st)); break;
     }
     return QG_OK;
+}
+
+// Arguments of the twisted search's entry points: the tables are given, K >= 1; PauliNetwork (its symmetry is applied inside the env by
+// add_perms) and a Permutation without packed observations (> 64 qubits) have no twisted search.
+int check_twisted(const qg_engine* e, const uint8_t* qperm_inv_dev, const int32_t* act_perm_dev, bool need_act, int32_t num_twists, const int32_t* twist_dev) {
+    if (!e || !qperm_inv_dev || (need_act && !act_perm_dev) || !twist_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (num_twists < 1) { set_error("the twisted search needs num_twists >= 1"); return QG_ERR_INVALID; }
+    if (e->L.kind == QG_ENV_PAULI_NETWORK) { set_error("PauliNetwork has no twisted search: its qubit symmetry is applied inside the env (add_perms)"); return QG_ERR_UNSUPPORTED; }
+    if (e->L.kind == QG_ENV_PERMUTATION && e->L.OW == 0) { set_error("packed observations need num_qubits <= 64 for Permutation"); return QG_ERR_UNSUPPORTED; }
+    return QG_OK;
+}
+
+int launch_observe_twisted(qg_engine* e, uint32_t* obs_bits_dev, const uint8_t* qperm_inv_dev, int32_t num_twists, int32_t* twist_dev, cudaStream_t st) {
+    if (e->B == 0) return QG_OK;
+    const int ow = (e->L.obs_size + 31) / 32, d = e->L.kind == QG_ENV_CLIFFORD ? 2 * e->L.n : e->L.n;
+    const int64_t total = e->B * (int64_t)ow;
+    const unsigned grid = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16);
+    switch (e->L.kind) {
+        case QG_ENV_PERMUTATION: k_observe_twisted<QG_ENV_PERMUTATION><<<grid, 256, 0, st>>>(e->dc, obs_bits_dev, ow, qperm_inv_dev, (uint32_t)num_twists, d, twist_dev); break;
+        case QG_ENV_LINEAR_FUNCTION: k_observe_twisted<QG_ENV_LINEAR_FUNCTION><<<grid, 256, 0, st>>>(e->dc, obs_bits_dev, ow, qperm_inv_dev, (uint32_t)num_twists, d, twist_dev); break;
+        default: k_observe_twisted<QG_ENV_CLIFFORD><<<grid, 256, 0, st>>>(e->dc, obs_bits_dev, ow, qperm_inv_dev, (uint32_t)num_twists, d, twist_dev); break;
+    }
+    CUDA_OK(cudaGetLastError());
+    return QG_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int qg_search_run(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t max_decisions, uint32_t* obs_bits_dev, float* weights_dev,
+                  int32_t* decisions_dev, qg_stream stream) {
+    return search_run(e, pol, deterministic, max_decisions, obs_bits_dev, weights_dev, decisions_dev, nullptr, nullptr, stream);
+}
+
+int qg_search_observe_twisted(qg_engine* e, uint32_t* obs_bits_dev, const uint8_t* qperm_inv_dev, int32_t num_twists, int32_t* twist_dev, qg_stream stream) {
+    const int rc = check_twisted(e, qperm_inv_dev, nullptr, false, num_twists, twist_dev);
+    if (rc != QG_OK) return rc;
+    if (!obs_bits_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    CUDA_OK(cudaSetDevice(e->device));
+    return launch_observe_twisted(e, obs_bits_dev, qperm_inv_dev, num_twists, twist_dev, (cudaStream_t)stream);
+}
+
+int qg_search_step_twisted(qg_engine* e, const float* weights_dev, int32_t deterministic, uint32_t* obs_bits_dev, const uint8_t* qperm_inv_dev,
+                           const int32_t* act_perm_dev, int32_t num_twists, int32_t* twist_dev, int32_t* chosen_dev, int32_t* num_active_dev, qg_stream stream) {
+    const int rc = check_twisted(e, qperm_inv_dev, act_perm_dev, true, num_twists, twist_dev);
+    if (rc != QG_OK) return rc;
+    if (!weights_dev || !obs_bits_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    if (num_active_dev) CUDA_OK(cudaMemsetAsync(num_active_dev, 0, 4, st));
+    // the existing twisted step (the sampler reads weights[act_perm[twist[i]][a]], qg_collect_step_twisted_dev's path), then the next
+    // observation in the frame drawn from the post-step tick
+    StepArgs a{}; a.weights = weights_dev; a.deterministic = deterministic; a.chosen = chosen_dev; a.num_active = num_active_dev;
+    a.act_perm = act_perm_dev; a.twist = twist_dev;
+    const int src = launch_step(e, MODE_SEARCH, a, st);
+    if (src != QG_OK) return src;
+    return launch_observe_twisted(e, obs_bits_dev, qperm_inv_dev, num_twists, twist_dev, st);
+}
+
+int qg_search_run_twisted(qg_engine* e, qg_policy* pol, int32_t deterministic, int32_t max_decisions, uint32_t* obs_bits_dev, float* weights_dev,
+                          int32_t* decisions_dev, const uint8_t* qperm_inv_dev, const int32_t* act_perm_dev, int32_t num_twists, int32_t* twist_dev,
+                          qg_stream stream) {
+    const int rc = check_twisted(e, qperm_inv_dev, act_perm_dev, true, num_twists, twist_dev);
+    if (rc != QG_OK) return rc;
+    const SearchTwist tw{qperm_inv_dev, twist_dev, (uint32_t)num_twists, e->L.kind == QG_ENV_CLIFFORD ? 2 * e->L.n : e->L.n};
+    return search_run(e, pol, deterministic, max_decisions, obs_bits_dev, weights_dev, decisions_dev, &tw, act_perm_dev, stream);
 }
 
 int qg_search_best(qg_engine* e, int64_t* best_key_host, int64_t* best_env_host, qg_stream stream) {

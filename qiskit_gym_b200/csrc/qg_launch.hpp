@@ -23,13 +23,22 @@ cudaError_t launch_step_kind(int mode, int inv, const DevCfg& c, const StepArgs&
 template <int KIND>
 cudaError_t prepare_step_kind(size_t smem_bytes);
 
-// the whole rollout search in one launch (qg_search_fused.cuh); step_smem_bytes = one warp region of the step kernel
+// the whole rollout search in one launch (qg_search_fused.cuh); step_smem_bytes = one warp region of the step kernel; tw: the twisted
+// search's tables, or null
 struct PolicyDev;
+// The twisted search's tables (k_search_fused<KIND, true>; the launch's a.act_perm holds the [K][A] act perms and a.twist = twist).
+struct SearchTwist {
+    const uint8_t* qpinv;        // [K][n] inverse qubit permutation of every twist (collector.qubit_twist_table)
+    int32_t* twist;              // [B] the frame of each rollout's current decision
+    uint32_t K;
+    int32_t d;                   // side of the square observation: n (Permutation, LinearFunction) or 2n (Clifford)
+};
 template <int KIND>
-cudaError_t launch_search_fused(const DevCfg& c, const StepArgs& a, const PolicyDev& p, int max_decisions, int32_t* decisions_out, size_t step_smem_bytes, long long* acc0, const uint32_t* first_bits, cudaStream_t st);
+cudaError_t launch_search_fused(const DevCfg& c, const StepArgs& a, const PolicyDev& p, int max_decisions, int32_t* decisions_out, size_t step_smem_bytes, long long* acc0, const uint32_t* first_bits,
+                                const SearchTwist* tw, cudaStream_t st);
 // the shared memory a launch_search_fused CTA needs (the dynamic bytes it requests, the kernel's static bytes) and the most one block
 // may have on `device`
-template <int KIND>
+template <int KIND, bool TWIST>
 cudaError_t search_fused_smem(const PolicyDev& p, size_t step_smem_bytes, int device, size_t* dynamic_bytes, size_t* static_bytes, size_t* limit);
 
 }  // namespace qg

@@ -101,7 +101,9 @@ cudaError_t prepare_step_kind(size_t smem_bytes) {
 #define QG_INSTANTIATE_KIND(KIND)                                                                                              \
     template cudaError_t launch_step_kind<KIND>(int, int, const DevCfg&, const StepArgs&, const LaunchGeom&, cudaStream_t);    \
     template cudaError_t prepare_step_kind<KIND>(size_t);                                                                      \
-    template cudaError_t launch_search_fused<KIND>(const DevCfg&, const StepArgs&, const PolicyDev&, int, int32_t*, size_t, long long*, const uint32_t*, cudaStream_t); \
-    template cudaError_t search_fused_smem<KIND>(const PolicyDev&, size_t, int, size_t*, size_t*, size_t*);
+    template cudaError_t launch_search_fused<KIND>(const DevCfg&, const StepArgs&, const PolicyDev&, int, int32_t*, size_t, long long*, const uint32_t*,            \
+                                                   const SearchTwist*, cudaStream_t);                                                           \
+    template cudaError_t search_fused_smem<KIND, false>(const PolicyDev&, size_t, int, size_t*, size_t*, size_t*);                             \
+    template cudaError_t search_fused_smem<KIND, true>(const PolicyDev&, size_t, int, size_t*, size_t*, size_t*);
 
 }  // namespace qg

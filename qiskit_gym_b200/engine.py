@@ -474,6 +474,47 @@ class BatchedEnv:
         check(lib().qg_search_run(self._h, policy._h, 1 if deterministic else 0, int(max_decisions), _dptr(obs_bits), _dptr(weights),
                                   _dptr(decisions), self._stream()))
 
+    # ------------------------------------------------------------------ twisted search (the policy in a symmetry frame per rollout and decision)
+    def _twist_args(self, qperm_inv: torch.Tensor, twist: torch.Tensor, act_table: torch.Tensor | None = None):
+        assert qperm_inv.dtype == torch.uint8 and qperm_inv.is_cuda and qperm_inv.is_contiguous() and qperm_inv.dim() == 2
+        assert qperm_inv.shape[1] == int(self.cfg.num_qubits)
+        assert twist.dtype == torch.int32 and twist.is_cuda and twist.is_contiguous() and twist.numel() == self.batch
+        assert act_table is None or (act_table.dtype == torch.int32 and act_table.is_cuda and act_table.is_contiguous()
+                                     and tuple(act_table.shape) == (qperm_inv.shape[0], self._A))
+        return int(qperm_inv.shape[0])
+
+    def search_observe_twisted(self, obs_bits: torch.Tensor, qperm_inv: torch.Tensor, twist: torch.Tensor):
+        """qg_search_observe_twisted: after set_state and search_begin, every rollout's packed observation in the frame of its next decision
+        (drawn from the engine's seed, the rollout's global id and its step counter) -> obs_bits int32 [B, obs_words], the frames -> twist
+        int32 [B].  qperm_inv: uint8 [K, n] (collector.qubit_twist_table)."""
+        assert obs_bits.is_cuda and obs_bits.element_size() == 4 and obs_bits.is_contiguous() and obs_bits.numel() == self.batch * self.obs_words()
+        K = self._twist_args(qperm_inv, twist)
+        check(lib().qg_search_observe_twisted(self._h, _dptr(obs_bits), _dptr(qperm_inv), K, _dptr(twist), self._stream()))
+        return obs_bits
+
+    def search_step_twisted(self, weights: torch.Tensor, obs_bits: torch.Tensor, qperm_inv: torch.Tensor, act_table: torch.Tensor,
+                            twist: torch.Tensor, deterministic: bool = False, chosen: torch.Tensor | None = None,
+                            num_active: torch.Tensor | None = None):
+        """search_step_bits of the twisted search (qg_search_step_twisted): env action g of rollout i weighs weights[i, act_table[twist[i], g]];
+        the next observation is written in the frame drawn from the post-step counter, twist updated.  act_table: int32 [K, A]."""
+        assert weights.dtype == torch.float32 and weights.is_cuda and weights.is_contiguous() and weights.numel() == self.batch * self._A
+        assert obs_bits.is_cuda and obs_bits.element_size() == 4 and obs_bits.is_contiguous() and obs_bits.numel() == self.batch * self.obs_words()
+        K = self._twist_args(qperm_inv, twist, act_table)
+        check(lib().qg_search_step_twisted(self._h, _dptr(weights), 1 if deterministic else 0, _dptr(obs_bits), _dptr(qperm_inv), _dptr(act_table), K,
+                                           _dptr(twist), _dptr(chosen), _dptr(num_active), self._stream()))
+        return obs_bits
+
+    def search_run_twisted(self, policy, obs_bits: torch.Tensor, weights: torch.Tensor, max_decisions: int, qperm_inv: torch.Tensor,
+                           act_table: torch.Tensor, twist: torch.Tensor, deterministic: bool = False, decisions: torch.Tensor | None = None):
+        """search_run of the twisted search (qg_search_run_twisted); call set_state, search_begin and search_observe_twisted(obs_bits, ..,
+        twist) first."""
+        assert weights.dtype == torch.float32 and weights.is_cuda and weights.is_contiguous() and weights.numel() == self.batch * self._A
+        assert obs_bits.is_cuda and obs_bits.element_size() == 4 and obs_bits.is_contiguous() and obs_bits.numel() == self.batch * self.obs_words()
+        assert decisions is None or (decisions.dtype == torch.int32 and decisions.numel() >= (self.batch + 7) // 8)
+        K = self._twist_args(qperm_inv, twist, act_table)
+        check(lib().qg_search_run_twisted(self._h, policy._h, 1 if deterministic else 0, int(max_decisions), _dptr(obs_bits), _dptr(weights),
+                                          _dptr(decisions), _dptr(qperm_inv), _dptr(act_table), K, _dptr(twist), self._stream()))
+
     def search_best(self):
         key, env = C.c_int64(), C.c_int64()
         check(lib().qg_search_best(self._h, C.byref(key), C.byref(env), self._stream()))

@@ -16,7 +16,7 @@ import json
 
 import torch
 
-from .search import BasicPolicy, RolloutSearch, check_tensor_core_search, chunk_plan
+from .search import BasicPolicy, RolloutSearch, check_tensor_core_search, check_twisted_search, chunk_plan
 from .specs import SynthSpec
 
 _ENV_KINDS = {"PermutationEnv": 0, "LinearFunctionEnv": 1, "CliffordEnv": 2, "PauliNetworkEnv": 3}
@@ -87,26 +87,33 @@ class RLSynthesis:
         kw = {k: v for k, v in cfg.items() if k not in ("num_qubits", "gateset")}
         return _ENV_KINDS[self.env.cls_name], cfg["num_qubits"], cfg["gateset"], {**kw, **override}
 
-    def _search(self, num_searches: int, targets_per_launch: int | None = None, matmul_precision: str = "f32") -> RolloutSearch:
+    def _search(self, num_searches: int, targets_per_launch: int | None = None, matmul_precision: str = "f32", use_twists: bool = False) -> RolloutSearch:
         """The cached search of `num_searches` rollouts per target: the single-target one, or with targets_per_launch the one solve_many
         uses (rebuilt only when a call needs more targets per launch than it holds).  matmul_precision="tensor_core": the "tensor_core"
         backend, cached under its own key (it never replaces the f32 search) and with no fall-back.  A search refreshes its policy handle
-        from self.policy itself, so a weight update does not rebuild it."""
+        from self.policy itself, so a weight update does not rebuild it.
+        use_twists: the twisted search (RolloutSearch(use_twists=True)), cached under its own key; where the one-launch search cannot run
+        it raises instead of falling back to the untwisted "torch" backend."""
         key = num_searches if targets_per_launch is None else ("many", num_searches)
         if matmul_precision == "tensor_core":
             key = ("tensor_core", key)
+        if use_twists:
+            key = ("twisted", key)
         rs = self._searches.get(key)
         if rs is not None and targets_per_launch is not None and rs.targets_per_launch < targets_per_launch:
             rs = None
         if rs is None:
             self._searches.pop(key, None)                # (frees the old engine before the new one allocates)
-            kind, n, gs, kw = self._env_args(add_perms=False)
+            kind, n, gs, kw = self._env_args(add_perms=bool(use_twists))
 
             def make(backend):
                 return RolloutSearch(kind, n, gs, self.policy, num_searches, device=self.device, policy_backend=backend,
-                                     targets_per_launch=targets_per_launch or 1, **kw)
+                                     targets_per_launch=targets_per_launch or 1, use_twists=use_twists, **kw)
             if matmul_precision == "tensor_core":
                 rs = make("tensor_core")
+            elif use_twists:
+                rs = make("persistent")
+                rs.check_supported()
             else:
                 try:
                     rs = make("persistent")
@@ -128,10 +135,23 @@ class RLSynthesis:
             self._searches[key] = ms
         return ms
 
+    def _check_twists(self, use_twists: bool, num_mcts_searches: int):
+        """The refusals of use_twists=True, before anything is allocated: the tree search stays untwisted, and the twisted search has no
+        PauliNetwork / wide-Permutation form (search.check_twisted_search)."""
+        if not use_twists:
+            return
+        if num_mcts_searches:
+            raise NotImplementedError("use_twists applies to the rollout search (num_mcts_searches = 0); the tree search runs untwisted")
+        check_twisted_search(_ENV_KINDS[self.env.cls_name], self.env_config["num_qubits"], "persistent")
+
     def solve(self, state, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
-              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False):
+              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False, use_twists: bool = False):
         """twisterl `Algorithm.solve`: the action list of the best successful rollout, or None.
-        reuse_tree (tree search only): every decision but the first starts from the subtree below the action played (mcts.MCTSSearch)."""
+        reuse_tree (tree search only): every decision but the first starts from the subtree below the action played (mcts.MCTSSearch).
+        use_twists: every rollout runs the policy in a symmetry frame of the env drawn per decision, as the reference's twisted policy
+        does (RolloutSearch(use_twists=True)); NotImplementedError with num_mcts_searches > 0, for PauliNetwork and for a Permutation
+        wider than 64 qubits."""
+        self._check_twists(use_twists, num_mcts_searches)
         if reuse_tree and not num_mcts_searches:
             raise ValueError("reuse_tree needs a tree search (num_mcts_searches > 0)")
         if num_mcts_searches:
@@ -139,10 +159,10 @@ class RLSynthesis:
                 raise NotImplementedError("max_expand_depth != 1 is not supported by the device tree search (mcts.py)")
             return self._mcts(int(num_searches), int(num_mcts_searches), float(C), bool(reuse_tree)).solve(state, deterministic=deterministic,
                                                                                                              seed=seed).actions
-        return self._search(int(num_searches)).solve(state, deterministic=deterministic, seed=seed).actions
+        return self._search(int(num_searches), use_twists=use_twists).solve(state, deterministic=deterministic, seed=seed).actions
 
     def solve_many(self, states, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
-                   max_rollouts: int = 65536, matmul_precision: str = "f32"):
+                   max_rollouts: int = 65536, matmul_precision: str = "f32", use_twists: bool = False):
         """`solve` for many targets in few launches: a list with, for each state, the action list of its best successful rollout or None.
         Target t's result is that of solve(states[t]) on rollout ids t*num_searches .. (t+1)*num_searches - 1 (search.RolloutSearch.solve_many),
         so solve_many([x])[0] == solve(x).  Up to max_rollouts rollouts run per launch (the one-launch search keeps ~4 KB of first-layer
@@ -150,7 +170,10 @@ class RLSynthesis:
         matmul_precision: "f32" (the default: the searches of solve) or "tensor_core" (RolloutSearch's "tensor_core" backend: the policy on
         tcgen05 tensor cores, for large launches).  The two round differently, so "tensor_core" results equal a single-target "tensor_core"
         search, not solve(); it raises NotImplementedError where it cannot run (more than 127 actions, a Permutation wider than 64 qubits, a
-        device that is not sm_100) instead of falling back to another arithmetic."""
+        device that is not sm_100) instead of falling back to another arithmetic.
+        use_twists: the twisted search (solve's use_twists); target t's result is that of solve(states[t], use_twists=True) on rollout ids
+        t*num_searches ..."""
+        self._check_twists(use_twists, num_mcts_searches)
         if num_mcts_searches:
             raise NotImplementedError("solve_many runs rollout searches only (num_mcts_searches = 0): use solve() for the tree search")
         if matmul_precision not in ("f32", "tensor_core"):
@@ -165,15 +188,16 @@ class RLSynthesis:
         if not states:
             return []
         tpl = min(len(states), max(1, int(max_rollouts) // num_searches))
-        res = self._search(num_searches, tpl, matmul_precision).solve_many(states, deterministic=deterministic, seed=seed)
+        res = self._search(num_searches, tpl, matmul_precision, use_twists).solve_many(states, deterministic=deterministic, seed=seed)
         return [r.actions for r in res]
 
     def synth_many(self, inputs, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
-                   max_rollouts: int = 65536, matmul_precision: str = "f32"):
+                   max_rollouts: int = 65536, matmul_precision: str = "f32", use_twists: bool = False):
         """`synth` for many inputs (solve_many): a list of circuits (or gate lists), None where a target has no successful rollout."""
+        self._check_twists(use_twists, num_mcts_searches)
         inputs = list(inputs)
         actions = self.solve_many([self.env.get_state(x) for x in inputs], deterministic, num_searches, num_mcts_searches, seed, max_rollouts,
-                                  matmul_precision)
+                                  matmul_precision, use_twists)
         out = []
         for x, a in zip(inputs, actions):
             if a is None:
@@ -184,10 +208,13 @@ class RLSynthesis:
         return out
 
     def synth(self, input, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
-              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False):
-        """rl/synthesis.py:112-126.  Returns the synthesised circuit (QuantumCircuit with Qiskit, else a gate list) or None."""
+              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False, use_twists: bool = False):
+        """rl/synthesis.py:112-126.  Returns the synthesised circuit (QuantumCircuit with Qiskit, else a gate list) or None.
+        use_twists: see solve."""
+        self._check_twists(use_twists, num_mcts_searches)
         state = self.env.get_state(input)
-        actions = self.solve(state, deterministic, num_searches, num_mcts_searches, C, max_expand_depth, seed=seed, reuse_tree=reuse_tree)
+        actions = self.solve(state, deterministic, num_searches, num_mcts_searches, C, max_expand_depth, seed=seed, reuse_tree=reuse_tree,
+                             use_twists=use_twists)
         if actions is not None:
             return self.env.build_circuit_from_solution(actions, input)
 

@@ -106,6 +106,18 @@ def check_tensor_core_search(env_kind: int, num_qubits: int, num_actions: int, d
         raise NotImplementedError("the tensor-core search needs an sm_100 device (tcgen05)")
 
 
+def check_twisted_search(env_kind: int, num_qubits: int, policy_backend: str):
+    """Raises NotImplementedError where the twisted search (RolloutSearch(use_twists=True)) cannot run: the "torch" backend, PauliNetwork
+    (its qubit symmetry is applied inside the env by add_perms), a Permutation wider than 64 qubits (no packed observations).  Needs no
+    device."""
+    if policy_backend == "torch":
+        raise NotImplementedError("the twisted search runs on the packed-observation backends (persistent, fused, tensor_core), not torch")
+    if env_kind == _abi.ENV_PAULI_NETWORK:
+        raise NotImplementedError("PauliNetwork has no twisted search: its qubit symmetry is applied inside the env (add_perms)")
+    if env_kind == _abi.ENV_PERMUTATION and num_qubits > 64:
+        raise NotImplementedError(f"the twisted search needs packed observations: a Permutation of {num_qubits} > 64 qubits has none")
+
+
 def reduce_best(local_key: int, local_solution, group=None, device=None):
     """Cross-rank best-rollout reduction in two collectives: an all-gather of (packed key, solution length) — the owner of the winning
     rollout is the rank holding the largest key; keys are unique, they embed the global rollout id — then the owner broadcasts its action
@@ -163,7 +175,7 @@ class RolloutSearch:
 
     def __init__(self, env_kind, num_qubits, gateset, policy: torch.nn.Module, num_rollouts: int, device=None,
                  max_depth: int = 128, use_cuda_graph: bool = True, policy_backend: str = "persistent", targets_per_launch: int = 1,
-                 **env_kwargs):
+                 use_twists: bool = False, **env_kwargs):
         """policy_backend: "persistent" = the whole search in ONE kernel launch (qg_search_run: every CTA loops policy -> sample ->
         step for its 8 rollouts); "fused" = two launches per decision (policy.FusedPolicy + qg_search_step_bits) in a CUDA graph;
         "torch" = dense f32 observations + the PyTorch module (cuBLAS GEMMs, softmax).  "persistent" and "fused" take identical
@@ -179,11 +191,21 @@ class RolloutSearch:
         update (optimizer step, load_state_dict) or another module assigned to `policy` is what the next search runs.  "tensor_core" copies
         a weight update into the handle in place (captured graphs stay valid).
         targets_per_launch: solve_many searches that many targets together, each with its own `num_rollouts` rollouts (the engine
-        holds targets_per_launch * num_rollouts); solve() needs targets_per_launch == 1."""
-        env_kwargs.setdefault("add_perms", False)
+        holds targets_per_launch * num_rollouts); solve() needs targets_per_launch == 1.
+        use_twists: the twisted search (include/qg_engine.h qg_search_run_twisted): every rollout runs the policy, at every decision, in a
+        symmetry frame of the env (its twists() with add_perms, as the collector trains it) drawn from the seed, the rollout's global id
+        and the decision index; the env's actions are weighed through the frame's act perm.  Backends "persistent", "fused" and
+        "tensor_core"; Permutation (<= 64 qubits), LinearFunction and Clifford.  NotImplementedError, before anything is allocated, for
+        "torch", PauliNetwork (its symmetry is applied inside the env) and a Permutation wider than 64 qubits."""
         if targets_per_launch < 1:
             raise ValueError("targets_per_launch must be >= 1")
         assert policy_backend in ("persistent", "fused", "torch", "tensor_core")
+        if use_twists:
+            check_twisted_search(env_kind, num_qubits, policy_backend)
+            if env_kwargs.get("add_perms") is False:
+                raise ValueError("use_twists needs the env's twists: add_perms=False contradicts it")
+            env_kwargs["add_perms"] = True
+        env_kwargs.setdefault("add_perms", False)
         self.env_kind, self.num_qubits = env_kind, num_qubits
         self.R, self.targets_per_launch = num_rollouts, targets_per_launch
         self.env = BatchedEnv(env_kind, num_qubits, gateset, targets_per_launch * num_rollouts, device=device, max_depth=max_depth, **env_kwargs)
@@ -204,8 +226,19 @@ class RolloutSearch:
             self.obs_bits = self.env.new_obs_bits()
         self.probs = torch.zeros((self.B, self.env.num_actions()), dtype=torch.float32, device=dev)
         self.num_active = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.use_twists = bool(use_twists)
+        self.qperm_table = self.act_table = self.twist = None
+        if self.use_twists:
+            # the env's twists, once, on the device: uint8 [K, n] inverse qubit permutations, int32 [K, A] act perms; the frames int32 [B]
+            from .collector import qubit_twist_table
+            obs_perms, act_perms = self.env.twists()
+            self.qperm_table = torch.from_numpy(qubit_twist_table(obs_perms, num_qubits)).to(dev)
+            self.act_table = torch.from_numpy(np.asarray(act_perms, dtype=np.int32)).to(dev)
+            self.twist = torch.zeros(self.B, dtype=torch.int32, device=dev)
+        self.num_twists = 0 if self.qperm_table is None else int(self.qperm_table.shape[0])
         self.use_graph = use_cuda_graph
-        self.hook = None            # tests: hook(probs, obs_bits) sees every decision's policy output before the step reads it (no graph)
+        self.hook = None            # tests: hook(probs, obs_bits) sees every decision's policy output before the step reads it (no graph);
+                                    # twisted searches call hook(probs, obs_bits, twist) with the decision's frames
         self._graphs = {}
         self._stream = torch.cuda.Stream(device=dev)
         self._decisions = torch.zeros((self.B + 7) // 8, dtype=torch.int32, device=dev)
@@ -218,11 +251,24 @@ class RolloutSearch:
         """Raises NotImplementedError (QG_ERR_UNSUPPORTED) now rather than in the first solve() when the one-launch search cannot run
         this env / policy pair: a zero-decision qg_search_run goes through all of its checks without launching anything."""
         if self.backend == "persistent":
-            self.env.search_run(self.handle, self.obs_bits, self.probs, 0, deterministic=True, decisions=self._decisions)
+            self._run(0, True)
+
+    def _run(self, max_decisions, deterministic):
+        if self.use_twists:
+            self.env.search_run_twisted(self.handle, self.obs_bits, self.probs, max_decisions, self.qperm_table, self.act_table, self.twist,
+                                        deterministic=deterministic, decisions=self._decisions)
+        else:
+            self.env.search_run(self.handle, self.obs_bits, self.probs, max_decisions, deterministic=deterministic, decisions=self._decisions)
 
     def _iteration(self, deterministic):
         if self.backend in ("fused", "tensor_core"):
             self.handle.forward_bits(self.obs_bits, probs=self.probs)
+            if self.use_twists:
+                if self.hook is not None:
+                    self.hook(self.probs, self.obs_bits, self.twist)
+                self.env.search_step_twisted(self.probs, self.obs_bits, self.qperm_table, self.act_table, self.twist, deterministic=deterministic,
+                                             num_active=self.num_active)
+                return
             if self.hook is not None:
                 self.hook(self.probs, self.obs_bits)
             self.env.search_step_bits(self.probs, self.obs_bits, deterministic=deterministic, num_active=self.num_active)
@@ -233,7 +279,9 @@ class RolloutSearch:
         self.env.search_step(self.probs, deterministic=deterministic, obs=True, num_active=self.num_active)
 
     def _observe(self):
-        if self.backend != "torch":
+        if self.use_twists:
+            self.env.search_observe_twisted(self.obs_bits, self.qperm_table, self.twist)
+        elif self.backend != "torch":
             self.env.observe_bits(self.obs_bits)
         else:
             self.env.observe()
@@ -270,7 +318,7 @@ class RolloutSearch:
             load()
             env.search_begin(seed, first_rollout_id)
             self._observe()
-            env.search_run(self.handle, self.obs_bits, self.probs, self.max_depth, deterministic=deterministic, decisions=self._decisions)
+            self._run(self.max_depth, deterministic)
             return None
         load()
         use_graph = self.use_graph and self.hook is None
