@@ -514,6 +514,35 @@ QG_API int qg_mcts_reroot(const qg_mcts_tree* t, qg_engine* pool, const qg_engin
 QG_API int qg_mcts_begin_keep(const qg_mcts_tree* t, const float* root_prior_dev, const uint8_t* root_final_dev, const uint8_t* reused_dev,
                               qg_stream stream);
 
+/* The twisted tree search: every policy evaluation of a tree runs in a symmetry frame of the env (its twists, qg_twists_copy of a config
+ * with add_perms = 1).  Tree i belongs to the rollout with global id g = first_rollout_id + i; evaluation e = 0 is its root, e = s + 1 the
+ * leaf created by simulation s of the decision.  Its frame is  k(i, e) = mulhi(philox(seed; g + (e << 32), tick_i, stream 5), num_twists),
+ * tick_i = the rollout's step counter at decision time, so k(i, 0) is the frame qg_search_observe_twisted draws.  The policy sees the node's
+ * observation in frame k (entry j moves to obs_perms[k][j], as qg_twist_bits); the node stores its prior in env action order,
+ * P(a) = probs[act_perm[k][a]]; the value is used as is.  PUCT, back-up, root weights, re-rooting and the decision do not change.  A table
+ * holding only the identity reproduces the untwisted search bit for bit.  Permutation (<= 64 qubits), LinearFunction and Clifford;
+ * QG_ERR_UNSUPPORTED for PauliNetwork and for a Permutation without packed observations.
+ * search_key_dev uint64[2] = {seed, first_rollout_id} (those of qg_search_begin) and eval_dev int32[1] = the current evaluation index minus
+ * one are read in device memory when the kernels run, so one captured CUDA graph serves every decision and every seed: the caller rewrites
+ * search_key_dev when the search restarts.  Tables: qperm_inv_dev uint8[num_twists][num_qubits] and act_perm_dev int32[num_twists][num_actions]
+ * as for qg_search_run_twisted; twist_dev int32[num_trees] holds the frame of each tree's last evaluation.
+ * - qg_mcts_observe_twisted, root pass (pool NULL): the root observations, read from `rollouts` records, in frames k(i, 0) ->
+ *   obs_bits_dev uint32[num_trees][qg_obs_words], the frames -> twist_dev; resets *eval_dev to 0.  Leaf pass (after qg_mcts_select and
+ *   qg_step_slots): tree i with action_dev[i] >= 0 observes pool slot dst_slot_dev[i] in frame k(i, *eval_dev + 1); the other trees' rows
+ *   and frames are left untouched.  The tick and the ids come from `rollouts`, which must not step during the decision.
+ * - qg_mcts_begin_twisted / qg_mcts_begin_keep_twisted: qg_mcts_begin / qg_mcts_begin_keep with root_prior_dev in frames twist_dev.
+ * - qg_mcts_backup_twisted: qg_mcts_backup with prior_dev in frames twist_dev; then advances *eval_dev by one (the simulation is over). */
+QG_API int qg_mcts_observe_twisted(const qg_engine* rollouts, const qg_engine* pool, const int32_t* dst_slot_dev, const int32_t* action_dev,
+                                   const uint64_t* search_key_dev, int32_t* eval_dev, const uint8_t* qperm_inv_dev, int32_t num_twists,
+                                   uint32_t* obs_bits_dev, int32_t* twist_dev, qg_stream stream);
+QG_API int qg_mcts_begin_twisted(const qg_mcts_tree* t, const float* root_prior_dev, const uint8_t* root_final_dev, const int32_t* act_perm_dev,
+                                 int32_t num_twists, const int32_t* twist_dev, qg_stream stream);
+QG_API int qg_mcts_begin_keep_twisted(const qg_mcts_tree* t, const float* root_prior_dev, const uint8_t* root_final_dev, const uint8_t* reused_dev,
+                                      const int32_t* act_perm_dev, int32_t num_twists, const int32_t* twist_dev, qg_stream stream);
+QG_API int qg_mcts_backup_twisted(const qg_mcts_tree* t, const float* prior_dev, const float* value_dev, const float* reward_dev,
+                                  const uint8_t* done_dev, const int32_t* act_perm_dev, int32_t num_twists, const int32_t* twist_dev,
+                                  int32_t* eval_dev, qg_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

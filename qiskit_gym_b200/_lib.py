@@ -36,6 +36,7 @@ SYMBOLS = [
     "qg_reset_select_dev", "qg_collect_step_dev", "qg_collect_step_twisted_dev", "qg_twist_bits", "qg_policy_tc_load_weights_dev",
     "qg_policy_tc_enable_training", "qg_policy_tc_generation", "qg_policy_tc_backward", "qg_set_state_grouped", "qg_search_best_grouped",
     "qg_search_observe_twisted", "qg_search_step_twisted", "qg_search_run_twisted",
+    "qg_mcts_observe_twisted", "qg_mcts_begin_twisted", "qg_mcts_begin_keep_twisted", "qg_mcts_backup_twisted",
 ]
 
 
@@ -137,6 +138,10 @@ def lib():
     L.qg_mcts_root_weights.argtypes = [treep, vp, vp]
     L.qg_mcts_reroot.argtypes = [treep, vp, vp, vp, i32, vp, vp]
     L.qg_mcts_begin_keep.argtypes = [treep, vp, vp, vp, vp]
+    L.qg_mcts_observe_twisted.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
+    L.qg_mcts_begin_twisted.argtypes = [treep, vp, vp, vp, i32, vp, vp]
+    L.qg_mcts_begin_keep_twisted.argtypes = [treep, vp, vp, vp, vp, i32, vp, vp]
+    L.qg_mcts_backup_twisted.argtypes = [treep, vp, vp, vp, vp, vp, i32, vp, vp, vp]
     L.qg_search_run.argtypes = [vp, vp, i32, i32, vp, vp, vp, vp]
     L.qg_solutions.argtypes = [vp, i64, i64, vp, i32, vp, vp]
     L.qg_solutions_host.argtypes = [vp, i64, i64, vp, i32, vp, vp]

@@ -108,9 +108,8 @@ __global__ void k_twist_bits(const uint32_t* __restrict__ in, uint32_t* __restri
 }
 
 // The twisted search's observation (qg_search_observe_twisted, qg_search_step_twisted): the packed observation of every rollout in the
-// frame of its next decision, k = twist_draw(seed, first_id + b, HD_TICK), read straight from the records (the state bit stream of a
-// LinearFunction / Clifford IS its observation; a Permutation's is the one-hot of its bytes, bit i * n + state[i]); k goes to twist[b].
-// Thread = (rollout, output word).
+// frame of its next decision, k = twist_draw(seed, first_id + b, HD_TICK), read straight from the records (record_twist_word); k goes to
+// twist[b].  Thread = (rollout, output word).
 template <int KIND>
 __global__ void k_observe_twisted(const __grid_constant__ DevCfg c, uint32_t* __restrict__ out, int ow, const uint8_t* __restrict__ qpinv, uint32_t K, int d,
                                   int32_t* __restrict__ twist) {
@@ -123,15 +122,7 @@ __global__ void k_observe_twisted(const __grid_constant__ DevCfg c, uint32_t* __
         const uint32_t k = twist_draw(seed, c.first_id + b, c.rec[(size_t)HD_TICK * c.Bpad + b], K);
         if (w == 0) twist[b] = (int32_t)k;
         const uint32_t* const st = c.rec + (size_t)c.off_state * c.Bpad + b;         // state word v of rollout b at st[v * Bpad]
-        const uint8_t* const pk = qpinv + (size_t)k * n;
-        if (KIND == QG_ENV_PERMUTATION) {
-            out[i] = twist_word([&](int s) {
-                const int q = s / n;
-                return ((st[(size_t)(q >> 2) * c.Bpad] >> ((q & 3) * 8)) & 0xFFu) == (uint32_t)(s - q * n) ? 1u : 0u;
-            }, w, c.obs_size, n, d, pk);
-        } else {
-            out[i] = twist_word([&](int s) { return (st[(size_t)(s >> 5) * c.Bpad] >> (s & 31)) & 1u; }, w, c.obs_size, n, d, pk);
-        }
+        out[i] = record_twist_word<KIND>(st, c.Bpad, w, c.obs_size, n, d, qpinv + (size_t)k * n);
     }
 }
 

@@ -102,6 +102,19 @@ __device__ __forceinline__ uint32_t twist_word(const InBit& in_bit, int w, int o
     }
     return acc;
 }
+// twist_word of an env's observation read straight from its record (st = the record's first state word, word v at st[v * bpad]): the state
+// bit stream of a LinearFunction / Clifford IS its observation; a Permutation's is the one-hot of its bytes, bit i * n + state[i].
+// (bpad by reference: k_observe_twisted hands in its grid constant's Bpad, read where it is used, as the code was before this helper.)
+template <int KIND>
+__device__ __forceinline__ uint32_t record_twist_word(const uint32_t* st, const int64_t& bpad, int w, int obs_size, int n, int d, const uint8_t* __restrict__ pk) {
+    if (KIND == QG_ENV_PERMUTATION) {
+        return twist_word([&](int s) {
+            const int q = s / n;
+            return ((st[(size_t)(q >> 2) * bpad] >> ((q & 3) * 8)) & 0xFFu) == (uint32_t)(s - q * n) ? 1u : 0u;
+        }, w, obs_size, n, d, pk);
+    }
+    return twist_word([&](int s) { return (st[(size_t)(s >> 5) * bpad] >> (s & 31)) & 1u; }, w, obs_size, n, d, pk);
+}
 // The twist frame of a rollout's decision in the twisted search: mulhi(philox(seed; global rollout id, tick, STREAM_TWIST), K), keyed on
 // the step counter HD_TICK like the decision's sample draw.
 __device__ __forceinline__ uint32_t twist_draw(uint64_t seed, int64_t id, uint32_t tick, uint32_t K) {

@@ -21,6 +21,17 @@
 //                node's parent), renumbered in that order so that c becomes node 0; prior, N, W, remapped children, reward, final flag
 //                and pool record move with each node.  An edge whose child was dropped keeps N and W and gets child = -1.  The root keeps
 //                its stored prior (qg_mcts_begin_keep skips it); every other tree starts fresh.  The decision then adds S simulations.
+//   twists (opt-in, MCTSSearch(use_twists=True); restated in tests/test_mcts_twist.py): tree i belongs to the rollout with global id
+//                g = first_id + i, and each policy evaluation of the tree runs in its own symmetry frame of the env.  Evaluation e = 0 is
+//                the root, e = s + 1 the leaf created by simulation s; its frame is
+//                    k(i, e) = mulhi(philox(seed; g + (e << 32), tick_i, STREAM_TWIST), K)
+//                with tick_i the rollout's HD_TICK at decision time and K the number of twists (env.twists() with add_perms).  For e = 0
+//                this is the twisted rollout search's twist_draw (global ids stay below 2^30, so the high word never meets a rollout id).
+//                The policy sees the node's observation in frame k (twist_word, the bits of qg_twist_bits / k_observe_twisted); the node
+//                stores its prior in env action order, P(a) = probs[act_perm[k][a]]; the value is used as is.  Everything else above is
+//                unchanged; a re-rooted tree keeps its env-order priors.  seed, first_id and e are read in device memory at run time
+//                (e: a counter the root pass resets and each twisted back-up advances), so the captured decision graphs stay valid for
+//                every decision and seed.
 // Every f32 operation is rounded on its own (no FMA contraction) so the CPU restatement reproduces each argmax.
 //
 // Decomposition: one warp per tree; lanes stride over the actions of a node for the PUCT arg-max and for initialising a
@@ -41,11 +52,14 @@ __device__ __forceinline__ void warp_argmax(float& s, int& a) {
     }
 }
 
-__device__ __forceinline__ void begin_tree(const qg_mcts_tree& t, int tree, int lane, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final) {
+// TWIST: the priors come in the policy's frame; env action a takes root_prior[perm[a]] (perm = the act perm of the tree's frame)
+template <bool TWIST>
+__device__ __forceinline__ void begin_tree(const qg_mcts_tree& t, int tree, int lane, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final,
+                                           const int32_t* __restrict__ perm) {
     const size_t base = (size_t)tree * t.node_cap;
     for (int a = lane; a < t.num_actions; a += 32) {
         const size_t k = base * t.num_actions + a;
-        t.prior[k] = root_prior[(size_t)tree * t.num_actions + a];
+        t.prior[k] = root_prior[(size_t)tree * t.num_actions + (TWIST ? __ldg(perm + a) : a)];
         t.visits[k] = 0; t.value_sum[k] = 0.0f; t.child[k] = -1;
     }
     if (lane == 0) { t.node_count[tree] = 1; t.node_reward[base] = 0.0f; t.node_final[base] = root_final[tree] ? 1 : 0; t.path_len[tree] = 0; t.new_node[tree] = -1; }
@@ -54,14 +68,58 @@ __device__ __forceinline__ void begin_tree(const qg_mcts_tree& t, int tree, int 
 __global__ void k_mcts_begin(const qg_mcts_tree t, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final) {
     const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
     if (tree >= t.num_trees) return;
-    begin_tree(t, tree, lane, root_prior, root_final);
+    begin_tree<false>(t, tree, lane, root_prior, root_final, nullptr);
 }
 
 __global__ void k_mcts_begin_keep(const qg_mcts_tree t, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final,
                                   const uint8_t* __restrict__ reused) {
     const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
     if (tree >= t.num_trees || reused[tree]) return;
-    begin_tree(t, tree, lane, root_prior, root_final);
+    begin_tree<false>(t, tree, lane, root_prior, root_final, nullptr);
+}
+
+// The twisted forms (qg_mcts_begin_twisted, qg_mcts_begin_keep_twisted): tree i's root priors came in frame twist[i].
+__global__ void k_mcts_begin_twisted(const qg_mcts_tree t, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final,
+                                     const int32_t* __restrict__ act_perm, const int32_t* __restrict__ twist) {
+    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (tree >= t.num_trees) return;
+    begin_tree<true>(t, tree, lane, root_prior, root_final, act_perm + (size_t)twist[tree] * t.num_actions);
+}
+
+__global__ void k_mcts_begin_keep_twisted(const qg_mcts_tree t, const float* __restrict__ root_prior, const uint8_t* __restrict__ root_final,
+                                          const uint8_t* __restrict__ reused, const int32_t* __restrict__ act_perm, const int32_t* __restrict__ twist) {
+    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (tree >= t.num_trees || reused[tree]) return;
+    begin_tree<true>(t, tree, lane, root_prior, root_final, act_perm + (size_t)twist[tree] * t.num_actions);
+}
+
+// The twisted search's node observation (qg_mcts_observe_twisted).  Root pass (dst_slot null): tree i evaluates the rollout's env, read
+// from the rollout engine's record i, in frame k(i, 0), and the evaluation counter is reset to 0.  Leaf pass: tree i evaluates the node
+// created by the current simulation, pool record dst_slot[i], in frame k(i, *eval + 1); trees that created none (action[i] < 0) are
+// skipped.  k(i, e) = mulhi(philox(seed; g + (e << 32), tick_i, STREAM_TWIST), K), g = first rollout id + i, tick_i = the rollout's HD_TICK;
+// seed and first id come from key[0..1] at run time, as does e, so a captured graph draws the frames of every replay.
+// Thread = (tree, output word), as k_observe_twisted.
+template <int KIND>
+__global__ void k_mcts_observe_twisted(const __grid_constant__ DevCfg c, const uint32_t* __restrict__ leaf_rec, int64_t leaf_bpad,
+                                       const int32_t* __restrict__ dst_slot, const int32_t* __restrict__ action, const uint64_t* __restrict__ key,
+                                       int32_t* eval, uint32_t* __restrict__ out, int ow, const uint8_t* __restrict__ qpinv, uint32_t K, int d,
+                                       int32_t* __restrict__ twist) {
+    const bool leaf = dst_slot != nullptr;
+    const int64_t total = c.B * (int64_t)ow;
+    const int n = c.n;
+    const uint64_t seed = key[0];
+    const int64_t first = (int64_t)key[1];
+    const uint32_t e = leaf ? (uint32_t)*eval + 1u : 0u;
+    if (!leaf && blockIdx.x == 0 && threadIdx.x == 0) *eval = 0;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t b = i / ow;
+        const int w = (int)(i - b * ow);
+        if (leaf && action[b] < 0) continue;
+        const uint32_t k = twist_draw(seed, first + b + ((int64_t)e << 32), c.rec[(size_t)HD_TICK * c.Bpad + b], K);
+        if (w == 0) twist[b] = (int32_t)k;
+        const uint32_t* const st = leaf ? leaf_rec + (size_t)c.off_state * leaf_bpad + dst_slot[b] : c.rec + (size_t)c.off_state * c.Bpad + b;
+        out[i] = record_twist_word<KIND>(st, leaf ? leaf_bpad : c.Bpad, w, c.obs_size, n, d, qpinv + (size_t)k * n);
+    }
 }
 
 // Re-rooting (protocol above).  path_node of tree i holds the old -> new node id map: >= 0 kept under that id, -2 a member of c's subtree
@@ -170,17 +228,18 @@ __global__ void k_mcts_select(const qg_mcts_tree t, float c_puct, int32_t* __res
     }
 }
 
-__global__ void k_mcts_backup(const qg_mcts_tree t, const float* __restrict__ prior_in, const float* __restrict__ value_in,
-                              const float* __restrict__ reward_in, const uint8_t* __restrict__ done_in) {
-    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
-    if (tree >= t.num_trees) return;
+// TWIST: as begin_tree; perm_of() gives the act perm of the frame the new node was evaluated in
+template <bool TWIST, class PermOf>
+__device__ __forceinline__ void backup_tree(const qg_mcts_tree& t, int tree, int lane, const float* __restrict__ prior_in, const float* __restrict__ value_in,
+                                            const float* __restrict__ reward_in, const uint8_t* __restrict__ done_in, const PermOf& perm_of) {
     const size_t base = (size_t)tree * t.node_cap;
     const int A = t.num_actions, len = t.path_len[tree], newn = t.new_node[tree];
     float v = 0.0f;
     if (newn >= 0) {
         const size_t row = (base + newn) * A;
+        const int32_t* const perm = perm_of();
         for (int a = lane; a < A; a += 32) {
-            t.prior[row + a] = prior_in[(size_t)tree * A + a];
+            t.prior[row + a] = prior_in[(size_t)tree * A + (TWIST ? __ldg(perm + a) : a)];
             t.visits[row + a] = 0; t.value_sum[row + a] = 0.0f; t.child[row + a] = -1;
         }
         const bool fin = done_in[tree] != 0;
@@ -197,6 +256,23 @@ __global__ void k_mcts_backup(const qg_mcts_tree t, const float* __restrict__ pr
             t.value_sum[k] = __fadd_rn(t.value_sum[k], G);
         }
     }
+}
+
+__global__ void k_mcts_backup(const qg_mcts_tree t, const float* __restrict__ prior_in, const float* __restrict__ value_in,
+                              const float* __restrict__ reward_in, const uint8_t* __restrict__ done_in) {
+    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (tree >= t.num_trees) return;
+    backup_tree<false>(t, tree, lane, prior_in, value_in, reward_in, done_in, [] { return (const int32_t*)nullptr; });
+}
+
+// qg_mcts_backup_twisted: the leaf priors came in frame twist[i]; the simulation is over, so the evaluation counter advances
+__global__ void k_mcts_backup_twisted(const qg_mcts_tree t, const float* __restrict__ prior_in, const float* __restrict__ value_in,
+                                      const float* __restrict__ reward_in, const uint8_t* __restrict__ done_in, const int32_t* __restrict__ act_perm,
+                                      const int32_t* __restrict__ twist, int32_t* __restrict__ eval) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) *eval += 1;
+    const int tree = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (tree >= t.num_trees) return;
+    backup_tree<true>(t, tree, lane, prior_in, value_in, reward_in, done_in, [&] { return act_perm + (size_t)twist[tree] * t.num_actions; });
 }
 
 __global__ void k_mcts_root_weights(const qg_mcts_tree t, float* __restrict__ weights) {
@@ -298,6 +374,89 @@ int qg_mcts_begin_keep(const qg_mcts_tree* t, const float* root_prior_dev, const
     if (!root_prior_dev || !root_final_dev || !reused_dev) { set_error("null argument"); return QG_ERR_INVALID; }
     if (t->num_trees == 0) return QG_OK;
     k_mcts_begin_keep<<<tree_grid(t), 128, 0, (cudaStream_t)stream>>>(*t, root_prior_dev, root_final_dev, reused_dev);
+    MCTS_LAUNCHED();
+    return QG_OK;
+}
+
+// ---- the twisted tree search (protocol above) ----------------------------------------------------------------------------------------
+static int check_act_twist(const int32_t* act_perm_dev, int32_t num_twists, const int32_t* twist_dev) {
+    if (!act_perm_dev || !twist_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (num_twists < 1) { set_error("the twisted tree search needs num_twists >= 1"); return QG_ERR_INVALID; }
+    return QG_OK;
+}
+
+int qg_mcts_observe_twisted(const qg_engine* rollouts, const qg_engine* pool, const int32_t* dst_slot_dev, const int32_t* action_dev,
+                            const uint64_t* search_key_dev, int32_t* eval_dev, const uint8_t* qperm_inv_dev, int32_t num_twists,
+                            uint32_t* obs_bits_dev, int32_t* twist_dev, qg_stream stream) {
+    if (!rollouts || !search_key_dev || !eval_dev || !qperm_inv_dev || !obs_bits_dev || !twist_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (pool && (!dst_slot_dev || !action_dev)) { set_error("qg_mcts_observe_twisted: the leaf pass needs dst_slot and action"); return QG_ERR_INVALID; }
+    if (num_twists < 1) { set_error("the twisted tree search needs num_twists >= 1"); return QG_ERR_INVALID; }
+    const Layout& L = rollouts->L;
+    if (L.kind == QG_ENV_PAULI_NETWORK) { set_error("PauliNetwork has no twisted tree search: its qubit symmetry is applied inside the env (add_perms)"); return QG_ERR_UNSUPPORTED; }
+    if (L.kind == QG_ENV_PERMUTATION && L.OW == 0) { set_error("packed observations need num_qubits <= 64 for Permutation"); return QG_ERR_UNSUPPORTED; }
+    if (pool && (pool->L.kind != L.kind || pool->L.n != L.n || pool->L.W != L.W || pool->L.A != L.A || pool->device != rollouts->device || pool->B < rollouts->B)) {
+        set_error("qg_mcts_observe_twisted: the pool must share env kind, qubits, gateset size and device with the rollouts and hold a slot per tree");
+        return QG_ERR_INVALID;
+    }
+    if (rollouts->B == 0) return QG_OK;
+    CUDA_OK(cudaSetDevice(rollouts->device));
+    const int ow = (L.obs_size + 31) / 32, d = L.kind == QG_ENV_CLIFFORD ? 2 * L.n : L.n;
+    const int64_t total = rollouts->B * (int64_t)ow;
+    const unsigned grid = (unsigned)std::min<int64_t>((total + 255) / 256, 148 * 16);
+    const uint32_t* leaf_rec = pool ? pool->dc.rec : nullptr;
+    const int64_t leaf_bpad = pool ? pool->Bpad : 0;
+    const int32_t* slot = pool ? dst_slot_dev : nullptr;
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (L.kind) {
+        case QG_ENV_PERMUTATION:
+            k_mcts_observe_twisted<QG_ENV_PERMUTATION><<<grid, 256, 0, st>>>(rollouts->dc, leaf_rec, leaf_bpad, slot, action_dev, search_key_dev, eval_dev, obs_bits_dev,
+                                                                              ow, qperm_inv_dev, (uint32_t)num_twists, d, twist_dev);
+            break;
+        case QG_ENV_LINEAR_FUNCTION:
+            k_mcts_observe_twisted<QG_ENV_LINEAR_FUNCTION><<<grid, 256, 0, st>>>(rollouts->dc, leaf_rec, leaf_bpad, slot, action_dev, search_key_dev, eval_dev, obs_bits_dev,
+                                                                                  ow, qperm_inv_dev, (uint32_t)num_twists, d, twist_dev);
+            break;
+        default:
+            k_mcts_observe_twisted<QG_ENV_CLIFFORD><<<grid, 256, 0, st>>>(rollouts->dc, leaf_rec, leaf_bpad, slot, action_dev, search_key_dev, eval_dev, obs_bits_dev,
+                                                                           ow, qperm_inv_dev, (uint32_t)num_twists, d, twist_dev);
+            break;
+    }
+    MCTS_LAUNCHED();
+    return QG_OK;
+}
+
+int qg_mcts_begin_twisted(const qg_mcts_tree* t, const float* root_prior_dev, const uint8_t* root_final_dev, const int32_t* act_perm_dev, int32_t num_twists,
+                          const int32_t* twist_dev, qg_stream stream) {
+    int rc = check_tree(t);
+    if (rc == QG_OK) rc = check_act_twist(act_perm_dev, num_twists, twist_dev);
+    if (rc != QG_OK) return rc;
+    if (!root_prior_dev || !root_final_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (t->num_trees == 0) return QG_OK;
+    k_mcts_begin_twisted<<<tree_grid(t), 128, 0, (cudaStream_t)stream>>>(*t, root_prior_dev, root_final_dev, act_perm_dev, twist_dev);
+    MCTS_LAUNCHED();
+    return QG_OK;
+}
+
+int qg_mcts_begin_keep_twisted(const qg_mcts_tree* t, const float* root_prior_dev, const uint8_t* root_final_dev, const uint8_t* reused_dev,
+                               const int32_t* act_perm_dev, int32_t num_twists, const int32_t* twist_dev, qg_stream stream) {
+    int rc = check_tree(t);
+    if (rc == QG_OK) rc = check_act_twist(act_perm_dev, num_twists, twist_dev);
+    if (rc != QG_OK) return rc;
+    if (!root_prior_dev || !root_final_dev || !reused_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (t->num_trees == 0) return QG_OK;
+    k_mcts_begin_keep_twisted<<<tree_grid(t), 128, 0, (cudaStream_t)stream>>>(*t, root_prior_dev, root_final_dev, reused_dev, act_perm_dev, twist_dev);
+    MCTS_LAUNCHED();
+    return QG_OK;
+}
+
+int qg_mcts_backup_twisted(const qg_mcts_tree* t, const float* prior_dev, const float* value_dev, const float* reward_dev, const uint8_t* done_dev,
+                           const int32_t* act_perm_dev, int32_t num_twists, const int32_t* twist_dev, int32_t* eval_dev, qg_stream stream) {
+    int rc = check_tree(t);
+    if (rc == QG_OK) rc = check_act_twist(act_perm_dev, num_twists, twist_dev);
+    if (rc != QG_OK) return rc;
+    if (!prior_dev || !value_dev || !reward_dev || !done_dev || !eval_dev) { set_error("null argument"); return QG_ERR_INVALID; }
+    if (t->num_trees == 0) return QG_OK;
+    k_mcts_backup_twisted<<<tree_grid(t), 128, 0, (cudaStream_t)stream>>>(*t, prior_dev, value_dev, reward_dev, done_dev, act_perm_dev, twist_dev, eval_dev);
     MCTS_LAUNCHED();
     return QG_OK;
 }

@@ -54,6 +54,7 @@ class BatchedEnv:
         self.done = torch.zeros(B, dtype=torch.bool, device=dev)
         self.success = torch.zeros(B, dtype=torch.bool, device=dev)
         self._twists = None
+        self.search_key = (0, 0)            # (seed, first rollout id) of the last search_begin
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -379,6 +380,7 @@ class BatchedEnv:
 
     def search_begin(self, seed: int = 0, first_rollout_id: int = 0):
         check(lib().qg_search_begin(self._h, C.c_uint64(seed & (2**64 - 1)), first_rollout_id, self._stream()))
+        self.search_key = (seed & (2**64 - 1), int(first_rollout_id))      # (the twisted tree search hands them to its kernels)
 
     def search_step(self, weights: torch.Tensor, deterministic: bool = False, obs: torch.Tensor | None | bool = True,
                     chosen: torch.Tensor | None = None, num_active: torch.Tensor | None = None):

@@ -11,6 +11,10 @@ a child node's env is the parent's record cloned and stepped in one pass through
 With `reuse_tree=True` a decision starts from the subtree below the action the rollout played (AlphaGo Zero's tree reuse), kept
 when the tree's node for it holds the env the rollout reached (csrc/qg_mcts.cu states the rule).
 
+With `use_twists=True` every policy evaluation of a tree (its root, each new leaf) runs in a symmetry frame of the env drawn per
+rollout, decision and evaluation, the way the collector trains the policy; the trees keep their priors in env action order
+(csrc/qg_mcts.cu states the protocol).
+
 twisterl's own tree search is not in the reference tree: the protocol (stated in csrc/qg_mcts.cu) is this engine's, and
 `max_expand_depth` — whose exact meaning cannot be recovered from the reference — is accepted and must be 1.
 """
@@ -24,7 +28,7 @@ import torch
 from . import _abi
 from ._lib import check, lib
 from .engine import BatchedEnv, _dptr
-from .search import SearchResult, best_rollout, search_result
+from .search import SearchResult, best_rollout, check_twisted_search, search_result, twist_tables
 
 
 class TreeArrays:
@@ -63,6 +67,41 @@ class TreeArrays:
     def begin_keep(self, root_prior, root_final, reused):
         check(lib().qg_mcts_begin_keep(C.byref(self.c), _dptr(root_prior), _dptr(root_final), _dptr(reused), self._st()))
 
+    # the twisted forms: priors in the policy's frame twist[i] (act_table int32 [K, A]), stored in env action order
+    def begin_twisted(self, root_prior, root_final, act_table, twist, reused=None):
+        K = int(act_table.shape[0])
+        if reused is None:
+            check(lib().qg_mcts_begin_twisted(C.byref(self.c), _dptr(root_prior), _dptr(root_final), _dptr(act_table), K, _dptr(twist), self._st()))
+        else:
+            check(lib().qg_mcts_begin_keep_twisted(C.byref(self.c), _dptr(root_prior), _dptr(root_final), _dptr(reused), _dptr(act_table), K,
+                                                   _dptr(twist), self._st()))
+
+    def backup_twisted(self, prior, value, reward, done, act_table, twist, eval_index):
+        check(lib().qg_mcts_backup_twisted(C.byref(self.c), _dptr(prior), _dptr(value), _dptr(reward), _dptr(done), _dptr(act_table),
+                                           int(act_table.shape[0]), _dptr(twist), _dptr(eval_index), self._st()))
+
+
+def observe_twisted(rollouts: BatchedEnv, pool: BatchedEnv | None, dst_slot, action, search_key, eval_index, qperm_table, obs_bits, twist):
+    """qg_mcts_observe_twisted: the root pass (pool None) or the leaf pass of the twisted tree search -> packed bits obs_bits int32
+    [R, obs_words] and frames twist int32 [R].  search_key int64 [2] = (seed, first rollout id), eval_index int32 [1]: device memory."""
+    check(lib().qg_mcts_observe_twisted(rollouts._h, None if pool is None else pool._h, _dptr(dst_slot), _dptr(action), _dptr(search_key),
+                                        _dptr(eval_index), _dptr(qperm_table), int(qperm_table.shape[0]), _dptr(obs_bits), _dptr(twist),
+                                        rollouts._stream()))
+
+
+def check_twisted_tree_search(env_kind: int, num_qubits: int, policy: torch.nn.Module, policy_backend: str, env_kwargs: dict):
+    """Raises, before anything is allocated, where the twisted tree search cannot run: NotImplementedError for the "torch" backend, a
+    policy without single-Linear action / value heads (nothing fused to run), PauliNetwork and a Permutation wider than 64 qubits;
+    ValueError for an explicit add_perms=False."""
+    from .policy import simple_value_head
+    if policy_backend == "torch":
+        raise NotImplementedError("the twisted tree search evaluates packed observations on the fused policy, not the torch backend")
+    check_twisted_search(env_kind, num_qubits, "fused")
+    if simple_value_head(policy) is None:
+        raise NotImplementedError("the twisted tree search runs the fused policy: it needs single-Linear action / value heads")
+    if env_kwargs.get("add_perms") is False:
+        raise ValueError("use_twists needs the env's twists: add_perms=False contradicts it")
+
 
 class MCTSSearch:
     """`solve` with a tree search per decision.  Owns the rollout engine (R envs, solutions tracked) and a slot-pool engine of
@@ -70,7 +109,7 @@ class MCTSSearch:
 
     def __init__(self, env_kind, num_qubits, gateset, policy: torch.nn.Module, num_rollouts: int, num_mcts_searches: int, C: float = 2 ** 0.5,
                  device=None, max_depth: int = 128, use_cuda_graph: bool = True, policy_backend: str = "auto", reuse_tree: bool = False,
-                 **env_kwargs):
+                 use_twists: bool = False, **env_kwargs):
         """use_cuda_graph: a decision's launches (root evaluation, then per simulation PUCT descent -> clone + step -> policy -> back-up)
         are captured once and replayed: the whole decision as one graph up to 128 simulations, one graph per simulation beyond.
         policy_backend: "fused" = priors and values of the root / the leaves from packed observations in one kernel (policy.FusedPolicy
@@ -79,8 +118,16 @@ class MCTSSearch:
         reuse_tree: each decision after the first of a `solve` keeps up to num_mcts_searches + 1 nodes of the subtree below the action
         the rollout played, with their statistics, and adds num_mcts_searches simulations to them (qg_mcts_reroot).  The rollout's
         action must then reach `decide` through `chosen` (solve does it; a caller driving decide itself passes chosen=self.chosen
-        to search_step).  `reused[i]` tells whether tree i was kept at the last decision."""
+        to search_step).  `reused[i]` tells whether tree i was kept at the last decision.
+        use_twists: the twisted tree search (include/qg_engine.h qg_mcts_observe_twisted): the root and every new leaf are evaluated in
+        a symmetry frame of the env (its twists() with add_perms) drawn from the seed and first rollout id of env.search_begin, the
+        rollout's global id, its step counter and the evaluation index; the node stores P(a) = probs[act_perm[k][a]].  Runs on the fused
+        backend; `root_twist` holds the root frames of the last decision and `root_bits` the twisted root observations.  Raises before
+        anything is allocated where it cannot run (check_twisted_tree_search)."""
         assert num_mcts_searches >= 1 and policy_backend in ("auto", "fused", "torch")
+        if use_twists:
+            check_twisted_tree_search(env_kind, num_qubits, policy, policy_backend, env_kwargs)
+            env_kwargs["add_perms"] = True
         env_kwargs.setdefault("add_perms", False)
         self.env = BatchedEnv(env_kind, num_qubits, gateset, num_rollouts, device=device, max_depth=max_depth, **env_kwargs)
         pool_kwargs = dict(env_kwargs, track_solution=False)
@@ -104,7 +151,8 @@ class MCTSSearch:
         self.reused = torch.zeros(self.R, dtype=torch.uint8, device=dev)       # 1: tree i was re-rooted at the last decision
         self._fresh = True          # chosen is all -1: the next decision starts every tree afresh
         self.num_active = torch.zeros(1, dtype=torch.int32, device=dev)
-        self.hook = None            # tests: hook(kind, decision, simulation, tensors...) sees the policy outputs the trees consumed
+        self.hook = None            # tests: hook(kind, decision, simulation, prior, value) sees the policy outputs the trees consumed;
+                                    # twisted searches call hook(kind, decision, simulation, prior, value, frames, obs_bits)
         from .policy import FusedPolicy, simple_value_head
         can_fuse = simple_value_head(self.policy) is not None and not (env_kind == 0 and num_qubits > 64)      # (no packed observations for n > 64 permutations)
         if policy_backend == "fused" and not can_fuse:
@@ -117,6 +165,16 @@ class MCTSSearch:
             self.pri = torch.zeros((self.R, A), dtype=torch.float32, device=dev)
             self.val = torch.zeros(self.R, dtype=torch.float32, device=dev)
             self.fused = FusedPolicy(self.policy, device=dev, with_value=True)
+        self.use_twists = bool(use_twists)
+        self.num_twists = 0
+        if self.use_twists:
+            self.qperm_table, self.act_table = twist_tables(self.env)
+            self.num_twists = int(self.act_table.shape[0])
+            self.root_twist = torch.zeros(self.R, dtype=i32, device=dev)      # frames of the root evaluations of the last decision
+            self.leaf_twist = torch.zeros(self.R, dtype=i32, device=dev)      # frames of the last simulation's leaf evaluations
+            self.search_key = torch.zeros(2, dtype=torch.int64, device=dev)   # (seed, first rollout id) of env.search_begin, read by the kernels
+            self.eval_index = torch.zeros(1, dtype=i32, device=dev)           # evaluation index - 1 (reset by the root pass, advanced by back-up)
+            self._key = None
         self.use_graph = bool(use_cuda_graph)
         self._graphs = None         # (module captured, root graph or None, simulation graph or None, whole-decision graph or None)
         self._stream = torch.cuda.Stream(device=dev)
@@ -131,6 +189,14 @@ class MCTSSearch:
         if self.reuse:
             tree.reroot(pool, env, self.chosen, self.NC - self.S, self.reused)
         _, done, _, _ = env.status()
+        if self.use_twists:
+            observe_twisted(env, None, None, None, self.search_key, self.eval_index, self.qperm_table, self.root_bits, self.root_twist)
+            self.fused.forward_bits(self.root_bits, probs=self.pri, values=self.val)
+            if self.hook:
+                self.hook("root", decision, -1, self.pri, None, self.root_twist, self.root_bits)
+            pool.copy_records_from(env, self.root_slots)
+            tree.begin_twisted(self.pri, done, self.act_table, self.root_twist, self.reused if self.reuse else None)
+            return
         if self.backend == "fused":
             env.observe_bits(self.root_bits)
             self.fused.forward_bits(self.root_bits, probs=self.pri, values=self.val)
@@ -149,6 +215,14 @@ class MCTSSearch:
     def _simulation(self, decision: int = 0, s: int = 0):
         pool, tree = self.pool, self.tree
         tree.select(self.c_puct, self.src, self.dst, self.act)
+        if self.use_twists:
+            pool.step_slots(self.src, self.dst, self.act, reward=self.leaf_reward, done=self.leaf_done)
+            observe_twisted(self.env, pool, self.dst, self.act, self.search_key, self.eval_index, self.qperm_table, self.leaf_bits, self.leaf_twist)
+            self.fused.forward_bits(self.leaf_bits, probs=self.pri, values=self.val)
+            if self.hook:
+                self.hook("leaf", decision, s, self.pri, self.val, self.leaf_twist, self.leaf_bits)
+            tree.backup_twisted(self.pri, self.val, self.leaf_reward, self.leaf_done, self.act_table, self.leaf_twist, self.eval_index)
+            return
         if self.backend == "fused":
             pool.step_slots(self.src, self.dst, self.act, obs_bits=self.leaf_bits, reward=self.leaf_reward, done=self.leaf_done)
             self.fused.forward_bits(self.leaf_bits, probs=self.pri, values=self.val)
@@ -195,6 +269,13 @@ class MCTSSearch:
         if (self.fused is not None and self.fused.refresh(self.policy)) or (self._graphs is not None and self._graphs[0] is not self.policy):
             self._graphs = None
         fresh, self._fresh = self._fresh, False
+        if self.use_twists and self._key != self.env.search_key:
+            # read by the kernels at run time, so the captured graphs serve every seed; written outside them, on the caller's stream
+            # (fills carry the values as kernel arguments: no host synchronisation)
+            seed, first = self.env.search_key
+            self.search_key[0].fill_(seed - (1 << 64) if seed >= (1 << 63) else seed)
+            self.search_key[1].fill_(first)
+            self._key = self.env.search_key
         if not self.use_graph or self.hook is not None:
             return self._decide_eager(decision)
         if self._graphs is None:

@@ -382,13 +382,20 @@ class AlphaZero(Trainer):
     `num_mcts_searches` PUCT simulations; the action is sampled from the root's visit counts; the policy is trained towards
     the visit distribution (cross entropy) and the value head towards the episode's return-to-go (undiscounted, like the tree's
     own back-up; episodes cut by the end of the collection bootstrap from the value head).  Config: AlphaZeroConfig.to_json()
-    (configs.py:404-429).  twisterl's AZ is not in the reference tree: this follows the config docstrings (295-323), not its code."""
+    (configs.py:404-429).  twisterl's AZ is not in the reference tree: this follows the config docstrings (295-323), not its code.
+    use_twists: self-play runs the twisted tree search (MCTSSearch(use_twists=True)), so the policy learns in the env's symmetry frames
+    as PPO's collector trains it.  A sample is the root observation as the root evaluation saw it (in frame k), and its target is the
+    visit distribution in the policy's action order, tgt[act_perm[k][a]] = w[a]; the env still plays the sampled env action.  Raises
+    before anything is allocated where the twisted tree search cannot run (mcts.check_twisted_tree_search)."""
 
     algorithm = "AZ"
 
     def __init__(self, env_kind: int, num_qubits: int, gateset, policy: torch.nn.Module, config: dict | None = None, device=None,
-                 seed: int = 0, minibatch_size: int | None = None, vf_coef: float = 1.0, **env_kwargs):
-        from .mcts import MCTSSearch
+                 seed: int = 0, minibatch_size: int | None = None, vf_coef: float = 1.0, use_twists: bool = False, **env_kwargs):
+        from .mcts import MCTSSearch, check_twisted_tree_search
+        self.use_twists = bool(use_twists)
+        if self.use_twists:
+            check_twisted_tree_search(env_kind, num_qubits, policy, "auto", env_kwargs)
         self._mcts_cls = MCTSSearch
         self._policy_for_env = policy
         self.vf_coef = float(vf_coef)
@@ -402,47 +409,14 @@ class AlphaZero(Trainer):
         if int(c["max_expand_depth"]) != 1:
             raise NotImplementedError("max_expand_depth != 1 is not supported by the device tree search (mcts.py)")
         kind, n, gs, kw = self.spec
-        self.search = self._mcts_cls(kind, n, gs, self._policy_for_env, batch, int(c["num_mcts_searches"]), C=float(c["C"]), device=device, **kw)
+        twist_kw = {"use_twists": True} if self.use_twists else {}
+        self.search = self._mcts_cls(kind, n, gs, self._policy_for_env, batch, int(c["num_mcts_searches"]), C=float(c["C"]), device=device,
+                                     **twist_kw, **kw)
         return self.search.env
 
     def iterate(self) -> dict:
-        from .collector import gae
-        env, ms, T, B = self.env, self.search, self._episode_steps(), self.env.batch
-        ms.policy = self.policy.eval()
-        dev, A = self.device, env.num_actions()
-        obs_buf = torch.empty((T, B) + tuple(env.obs_shape()), dtype=torch.float32, device=dev)
-        pi = torch.zeros((T, B, A), dtype=torch.float32, device=dev)
-        actions = torch.full((T, B), -1, dtype=torch.int32, device=dev)
-        rewards = torch.zeros((T, B), dtype=torch.float32, device=dev)
-        dones = torch.zeros((T, B), dtype=torch.bool, device=dev)
-        succ = torch.zeros((T, B), dtype=torch.bool, device=dev)
-        for t in range(T):
-            s = decision_seed(self.seed + 104729 * self.rank, self.counter)
-            env.reset_select(s, self.rank * B)
-            w = ms.decide(t)                         # grows the trees from the root observation, leaves N(a) / sum N in ms.weights
-            if ms.backend == "fused":
-                # the fused backend observes into packed bits only (ms.root_bits): the training sample is what the root evaluation saw
-                # (for PauliNetwork with add_perms that includes the qubit permutation observe() picked)
-                obs_buf[t].copy_(unpack_bits(ms.root_bits, env._obs_size).reshape(obs_buf[t].shape))
-            else:
-                obs_buf[t].copy_(env.obs)
-            pi[t].copy_(w)
-            env.collect_step(w, s, deterministic=False, obs=False, chosen=actions[t], reward=rewards[t], done=dones[t], success=succ[t])
-            self.counter += 1
-        valid = actions >= 0
-        values = torch.zeros((T + 1, B), dtype=torch.float32, device=dev)
-        with torch.no_grad():
-            values[T] = self.policy(env.observe())[1].float().reshape(-1)
-        _, ret = gae(rewards, values, dones, 1.0, 1.0, valid)        # V = 0 inside, gamma = lambda = 1: the return-to-go (+ bootstrap)
-        fin = dones & valid
-        n_ep = int(fin.sum().item())
-        rec = {"episodes": n_ep, "collect_success": (float((succ & fin).sum().item()) / n_ep) if n_ep else 0.0,
-               "mean_reward": float(rewards[valid].mean().item()) if bool(valid.any()) else 0.0}
-        idx = valid.reshape(-1).nonzero(as_tuple=False).squeeze(1)
-        obs = obs_buf.reshape((-1,) + tuple(obs_buf.shape[2:]))[idx]
-        tgt_pi = pi.reshape(-1, A)[idx]
-        tgt_v = ret.reshape(-1)[idx]
-        n = int(idx.numel())
+        rec, obs, tgt_pi, tgt_v, _ = self.self_play()
+        n = int(obs.shape[0])
         self.policy.train()
         stats = {}
         for _ in range(int(self.cfg["training"]["num_epochs"])):
@@ -457,3 +431,47 @@ class AlphaZero(Trainer):
         self.policy.eval()
         rec.update({k: float(v.item()) for k, v in stats.items()} | {"samples": n})
         return rec
+
+    def self_play(self):
+        """One collection of self-play: -> (episode stats, the training samples' observations, policy targets and value targets, and
+        the samples' indices into the flattened [steps, envs] decisions)."""
+        from .collector import gae
+        env, ms, T, B = self.env, self.search, self._episode_steps(), self.env.batch
+        ms.policy = self.policy.eval()
+        dev, A = self.device, env.num_actions()
+        obs_buf = torch.empty((T, B) + tuple(env.obs_shape()), dtype=torch.float32, device=dev)
+        pi = torch.zeros((T, B, A), dtype=torch.float32, device=dev)
+        actions = torch.full((T, B), -1, dtype=torch.int32, device=dev)
+        rewards = torch.zeros((T, B), dtype=torch.float32, device=dev)
+        dones = torch.zeros((T, B), dtype=torch.bool, device=dev)
+        succ = torch.zeros((T, B), dtype=torch.bool, device=dev)
+        for t in range(T):
+            s = decision_seed(self.seed + 104729 * self.rank, self.counter)
+            env.reset_select(s, self.rank * B)
+            if self.use_twists:
+                env.search_begin(s, self.rank * B)   # the frames' seed and global ids (AZ reads no search returns)
+            w = ms.decide(t)                         # grows the trees from the root observation, leaves N(a) / sum N in ms.weights
+            if ms.backend == "fused":
+                # the fused backend observes into packed bits only (ms.root_bits): the training sample is what the root evaluation saw
+                # (for PauliNetwork with add_perms that includes the qubit permutation observe() picked)
+                obs_buf[t].copy_(unpack_bits(ms.root_bits, env._obs_size).reshape(obs_buf[t].shape))
+            else:
+                obs_buf[t].copy_(env.obs)
+            if self.use_twists:
+                pi[t].scatter_(1, ms.act_table[ms.root_twist.long()].long(), w)      # the target in the policy's action order
+            else:
+                pi[t].copy_(w)
+            env.collect_step(w, s, deterministic=False, obs=False, chosen=actions[t], reward=rewards[t], done=dones[t], success=succ[t])
+            self.counter += 1
+        valid = actions >= 0
+        values = torch.zeros((T + 1, B), dtype=torch.float32, device=dev)
+        with torch.no_grad():
+            values[T] = self.policy(env.observe())[1].float().reshape(-1)
+        _, ret = gae(rewards, values, dones, 1.0, 1.0, valid)        # V = 0 inside, gamma = lambda = 1: the return-to-go (+ bootstrap)
+        fin = dones & valid
+        n_ep = int(fin.sum().item())
+        rec = {"episodes": n_ep, "collect_success": (float((succ & fin).sum().item()) / n_ep) if n_ep else 0.0,
+               "mean_reward": float(rewards[valid].mean().item()) if bool(valid.any()) else 0.0}
+        idx = valid.reshape(-1).nonzero(as_tuple=False).squeeze(1)
+        obs = obs_buf.reshape((-1,) + tuple(obs_buf.shape[2:]))[idx]
+        return rec, obs, pi.reshape(-1, A)[idx], ret.reshape(-1)[idx], idx

@@ -141,7 +141,7 @@ class RLSynthesis:
         if not use_twists:
             return
         if num_mcts_searches:
-            raise NotImplementedError("use_twists applies to the rollout search (num_mcts_searches = 0); the tree search runs untwisted")
+            raise NotImplementedError("use_twists applies to the rollout search (num_mcts_searches = 0); RLSynthesis runs the tree search untwisted (the twisted one is mcts.MCTSSearch(use_twists=True))")
         check_twisted_search(_ENV_KINDS[self.env.cls_name], self.env_config["num_qubits"], "persistent")
 
     def solve(self, state, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
@@ -219,13 +219,15 @@ class RLSynthesis:
             return self.env.build_circuit_from_solution(actions, input)
 
     def learn(self, initial_difficulty=1, num_iterations=int(1e10), tb_path=None, log=None, seed: int = 0, matmul_precision: str = "f32",
-              update_precision: str = "f32"):
+              update_precision: str = "f32", use_twists: bool | None = None):
         """rl/synthesis.py:128-139: PPO (`twisterl.rl.PPO`) or AlphaZero (`twisterl.rl.AZ`) on the device (ppo.py).  The trained
         policy is `self.policy` (searches built before the call are dropped so that `synth` uses the new weights).
         matmul_precision (PPO): how the collector runs the policy — "f32" (the reference's arithmetic, the default), "tf32", "bf16", or
         "tensor_core" (packed observations and the tcgen05 policy: RolloutCollector.collect_packed).
         update_precision (PPO): "f32" (the default) or "tensor_core" (the update's forward and backward on the tcgen05 kernels; needs
-        matmul_precision="tensor_core")."""
+        matmul_precision="tensor_core").
+        use_twists: train in the env's symmetry frames (PPO's collector, AlphaZero's twisted tree search); None keeps each trainer's own
+        default (PPO twisted, AlphaZero untwisted)."""
         from . import ppo
         algo = self.algorithm_cls.split(".")[-1]
         if algo not in ("PPO", "AZ"):
@@ -238,6 +240,8 @@ class RLSynthesis:
         if algo == "PPO":
             kw["matmul_precision"] = matmul_precision
             kw["update_precision"] = update_precision
+        if use_twists is not None:
+            kw["use_twists"] = bool(use_twists)
         trainer = (ppo.PPO if algo == "PPO" else ppo.AlphaZero)(kind, n, gs, self.policy, self.rl_config, device=self.device, seed=seed, **kw)
         if hasattr(self.env, "difficulty"):
             self.env.difficulty = initial_difficulty                # rl/synthesis.py:129 (a reference *Gym object; a SynthSpec owns no env)

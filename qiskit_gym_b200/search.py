@@ -118,6 +118,16 @@ def check_twisted_search(env_kind: int, num_qubits: int, policy_backend: str):
         raise NotImplementedError(f"the twisted search needs packed observations: a Permutation of {num_qubits} > 64 qubits has none")
 
 
+def twist_tables(env: BatchedEnv):
+    """The env's twists (env.twists(), built with add_perms), once, on its device: uint8 [K, n] inverse qubit permutations
+    (collector.qubit_twist_table) and int32 [K, A] act perms -- the tables of the twisted rollout and tree searches."""
+    from .collector import qubit_twist_table
+    obs_perms, act_perms = env.twists()
+    qperm = torch.from_numpy(qubit_twist_table(obs_perms, int(env.cfg.num_qubits))).to(env.device)
+    act = torch.from_numpy(np.asarray(act_perms, dtype=np.int32)).to(env.device)
+    return qperm, act
+
+
 def reduce_best(local_key: int, local_solution, group=None, device=None):
     """Cross-rank best-rollout reduction in two collectives: an all-gather of (packed key, solution length) — the owner of the winning
     rollout is the rank holding the largest key; keys are unique, they embed the global rollout id — then the owner broadcasts its action
@@ -229,11 +239,7 @@ class RolloutSearch:
         self.use_twists = bool(use_twists)
         self.qperm_table = self.act_table = self.twist = None
         if self.use_twists:
-            # the env's twists, once, on the device: uint8 [K, n] inverse qubit permutations, int32 [K, A] act perms; the frames int32 [B]
-            from .collector import qubit_twist_table
-            obs_perms, act_perms = self.env.twists()
-            self.qperm_table = torch.from_numpy(qubit_twist_table(obs_perms, num_qubits)).to(dev)
-            self.act_table = torch.from_numpy(np.asarray(act_perms, dtype=np.int32)).to(dev)
+            self.qperm_table, self.act_table = twist_tables(self.env)
             self.twist = torch.zeros(self.B, dtype=torch.int32, device=dev)
         self.num_twists = 0 if self.qperm_table is None else int(self.qperm_table.shape[0])
         self.use_graph = use_cuda_graph
