@@ -11,6 +11,9 @@ a child node's env is the parent's record cloned and stepped in one pass through
 With `reuse_tree=True` a decision starts from the subtree below the action the rollout played (AlphaGo Zero's tree reuse), kept
 when the tree's node for it holds the env the rollout reached (csrc/qg_mcts.cu states the rule).
 
+With `policy_backend="tensor_core"` the roots and leaves are evaluated by the tcgen05 tensor-core policy (policy.TensorCorePolicy) instead of
+the f32 FFMA kernel: opt-in, for searches over thousands of trees, where the FFMA policy is what a simulation waits for.
+
 With `use_twists=True` every policy evaluation of a tree (its root, each new leaf) runs in a symmetry frame of the env drawn per
 rollout, decision and evaluation, the way the collector trains the policy; the trees keep their priors in env action order
 (csrc/qg_mcts.cu states the protocol).
@@ -28,7 +31,7 @@ import torch
 from . import _abi
 from ._lib import check, lib
 from .engine import BatchedEnv, _dptr
-from .search import SearchResult, best_rollout, check_twisted_search, search_result, twist_tables
+from .search import SearchResult, best_rollout, check_tensor_core_search, check_twisted_search, search_result, twist_tables
 
 
 class TreeArrays:
@@ -103,6 +106,15 @@ def check_twisted_tree_search(env_kind: int, num_qubits: int, policy: torch.nn.M
         raise ValueError("use_twists needs the env's twists: add_perms=False contradicts it")
 
 
+def check_tensor_core_tree_search(env_kind: int, num_qubits: int, num_actions: int, policy: torch.nn.Module, device=None):
+    """Raises NotImplementedError, before anything is allocated, where the "tensor_core" tree search cannot run: the tensor-core search's
+    limits (search.check_tensor_core_search) and a policy without single-Linear action / value heads (the trees need the value head)."""
+    from .policy import simple_value_head
+    if simple_value_head(policy) is None:
+        raise NotImplementedError("the tensor-core tree search evaluates the value head with the policy: it needs single-Linear action / value heads")
+    check_tensor_core_search(env_kind, num_qubits, num_actions, device)
+
+
 class MCTSSearch:
     """`solve` with a tree search per decision.  Owns the rollout engine (R envs, solutions tracked) and a slot-pool engine of
     R * node_cap records for the tree nodes (node_cap = num_mcts_searches + 1, or 2 * num_mcts_searches + 1 with reuse_tree)."""
@@ -114,7 +126,17 @@ class MCTSSearch:
         are captured once and replayed: the whole decision as one graph up to 128 simulations, one graph per simulation beyond.
         policy_backend: "fused" = priors and values of the root / the leaves from packed observations in one kernel (policy.FusedPolicy
         with the value head, refreshed from `policy` before every decision), "torch" = the PyTorch module on dense observations, "auto" =
-        fused when the policy has the simple head layout and the env can pack its observations.
+        fused when the policy has the simple head layout and the env can pack its observations.  "tensor_core" = the "fused" decision with
+        the priors and values from the tcgen05 tensor-core policy (policy.TensorCorePolicy with max_batch = num_rollouts and the value
+        head) on the same packed observations; built for searches over thousands of trees.  It is opt-in and never chosen by "auto": its
+        f16 hi+lo split arithmetic rounds differently from the f32 backends, so its trees are not theirs (priors and values within
+        TensorCorePolicy's error bound of the float64 module).  Each row's outputs are bit-identical whatever the batch, so a tree's
+        search does not depend on how many trees share the launch.  NotImplementedError, before anything is allocated, where it cannot
+        run: more than 127 actions, a Permutation wider than 64 qubits, a device that is not sm_100 (search.check_tensor_core_search),
+        a policy without single-Linear action / value heads.
+        Every decision starts by refreshing the policy handle from `self.policy`: "fused" recreates it on a weight change (the decision
+        graphs are captured again), "tensor_core" loads a weight update (optimizer step, load_state_dict) in place, so the captured
+        graphs stay valid and replay the new weights.
         reuse_tree: each decision after the first of a `solve` keeps up to num_mcts_searches + 1 nodes of the subtree below the action
         the rollout played, with their statistics, and adds num_mcts_searches simulations to them (qg_mcts_reroot).  The rollout's
         action must then reach `decide` through `chosen` (solve does it; a caller driving decide itself passes chosen=self.chosen
@@ -122,12 +144,14 @@ class MCTSSearch:
         use_twists: the twisted tree search (include/qg_engine.h qg_mcts_observe_twisted): the root and every new leaf are evaluated in
         a symmetry frame of the env (its twists() with add_perms) drawn from the seed and first rollout id of env.search_begin, the
         rollout's global id, its step counter and the evaluation index; the node stores P(a) = probs[act_perm[k][a]].  Runs on the fused
-        backend; `root_twist` holds the root frames of the last decision and `root_bits` the twisted root observations.  Raises before
-        anything is allocated where it cannot run (check_twisted_tree_search)."""
-        assert num_mcts_searches >= 1 and policy_backend in ("auto", "fused", "torch")
+        and "tensor_core" backends; `root_twist` holds the root frames of the last decision and `root_bits` the twisted root
+        observations.  Raises before anything is allocated where it cannot run (check_twisted_tree_search)."""
+        assert num_mcts_searches >= 1 and policy_backend in ("auto", "fused", "torch", "tensor_core")
         if use_twists:
             check_twisted_tree_search(env_kind, num_qubits, policy, policy_backend, env_kwargs)
             env_kwargs["add_perms"] = True
+        if policy_backend == "tensor_core":
+            check_tensor_core_tree_search(env_kind, num_qubits, len(gateset), policy, device)
         env_kwargs.setdefault("add_perms", False)
         self.env = BatchedEnv(env_kind, num_qubits, gateset, num_rollouts, device=device, max_depth=max_depth, **env_kwargs)
         pool_kwargs = dict(env_kwargs, track_solution=False)
@@ -153,18 +177,24 @@ class MCTSSearch:
         self.num_active = torch.zeros(1, dtype=torch.int32, device=dev)
         self.hook = None            # tests: hook(kind, decision, simulation, prior, value) sees the policy outputs the trees consumed;
                                     # twisted searches call hook(kind, decision, simulation, prior, value, frames, obs_bits)
-        from .policy import FusedPolicy, simple_value_head
+        from .policy import FusedPolicy, TensorCorePolicy, simple_value_head
         can_fuse = simple_value_head(self.policy) is not None and not (env_kind == 0 and num_qubits > 64)      # (no packed observations for n > 64 permutations)
         if policy_backend == "fused" and not can_fuse:
             raise NotImplementedError("policy_backend='fused' needs single-Linear action / value heads")
-        self.backend = "fused" if (policy_backend != "torch" and can_fuse) else "torch"
-        self.fused = None
-        if self.backend == "fused":
+        if policy_backend == "tensor_core":
+            self.backend = "tensor_core"
+        else:
+            self.backend = "fused" if (policy_backend != "torch" and can_fuse) else "torch"
+        self.handle = None          # the policy's C handle (policy.FusedPolicy / TensorCorePolicy); None for "torch"
+        if self.backend != "torch":
             self.root_bits = self.env.new_obs_bits()
             self.leaf_bits = torch.zeros((self.R, self.env.obs_words()), dtype=torch.int32, device=dev)
             self.pri = torch.zeros((self.R, A), dtype=torch.float32, device=dev)
             self.val = torch.zeros(self.R, dtype=torch.float32, device=dev)
-            self.fused = FusedPolicy(self.policy, device=dev, with_value=True)
+            if self.backend == "fused":
+                self.handle = FusedPolicy(self.policy, device=dev, with_value=True)
+            else:
+                self.handle = TensorCorePolicy(self.policy, max_batch=self.R, device=dev, with_value=True)
         self.use_twists = bool(use_twists)
         self.num_twists = 0
         if self.use_twists:
@@ -179,6 +209,9 @@ class MCTSSearch:
         self._graphs = None         # (module captured, root graph or None, simulation graph or None, whole-decision graph or None)
         self._stream = torch.cuda.Stream(device=dev)
 
+    # the handle under the name it had before `handle` (read by existing callers): None for the other backends
+    fused = property(lambda self: self.handle if self.backend == "fused" else None)
+
     def _policy(self, obs):
         with torch.no_grad():
             logits, value = self.policy(obs)
@@ -191,15 +224,15 @@ class MCTSSearch:
         _, done, _, _ = env.status()
         if self.use_twists:
             observe_twisted(env, None, None, None, self.search_key, self.eval_index, self.qperm_table, self.root_bits, self.root_twist)
-            self.fused.forward_bits(self.root_bits, probs=self.pri, values=self.val)
+            self.handle.forward_bits(self.root_bits, probs=self.pri, values=self.val)
             if self.hook:
                 self.hook("root", decision, -1, self.pri, None, self.root_twist, self.root_bits)
             pool.copy_records_from(env, self.root_slots)
             tree.begin_twisted(self.pri, done, self.act_table, self.root_twist, self.reused if self.reuse else None)
             return
-        if self.backend == "fused":
+        if self.backend != "torch":
             env.observe_bits(self.root_bits)
-            self.fused.forward_bits(self.root_bits, probs=self.pri, values=self.val)
+            self.handle.forward_bits(self.root_bits, probs=self.pri, values=self.val)
             prior = self.pri
         else:
             env.observe()
@@ -218,14 +251,14 @@ class MCTSSearch:
         if self.use_twists:
             pool.step_slots(self.src, self.dst, self.act, reward=self.leaf_reward, done=self.leaf_done)
             observe_twisted(self.env, pool, self.dst, self.act, self.search_key, self.eval_index, self.qperm_table, self.leaf_bits, self.leaf_twist)
-            self.fused.forward_bits(self.leaf_bits, probs=self.pri, values=self.val)
+            self.handle.forward_bits(self.leaf_bits, probs=self.pri, values=self.val)
             if self.hook:
                 self.hook("leaf", decision, s, self.pri, self.val, self.leaf_twist, self.leaf_bits)
             tree.backup_twisted(self.pri, self.val, self.leaf_reward, self.leaf_done, self.act_table, self.leaf_twist, self.eval_index)
             return
-        if self.backend == "fused":
+        if self.backend != "torch":
             pool.step_slots(self.src, self.dst, self.act, obs_bits=self.leaf_bits, reward=self.leaf_reward, done=self.leaf_done)
-            self.fused.forward_bits(self.leaf_bits, probs=self.pri, values=self.val)
+            self.handle.forward_bits(self.leaf_bits, probs=self.pri, values=self.val)
             p, v = self.pri, self.val
         else:
             pool.step_slots(self.src, self.dst, self.act, obs=self.leaf_obs, reward=self.leaf_reward, done=self.leaf_done)
@@ -266,7 +299,7 @@ class MCTSSearch:
     def decide(self, decision: int = 0):
         """One decision's tree search for every rollout; leaves the root visit weights in self.weights."""
         # a graph holds the policy handle and the module's parameter tensors
-        if (self.fused is not None and self.fused.refresh(self.policy)) or (self._graphs is not None and self._graphs[0] is not self.policy):
+        if (self.handle is not None and self.handle.refresh(self.policy)) or (self._graphs is not None and self._graphs[0] is not self.policy):
             self._graphs = None
         fresh, self._fresh = self._fresh, False
         if self.use_twists and self._key != self.env.search_key:

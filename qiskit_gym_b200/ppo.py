@@ -386,16 +386,26 @@ class AlphaZero(Trainer):
     use_twists: self-play runs the twisted tree search (MCTSSearch(use_twists=True)), so the policy learns in the env's symmetry frames
     as PPO's collector trains it.  A sample is the root observation as the root evaluation saw it (in frame k), and its target is the
     visit distribution in the policy's action order, tgt[act_perm[k][a]] = w[a]; the env still plays the sampled env action.  Raises
-    before anything is allocated where the twisted tree search cannot run (mcts.check_twisted_tree_search)."""
+    before anything is allocated where the twisted tree search cannot run (mcts.check_twisted_tree_search).
+    matmul_precision: how self-play's tree search evaluates the policy, "f32" (the default: the fused FFMA kernel, or the PyTorch module
+    where that cannot run) or "tensor_core" (MCTSSearch(policy_backend="tensor_core"): the tcgen05 policy, for thousands of episodes per
+    iteration; NotImplementedError, before anything is allocated, where it cannot run).  The evals, the bootstrap value and the update
+    stay f32 PyTorch either way."""
 
     algorithm = "AZ"
 
     def __init__(self, env_kind: int, num_qubits: int, gateset, policy: torch.nn.Module, config: dict | None = None, device=None,
-                 seed: int = 0, minibatch_size: int | None = None, vf_coef: float = 1.0, use_twists: bool = False, **env_kwargs):
-        from .mcts import MCTSSearch, check_twisted_tree_search
+                 seed: int = 0, minibatch_size: int | None = None, vf_coef: float = 1.0, use_twists: bool = False, matmul_precision: str = "f32",
+                 **env_kwargs):
+        from .mcts import MCTSSearch, check_tensor_core_tree_search, check_twisted_tree_search
+        if matmul_precision not in ("f32", "tensor_core"):
+            raise ValueError(f"AlphaZero's matmul_precision must be f32 or tensor_core (got {matmul_precision!r})")
         self.use_twists = bool(use_twists)
+        self.policy_backend = "tensor_core" if matmul_precision == "tensor_core" else "auto"
         if self.use_twists:
-            check_twisted_tree_search(env_kind, num_qubits, policy, "auto", env_kwargs)
+            check_twisted_tree_search(env_kind, num_qubits, policy, self.policy_backend, env_kwargs)
+        if matmul_precision == "tensor_core":
+            check_tensor_core_tree_search(env_kind, num_qubits, len(gateset), policy, device)
         self._mcts_cls = MCTSSearch
         self._policy_for_env = policy
         self.vf_coef = float(vf_coef)
@@ -411,7 +421,7 @@ class AlphaZero(Trainer):
         kind, n, gs, kw = self.spec
         twist_kw = {"use_twists": True} if self.use_twists else {}
         self.search = self._mcts_cls(kind, n, gs, self._policy_for_env, batch, int(c["num_mcts_searches"]), C=float(c["C"]), device=device,
-                                     **twist_kw, **kw)
+                                     policy_backend=self.policy_backend, **twist_kw, **kw)
         return self.search.env
 
     def iterate(self) -> dict:
@@ -451,8 +461,8 @@ class AlphaZero(Trainer):
             if self.use_twists:
                 env.search_begin(s, self.rank * B)   # the frames' seed and global ids (AZ reads no search returns)
             w = ms.decide(t)                         # grows the trees from the root observation, leaves N(a) / sum N in ms.weights
-            if ms.backend == "fused":
-                # the fused backend observes into packed bits only (ms.root_bits): the training sample is what the root evaluation saw
+            if ms.backend != "torch":
+                # the packed backends observe into bits only (ms.root_bits): the training sample is what the root evaluation saw
                 # (for PauliNetwork with add_perms that includes the qubit permutation observe() picked)
                 obs_buf[t].copy_(unpack_bits(ms.root_bits, env._obs_size).reshape(obs_buf[t].shape))
             else:

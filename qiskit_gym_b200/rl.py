@@ -125,13 +125,17 @@ class RLSynthesis:
             self._searches[key] = rs
         return rs
 
-    def _mcts(self, num_searches: int, num_mcts_searches: int, C: float, reuse_tree: bool = False):
+    def _mcts(self, num_searches: int, num_mcts_searches: int, C: float, reuse_tree: bool = False, matmul_precision: str = "f32"):
+        """The cached tree search; matmul_precision="tensor_core": MCTSSearch's "tensor_core" backend, cached under its own key."""
         from .mcts import MCTSSearch
         key = ("mcts", num_searches, num_mcts_searches, C, reuse_tree)
+        backend = {}
+        if matmul_precision == "tensor_core":
+            key, backend = ("tensor_core", key), {"policy_backend": "tensor_core"}
         ms = self._searches.get(key)
         if ms is None:
             kind, n, gs, kw = self._env_args(add_perms=False)
-            ms = MCTSSearch(kind, n, gs, self.policy, num_searches, num_mcts_searches, C=C, device=self.device, reuse_tree=reuse_tree, **kw)
+            ms = MCTSSearch(kind, n, gs, self.policy, num_searches, num_mcts_searches, C=C, device=self.device, reuse_tree=reuse_tree, **backend, **kw)
             self._searches[key] = ms
         return ms
 
@@ -145,21 +149,31 @@ class RLSynthesis:
         check_twisted_search(_ENV_KINDS[self.env.cls_name], self.env_config["num_qubits"], "persistent")
 
     def solve(self, state, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
-              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False, use_twists: bool = False):
+              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False, use_twists: bool = False, matmul_precision: str = "f32"):
         """twisterl `Algorithm.solve`: the action list of the best successful rollout, or None.
         reuse_tree (tree search only): every decision but the first starts from the subtree below the action played (mcts.MCTSSearch).
         use_twists: every rollout runs the policy in a symmetry frame of the env drawn per decision, as the reference's twisted policy
         does (RolloutSearch(use_twists=True)); NotImplementedError with num_mcts_searches > 0, for PauliNetwork and for a Permutation
-        wider than 64 qubits."""
+        wider than 64 qubits.
+        matmul_precision: "f32" (the default) or "tensor_core": the policy on tcgen05 tensor cores, in the tree search
+        (MCTSSearch(policy_backend="tensor_core")) with num_mcts_searches > 0, else in the rollout search (RolloutSearch's "tensor_core"
+        backend).  It rounds differently from f32, so its results are those of a "tensor_core" search; NotImplementedError where it
+        cannot run (more than 127 actions, a Permutation wider than 64 qubits, a device that is not sm_100, and for the tree search a
+        policy without single-Linear action / value heads) instead of falling back to another arithmetic."""
         self._check_twists(use_twists, num_mcts_searches)
         if reuse_tree and not num_mcts_searches:
             raise ValueError("reuse_tree needs a tree search (num_mcts_searches > 0)")
-        if num_mcts_searches:
-            if max_expand_depth != 1:
-                raise NotImplementedError("max_expand_depth != 1 is not supported by the device tree search (mcts.py)")
-            return self._mcts(int(num_searches), int(num_mcts_searches), float(C), bool(reuse_tree)).solve(state, deterministic=deterministic,
-                                                                                                             seed=seed).actions
-        return self._search(int(num_searches), use_twists=use_twists).solve(state, deterministic=deterministic, seed=seed).actions
+        if num_mcts_searches and max_expand_depth != 1:
+            raise NotImplementedError("max_expand_depth != 1 is not supported by the device tree search (mcts.py)")
+        if matmul_precision not in ("f32", "tensor_core"):
+            raise ValueError(f"matmul_precision must be f32 or tensor_core (got {matmul_precision!r})")
+        if num_mcts_searches:                            # (MCTSSearch refuses what its "tensor_core" backend cannot run before it allocates)
+            ms = self._mcts(int(num_searches), int(num_mcts_searches), float(C), bool(reuse_tree), matmul_precision)
+            return ms.solve(state, deterministic=deterministic, seed=seed).actions
+        if matmul_precision == "tensor_core":
+            check_tensor_core_search(_ENV_KINDS[self.env.cls_name], self.env_config["num_qubits"], self.env.num_actions(), self.device)
+        return self._search(int(num_searches), matmul_precision=matmul_precision, use_twists=use_twists).solve(state, deterministic=deterministic,
+                                                                                                            seed=seed).actions
 
     def solve_many(self, states, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, seed: int = 0,
                    max_rollouts: int = 65536, matmul_precision: str = "f32", use_twists: bool = False):
@@ -208,13 +222,13 @@ class RLSynthesis:
         return out
 
     def synth(self, input, deterministic: bool = False, num_searches: int = 100, num_mcts_searches: int = 0, C: float = 2 ** 0.5,
-              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False, use_twists: bool = False):
+              max_expand_depth: int = 1, seed: int = 0, reuse_tree: bool = False, use_twists: bool = False, matmul_precision: str = "f32"):
         """rl/synthesis.py:112-126.  Returns the synthesised circuit (QuantumCircuit with Qiskit, else a gate list) or None.
-        use_twists: see solve."""
+        use_twists, matmul_precision: see solve."""
         self._check_twists(use_twists, num_mcts_searches)
         state = self.env.get_state(input)
         actions = self.solve(state, deterministic, num_searches, num_mcts_searches, C, max_expand_depth, seed=seed, reuse_tree=reuse_tree,
-                             use_twists=use_twists)
+                             use_twists=use_twists, matmul_precision=matmul_precision)
         if actions is not None:
             return self.env.build_circuit_from_solution(actions, input)
 
@@ -223,7 +237,8 @@ class RLSynthesis:
         """rl/synthesis.py:128-139: PPO (`twisterl.rl.PPO`) or AlphaZero (`twisterl.rl.AZ`) on the device (ppo.py).  The trained
         policy is `self.policy` (searches built before the call are dropped so that `synth` uses the new weights).
         matmul_precision (PPO): how the collector runs the policy — "f32" (the reference's arithmetic, the default), "tf32", "bf16", or
-        "tensor_core" (packed observations and the tcgen05 policy: RolloutCollector.collect_packed).
+        "tensor_core" (packed observations and the tcgen05 policy: RolloutCollector.collect_packed).  (AlphaZero): how self-play's tree
+        search evaluates the policy — "f32" (the default) or "tensor_core" (MCTSSearch(policy_backend="tensor_core")); "tf32" / "bf16" raise.
         update_precision (PPO): "f32" (the default) or "tensor_core" (the update's forward and backward on the tcgen05 kernels; needs
         matmul_precision="tensor_core").
         use_twists: train in the env's symmetry frames (PPO's collector, AlphaZero's twisted tree search); None keeps each trainer's own
@@ -232,13 +247,13 @@ class RLSynthesis:
         algo = self.algorithm_cls.split(".")[-1]
         if algo not in ("PPO", "AZ"):
             raise NotImplementedError(f"algorithm class {self.algorithm_cls} is not supported (twisterl.rl.PPO, twisterl.rl.AZ)")
-        if algo == "AZ" and matmul_precision != "f32":
-            raise NotImplementedError("matmul_precision applies to PPO only (AlphaZero evaluates its policy inside the tree search)")
+        if algo == "AZ" and matmul_precision not in ("f32", "tensor_core"):
+            raise NotImplementedError("AlphaZero's tree search runs its policy in f32 or on the tensor cores (matmul_precision f32 / tensor_core)")
         if algo == "AZ" and update_precision != "f32":
             raise NotImplementedError("update_precision applies to PPO only (the AlphaZero update runs in f32 PyTorch)")
         kind, n, gs, kw = self._env_args()
+        kw["matmul_precision"] = matmul_precision
         if algo == "PPO":
-            kw["matmul_precision"] = matmul_precision
             kw["update_precision"] = update_precision
         if use_twists is not None:
             kw["use_twists"] = bool(use_twists)
